@@ -3,6 +3,9 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (N>1: launched by torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference algorithm on the host CPU
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # + the last step's histograms as DIR/*.npy
+
+The inputs are generated from fixed seeds, so two builds run with the same arguments can be compared output for output.
 
 Workload (BASELINE.json configs[1], "C2", at its full size): synthetic LJ-like fluid, 100 000 atoms per frame,
 1 000 frames, triclinic cell (lx=ly=lz=167.19 A, xy=0.2lx, xz=0.1lx, yz=-0.15ly), all-pair RDF with r_cut = 20 A,
@@ -438,7 +441,7 @@ def run_gpu(args):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        step()
+        last = step()
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
@@ -447,6 +450,9 @@ def run_gpu(args):
     pair_ms, pair_n = ctx.timing_read(0)
     prep_ms, _ = ctx.timing_read(1)
     ctx.timing(False)
+    if args.dump_outputs and rank == 0:
+        dump_output(args.dump_outputs, "rdf_counts", last.cpu().numpy())
+    del last
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -1156,6 +1162,7 @@ def bench_c1(torch):
     from mdproptools_b200.structural import rdf_cn
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "tests", "golden_large", "c1_frames.tar.gz")
     if not os.path.exists(path):
+        sys.stderr.write("c1 leg skipped: tests/golden_large/c1_frames.tar.gz is absent (oracle/make_c1_fixture.py)\n")
         return None
     d = tempfile.mkdtemp(prefix="mdp_c1_")
     try:
@@ -1300,10 +1307,41 @@ def bench_dump_parse(reps=3, batch=32):
                     "text through pandas.read_csv + sort_values at ~24 MB/s (SURVEY 8f)"}
 
 
+DUMP_BYTES_MAX = 64 << 20
+
+
+def dump_output(d, name, arr):
+    """Write `arr` (leading axis = frames) as d/<name>.npy in float64, so that two builds can be compared output for
+    output.  Beyond DUMP_BYTES_MAX a fixed, seeded sample of frames is written instead, with the frame indices in
+    d/<name>_frames.npy."""
+    os.makedirs(d, exist_ok=True)
+    a = np.asarray(arr, dtype=np.float64)
+    idx = os.path.join(d, f"{name}_frames.npy")
+    if os.path.exists(idx):                                        # from an earlier, sampled run into the same DIR
+        os.remove(idx)
+    if a.nbytes > DUMP_BYTES_MAX:
+        k = (DUMP_BYTES_MAX - 4096) // (a[0].nbytes + 8)         # a frame and its index; 4 KB for the two .npy headers
+        keep = np.sort(np.random.default_rng(SEED).choice(len(a), k, replace=False))
+        np.save(idx, keep.astype(np.float64))
+        a = a[keep]
+    np.save(os.path.join(d, f"{name}.npy"), a)
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=8)
+    ap.add_argument("--steps", type=positive_int, default=8, help="timed steps of the headline RDF loop (passes of the hot path over all frames); the "
+                    "secondary legs set their own counts from it (end to end: 3..6, MSD: at least 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the per-frame integer RDF histograms of the last step [frames, 2, bins] "
+                         "(g_full and the 1-1 relation, 2 per pair as the reference counts) as DIR/rdf_counts.npy, float64")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--port-only", action="store_true", help="reference arm: time only the C port (skip the installed reference)")
@@ -1327,6 +1365,8 @@ def main():
     ap.add_argument("--c5-frames", type=int, default=5000)
     ap.add_argument("--skip-clusters", action="store_true")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's histograms; the reference arm times samples and has none")
     # stdout carries exactly one JSON line (rank 0): anything a library prints there while the bench runs (NCCL's
     # version banner, for one) is sent to stderr instead
     sys.stdout.flush()

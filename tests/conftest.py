@@ -31,10 +31,11 @@ def sample_dir(tmp_path_factory):
 @pytest.fixture(scope="session")
 def c1_dir(tmp_path_factory):
     """config C1 at full length: all 101 frames of the reference's data/mg_tfsi_dme, columns id type x y z xu yu zu
-    (oracle/make_c1_fixture.py; 24 MB, git-ignored, travels to the GPU box with the snapshot)"""
+    (oracle/make_c1_fixture.py; 24 MB, too large to commit, so git-ignored and absent from a fresh clone)"""
     path = os.path.join(ROOT, "tests", "golden_large", "c1_frames.tar.gz")
     if not os.path.exists(path):
-        pytest.skip("tests/golden_large/c1_frames.tar.gz is absent (python oracle/make_c1_fixture.py builds it from /root/reference)")
+        pytest.skip("tests/golden_large/c1_frames.tar.gz is absent (oracle/make_c1_fixture.py builds it from a checkout of the "
+                    "reference project named by MDPROP_REFERENCE_ROOT)")
     d = tmp_path_factory.mktemp("c1_frames")
     with tarfile.open(path) as tf:
         tf.extractall(d)

@@ -39,7 +39,13 @@ def test_product_never_imports_the_oracle():
 def test_no_cuda_means_loud_failure():
     import torch
     if torch.cuda.is_available():
-        pytest.skip("GPU present")
+        # the same check in a process that sees no device
+        code = ("import pytest\nfrom mdproptools_b200._lib import Context, MdpropError\n"
+                "with pytest.raises(MdpropError, match='no CPU fallback'):\n    Context.get()\n")
+        r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env={**os.environ, "CUDA_VISIBLE_DEVICES": ""},
+                           capture_output=True, text=True, timeout=300)
+        assert r.returncode == 0, r.stderr[-2000:]
+        return
     from mdproptools_b200._lib import Context, MdpropError
     with pytest.raises(MdpropError, match="no CPU fallback"):
         Context.get()
