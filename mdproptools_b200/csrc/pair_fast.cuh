@@ -10,6 +10,8 @@
 //      values are small -- |j_rel| <= half extent + r_cut -- and carry an absolute error of ~1e-6 A);
 //   2. evaluates d^2 in fp32 (3 FADD + FMUL + 2 FFMA), x = sqrt(d^2) * 2^s / ddr with MUFU.SQRT and one FFMA.RM that
 //      also floors (2^23 trick), so that one integer Y = floor(x * 2^s) + 1 holds the bin (Y >> s) and s fraction bits;
+//      the FP32 operations run two candidates at a time as packed FP32x2 instructions (FADD2, FMUL2, FFMA2), each half
+//      rounded exactly as the scalar operation, so nothing below depends on the packing;
 //   3. increments histogram word (Y >> s) unconditionally (misses are clamped to a per-lane scratch word behind the row,
 //      as in k_pair), and flags the pair as UNDECIDED when the fraction bits are all zero or all one, i.e. when x is
 //      within 2^-s of a bin edge.  s is chosen per unit from a rigorous bound E on |x_fp32 - x_exact| (below) such that
@@ -46,7 +48,8 @@ constexpr int FAST_CTAS_PER_SM = MDP_FAST_CTAS;
 #define MDP_FAST_UNROLL 4
 #endif
 constexpr int FU = MDP_FAST_UNROLL;           // candidates per round of the pair loop (ring runs are padded to a multiple of it)
-constexpr int FRING = 64;                     // candidate ring: float4 entries per warp
+static_assert(FU % 2 == 0, "the pair loop evaluates candidates two at a time");
+constexpr int FRING = 64;                     // candidate ring: 16-byte entries per warp
 constexpr int FQ_CAP = 64;                    // undecided-pair queue: entries per warp
 constexpr unsigned FMAGIC_BITS = 0x4b400000u; // bits of 12582912.0f = 1.5 * 2^23
 constexpr float FAST_PAD = 1.0e18f;           // coordinate of a padding candidate: d^2 = 1e36 stays finite, bin clamps to a miss
@@ -128,7 +131,8 @@ __device__ __forceinline__ float mixed_axis_lb(float a, float e, float l_dn, flo
 }
 
 // ---- shared-memory layout ----------------------------------------------------------------------------------------------
-// per warp:  ring   float4[FRING]        candidates (x, y, z relative to the group centre, w = sorted j position [<< 6 | class])
+// per warp:  ring   float[FRING][4]      candidates (x, y, z relative to the group centre, w = sorted j position [<< 6 | class]),
+//                                        interleaved in pairs (ring_put)
 //            xq     uint2[FQ_CAP]        undecided pairs: (w of the candidate, lane << 16 | bin already incremented)
 //            jst    double2[2][64]       two staged j chunks (1 KB each, filled by cp.async one chunk ahead of their use)
 //            gs     double[3][3]         g - S for the three uniform image classes of each axis (0: none, 1: j + l, 2: j - l);
@@ -154,6 +158,33 @@ struct FastShared {
     unsigned *hist;
     const unsigned *cptab;       // MULTICLS: byte offset of the histogram row of class pair (ci * nclsB + cj)
 };
+
+// The candidate ring is interleaved in pairs: candidate c is half (c & 1) of the 32-byte block c >> 1, laid out
+// {x0, x1, y0, y1}{z0, z1, w0, w1}.  Two LDS.128 then hand the pair loop each coordinate of two candidates as one register
+// pair, the operand of the packed FP32x2 instructions (one float4 per candidate would need a MOV per coordinate to pair
+// them).  These three functions are the only code that knows the layout.
+__device__ __forceinline__ void ring_put(float *ring, int c, float x, float y, float z, unsigned w)
+{
+    float *e = ring + (c >> 1) * 8 + (c & 1);
+    e[0] = x;
+    e[2] = y;
+    e[4] = z;
+    e[6] = __uint_as_float(w);
+}
+
+// candidates c and c + 1 (c even) of the run at shared address ja
+__device__ __forceinline__ void ring_get2(unsigned ja, int c, float2 &x, float2 &y, float2 &z, uint2 &w)
+{
+    const unsigned a = ja + (unsigned)(c >> 1) * 32u;
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(x.x), "=f"(x.y), "=f"(y.x), "=f"(y.y) : "r"(a));
+    asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=f"(z.x), "=f"(z.y), "=r"(w.x), "=r"(w.y) : "r"(a + 16u));
+}
+
+// shared address of the w of candidate c of the run at ja
+__device__ __forceinline__ unsigned ring_w_addr(unsigned ja, int c)
+{
+    return ja + (unsigned)(c >> 1) * 32u + 24u + (unsigned)(c & 1) * 4u;
+}
 
 __device__ __forceinline__ void pf_mbar_init(unsigned bar, unsigned count)
 {
@@ -285,44 +316,54 @@ __device__ __forceinline__ void fast_run(const FastRunP &R, const FastExact &ex,
                                          const float l32x, const float l32y, const float l32z, const int lane, int &qn, uint2 *xq,
                                          unsigned &uex)
 {
-    const float inv_s = R.inv_s, xi = R.xi, yi = R.yi, zi = R.zi;
+    const float2 xi = make_float2(R.xi, R.xi), yi = make_float2(R.yi, R.yi), zi = make_float2(R.zi, R.zi);
+    const float2 inv_s = make_float2(R.inv_s, R.inv_s), magic = make_float2(12582913.0f, 12582913.0f);
     const unsigned mask = R.mask, clampv = R.clampv, base = R.base;
     const int s = R.s;
+    const auto wrap = [](float d, float l) { return fminf(fabsf(d), fabsf(fabsf(d) - l)); };
 #pragma unroll 1
     for (int j0 = 0; j0 < nj; j0 += FU) {
         unsigned b[FU];
         bool unc = false;
-        float jx[FU], jy[FU], jz[FU];
-        unsigned jm[FU];
-        // the four candidates first (back-to-back loads, nothing depends on the previous one), then the arithmetic
+        float2 jx[FU / 2], jy[FU / 2], jz[FU / 2];
+        uint2 jm[FU / 2];
+        // all candidates of the round first (back-to-back loads, nothing depends on the previous one), then the arithmetic
 #pragma unroll
-        for (int u = 0; u < FU; ++u)
-            asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];"
-                         : "=f"(jx[u]), "=f"(jy[u]), "=f"(jz[u]), "=r"(jm[u])
-                         : "r"(ja + (unsigned)(j0 + u) * 16u));
+        for (int k = 0; k < FU / 2; ++k) ring_get2(ja, j0 + 2 * k, jx[k], jy[k], jz[k], jm[k]);
+        // candidates 2k and 2k + 1 share every FP32 instruction; each half is the scalar operation with its rounding, so Y,
+        // the histogram word and the undecided flag of every pair are what scalar code computes
 #pragma unroll
-        for (int u = 0; u < FU; ++u) {
-            float dx = xi - jx[u], dy = yi - jy[u], dz = zi - jz[u];
+        for (int k = 0; k < FU / 2; ++k) {
+            float2 dx = __fadd2_rn(xi, make_float2(-jx[k].x, -jx[k].y)), dy = __fadd2_rn(yi, make_float2(-jy[k].x, -jy[k].y)),
+                   dz = __fadd2_rn(zi, make_float2(-jz[k].x, -jz[k].y));
             if (MIXED) {
-                dx = fminf(fabsf(dx), fabsf(fabsf(dx) - l32x));
-                dy = fminf(fabsf(dy), fabsf(fabsf(dy) - l32y));
-                dz = fminf(fabsf(dz), fabsf(fabsf(dz) - l32z));
+                dx = make_float2(wrap(dx.x, l32x), wrap(dx.y, l32x));
+                dy = make_float2(wrap(dy.x, l32y), wrap(dy.y, l32y));
+                dz = make_float2(wrap(dz.x, l32z), wrap(dz.y, l32z));
             }
-            float r2 = __fmaf_rn(dz, dz, __fmaf_rn(dy, dy, dx * dx));
-            if (TRI) r2 = (j0 + u > lane) ? r2 : 1.0e36f;
-            float sq;
-            asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(sq) : "f"(r2));
-            unsigned v = __float_as_uint(__fmaf_rd(sq, inv_s, 12582913.0f));   // FMAGIC_BITS + floor(x * 2^s) + 1
-            v = v < clampv ? v : clampv;
-            b[u] = v;
-            unc = unc || ((v & mask) == 0u);
+            float2 r2 = __ffma2_rn(dz, dz, __ffma2_rn(dy, dy, __fmul2_rn(dx, dx)));
+            if (TRI) {
+                r2.x = (j0 + 2 * k > lane) ? r2.x : 1.0e36f;
+                r2.y = (j0 + 2 * k + 1 > lane) ? r2.y : 1.0e36f;
+            }
+            float2 sq;
+            asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(sq.x) : "f"(r2.x));
+            asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(sq.y) : "f"(r2.y));
+            const float2 y = __ffma2_rd(sq, inv_s, magic);   // FMAGIC_BITS + floor(x * 2^s) + 1
+            unsigned v0 = __float_as_uint(y.x), v1 = __float_as_uint(y.y);
+            v0 = v0 < clampv ? v0 : clampv;
+            v1 = v1 < clampv ? v1 : clampv;
+            b[2 * k] = v0;
+            b[2 * k + 1] = v1;
+            unc = unc || ((v0 & mask) == 0u) || ((v1 & mask) == 0u);
         }
 #pragma unroll
         for (int u = 0; u < FU; ++u) {
             unsigned a = base + ((b[u] >> s) << 2);
             if (MULTICLS) {
+                const unsigned w = (u & 1) ? jm[u / 2].y : jm[u / 2].x;
                 unsigned row;
-                asm volatile("ld.shared.u32 %0, [%1];" : "=r"(row) : "r"(R.cptab_mi_a + ((jm[u] & 63u) << 2)));
+                asm volatile("ld.shared.u32 %0, [%1];" : "=r"(row) : "r"(R.cptab_mi_a + ((w & 63u) << 2)));
                 a += row;
             }
             asm volatile("red.shared.add.u32 [%0], 1;" ::"r"(a) : "memory");
@@ -332,7 +373,7 @@ __device__ __forceinline__ void fast_run(const FastRunP &R, const FastExact &ex,
 #pragma unroll
             for (int u = 0; u < FU; ++u) {   // unrolled: b[] stays in registers; the candidate's w is re-read from the ring
                 unsigned jm;
-                asm volatile("ld.shared.u32 %0, [%1];" : "=r"(jm) : "r"(ja + (unsigned)(j0 + u) * 16u + 12u));
+                asm volatile("ld.shared.u32 %0, [%1];" : "=r"(jm) : "r"(ring_w_addr(ja, j0 + u)));
                 bool f = (b[u] & mask) == 0u && jm < FAST_PADMETA;
                 if (TRI) f = f && (j0 + u > lane);
                 const unsigned m = __ballot_sync(0xffffffffu, f);
@@ -353,12 +394,12 @@ __device__ __forceinline__ void fast_run(const FastRunP &R, const FastExact &ex,
 
 // the ring holds n pending candidates from `base`: pad to a multiple of FU and evaluate them (uniform-image variant)
 template <bool MULTICLS, bool TRICL>
-__device__ __forceinline__ void fast_flush(const FastRunP &R, const FastExact &ex, float4 *ring, unsigned ring_a, int head, int tail,
+__device__ __forceinline__ void fast_flush(const FastRunP &R, const FastExact &ex, float *ring, unsigned ring_a, int head, int tail,
                                            int lane, int &qn, uint2 *xq, unsigned &uex)
 {
     const int n = tail - head;
     const int np = (n + FU - 1) & ~(FU - 1);
-    if (lane < np - n) ring[(tail + lane) & (FRING - 1)] = make_float4(FAST_PAD, 0.f, 0.f, __uint_as_float(FAST_PADMETA));
+    if (lane < np - n) ring_put(ring, (tail + lane) & (FRING - 1), FAST_PAD, 0.f, 0.f, FAST_PADMETA);
     __syncwarp();
     fast_run<MULTICLS, TRICL, false, false>(R, ex, ring_a + (unsigned)(head & 32) * 16u, np, 0.f, 0.f, 0.f, lane, qn, xq, uex);
     __syncwarp();
@@ -369,22 +410,22 @@ __device__ __forceinline__ void fast_flush(const FastRunP &R, const FastExact &e
 // (jx, jy, jz) = my j point relative to the centre, unshifted when `mixed`.  Returns the 32-pair steps evaluated.
 template <bool MULTICLS, bool TRICL>
 __device__ __forceinline__ unsigned fast_special(int f_smax, float inv_ddr, const FastRunP &R, const FastExact &ex, const FrameConst *fc,
-                                                 float4 *ring, unsigned ring_a, float jx, float jy, float jz, unsigned jmeta, bool self,
+                                                 float *ring, unsigned ring_a, float jx, float jy, float jz, unsigned jmeta, bool self,
                                                  bool mixed, float extx, float exty, float extz, float rc2t, float e15m,
                                                  unsigned hist_a, int lane, int &qn, uint2 *xq, unsigned &uex)
 {
     int n = 32;
     if (self) {
-        ring[lane] = make_float4(jx, jy, jz, __uint_as_float(jmeta));
+        ring_put(ring, lane, jx, jy, jz, jmeta);
     } else {
         const float bx = mixed_axis_lb(fabsf(jx), extx, fc->ax[0][0], fc->ax[0][1]), by = mixed_axis_lb(fabsf(jy), exty, fc->ax[1][0], fc->ax[1][1]),
                     bz = mixed_axis_lb(fabsf(jz), extz, fc->ax[2][0], fc->ax[2][1]);
         const bool ok = __fmaf_rn(bz, bz, __fmaf_rn(by, by, bx * bx)) < rc2t && jmeta < FAST_PADMETA;
         const unsigned m = __ballot_sync(0xffffffffu, ok);
-        if (ok) ring[__popc(m & ((1u << lane) - 1u))] = make_float4(jx, jy, jz, __uint_as_float(jmeta));
+        if (ok) ring_put(ring, __popc(m & ((1u << lane) - 1u)), jx, jy, jz, jmeta);
         const int c = __popc(m);
         n = (c + FU - 1) & ~(FU - 1);
-        if (lane < n - c) ring[c + lane] = make_float4(FAST_PAD, 0.f, 0.f, __uint_as_float(FAST_PADMETA));
+        if (lane < n - c) ring_put(ring, c + lane, FAST_PAD, 0.f, 0.f, FAST_PADMETA);
     }
     __syncwarp();
     if (n > 0) {
@@ -414,7 +455,7 @@ __global__ void __launch_bounds__(NWARP * 32, NCTA) k_pair_fast(const PairParams
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     unsigned char *wp = smem_raw + (size_t)(threadIdx.x >> 5) * FAST_WARP_BYTES;
-    float4 *ring = reinterpret_cast<float4 *>(wp + FW_RING);
+    float *ring = reinterpret_cast<float *>(wp + FW_RING);
     uint2 *xq = reinterpret_cast<uint2 *>(wp + FW_XQ);
     double *gs = reinterpret_cast<double *>(wp + FW_GS);
     float4 *gas = reinterpret_cast<float4 *>(wp + FW_GA);
@@ -688,7 +729,7 @@ __global__ void __launch_bounds__(NWARP * 32, NCTA) k_pair_fast(const PairParams
                         const float bx = fmaxf(fabsf(jx) - extx, 0.f), by = fmaxf(fabsf(jy) - exty, 0.f), bz = fmaxf(fabsf(jz) - extz, 0.f);
                         const bool ok = __fmaf_rn(bz, bz, __fmaf_rn(by, by, bx * bx)) < rc2t && !jpad;
                         const unsigned m = __ballot_sync(0xffffffffu, ok);
-                        if (ok) ring[(tail + __popc(m & ((1u << lane) - 1u))) & (FRING - 1)] = make_float4(jx, jy, jz, __uint_as_float(jmeta));
+                        if (ok) ring_put(ring, (tail + __popc(m & ((1u << lane) - 1u))) & (FRING - 1), jx, jy, jz, jmeta);
                         tail += __popc(m);
                         if (tail - head >= 32) {
                             __syncwarp();
