@@ -37,7 +37,8 @@ int mdp_version(void);
 const char *mdp_last_error(void);
 int mdp_ctx_create(int device, mdp_ctx **out);
 void mdp_ctx_destroy(mdp_ctx *ctx);
-/* bytes of scratch currently held / upper bound the context may grow to (default 8 GiB) */
+/* bytes of scratch currently held / upper bound the context may grow to (default 8 GiB); the pair engine and the FFT
+ * correlation split their work (frames, channels) into batches that fit it */
 int64_t mdp_ctx_scratch_bytes(mdp_ctx *ctx);
 int mdp_ctx_set_scratch_limit(mdp_ctx *ctx, int64_t bytes);
 /* counters: number of kernels this library launched since creation (bench.py's gpu_launches) */

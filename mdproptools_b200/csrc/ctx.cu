@@ -2,6 +2,7 @@
 #include <stdarg.h>
 
 #include "common.cuh"
+#include "scratch_plan.h"
 
 static thread_local char g_err[1024] = "";
 
@@ -15,7 +16,7 @@ void mdp_set_error(const char *fmt, ...)
 
 int mdp_ctx::arena_reserve(size_t bytes)
 {
-    bytes = align256(bytes) + 4096;
+    bytes = mdp_scratch_reserved(bytes);   // batch sizes are planned on this same total (scratch_plan.h)
     if (bytes <= slab_bytes) return 0;
     if (bytes > slab_limit) {
         mdp_set_error("scratch request %zu B exceeds the context limit %zu B", bytes, slab_limit);

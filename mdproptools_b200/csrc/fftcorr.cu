@@ -12,6 +12,7 @@
 
 #include "common.cuh"
 #include "fft_corr.h"
+#include "scratch_plan.h"
 
 namespace {
 
@@ -100,10 +101,12 @@ int mdp_xcorr_fft(mdp_ctx *ctx, int nchan, int64_t T, const double *a, const dou
     const long long n = 1ll << p;
     const size_t per_chan = (size_t)n * sizeof(mdp_c64);
     const size_t wbytes = align256((size_t)(n / 2) * sizeof(mdp_c64));
-    // two work arrays per channel of the group; groups sized to 2 GiB of scratch (at least one channel)
+    // two work arrays per channel of the group; groups sized to 2 GiB of scratch (at least one channel), on the whole
+    // request and what arena_reserve adds to it (scratch_plan.h)
     const size_t budget = std::min<size_t>(ctx->slab_limit, (size_t)2 << 30);
-    const int group = (int)std::max<size_t>(1, std::min<size_t>((size_t)std::min(nchan, 65535), (budget - std::min(budget, wbytes)) / (2 * per_chan)));
-    int rc = ctx->arena_reserve(wbytes + 2 * align256((size_t)group * per_chan) + 4096);
+    const size_t fixed_req = wbytes + 4096, per_chan_req = 2 * align256(per_chan);
+    const int group = (int)mdp_scratch_units(budget, fixed_req, per_chan_req, (size_t)std::min(nchan, 65535));
+    int rc = ctx->arena_reserve(fixed_req + (size_t)group * per_chan_req);
     if (rc) return rc;
     ctx->arena_reset();
     mdp_c64 *W = (mdp_c64 *)ctx->arena_take((size_t)(n / 2) * sizeof(mdp_c64));

@@ -34,6 +34,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "scratch_plan.h"
 
 namespace {
 
@@ -1598,10 +1599,12 @@ static int run_pair_call(mdp_ctx *ctx, const PairCall &c, cudaStream_t st)
                              2 * align256((size_t)A.ntiles * 4) + 64 + 4;
     const size_t fixed = align256((size_t)(c.nbins + 2) * sizeof(double2)) + align256(MAX_CLS * MAX_CLS * 4) + 8192;
     const size_t target = std::min<size_t>(ctx->slab_limit, (size_t)3 << 29);   // 1.5 GiB working set
-    int Fsub = (int)std::max<size_t>(1, std::min<size_t>((size_t)c.nframes, (target - std::min(target, fixed)) / per_frame));
-    Fsub = std::min(Fsub, 1 << 19);
+    // the request is the fixed part + 64 KB of headroom + per frame its scratch and its box (48 B); Fsub is sized on all
+    // of it, and on what arena_reserve adds, so that a limit Fsub frames fit in is never exceeded (scratch_plan.h)
+    const size_t fixed_req = fixed + 65536, per_frame_req = per_frame + 48;
+    const int Fsub = (int)mdp_scratch_units(target, fixed_req, per_frame_req, (size_t)std::min(c.nframes, 1 << 19));
     MDP_REQUIRE((size_t)Fsub * items_worst < ((size_t)1 << 32), "pair: work list too long");
-    int rc = ctx->arena_reserve(fixed + (size_t)Fsub * per_frame + (size_t)Fsub * 48 + 65536);
+    int rc = ctx->arena_reserve(fixed_req + (size_t)Fsub * per_frame_req);
     if (rc) return rc;
 
     // edge pairs / class-pair table (host side staging)

@@ -424,6 +424,53 @@ def test_fft_correlation_on_host(tmp_path):
     assert worst < 1e-12
 
 
+def test_scratch_plan_on_host(tmp_path):
+    """The batch planner of the pair engine (frames per sub-batch) and the FFT correlation (channels per group),
+    csrc/scratch_plan.h, against arena_reserve's own test -- round the request up to 256 bytes, add 4096, refuse it above
+    the limit -- restated here: over random sizes and over limits swept through the windows just above each multiple
+    of the unit, the request of the planned count passes whenever one unit does, one unit more would not pass (or the
+    count is at its cap), and the count never decreases as the limit grows."""
+    import ctypes
+    so = tmp_path / "scratch_plan_host.so"
+    src = os.path.join(ROOT, "tests", "native", "scratch_plan_host.cpp")
+    subprocess.run(["g++", "-O1", "-std=c++17", "-shared", "-fPIC", "-o", str(so), src], check=True)
+    lib = ctypes.CDLL(str(so))
+    U = ctypes.c_ulonglong
+    for fn, nargs in ((lib.plan_units, 4), (lib.plan_reserved, 1)):
+        fn.restype = U
+        fn.argtypes = [U] * nargs
+
+    def reserved(b):                        # mdp_ctx::arena_reserve (csrc/ctx.cu)
+        return (b + 255) // 256 * 256 + 4096
+
+    def fits(limit, fixed, per, n):
+        return reserved(fixed + n * per) <= limit
+
+    rng = np.random.default_rng(17)
+    for b in list(rng.integers(0, 1 << 40, 2000)) + list(range(0, 1025)):
+        assert lib.plan_reserved(int(b)) == reserved(int(b))
+    for _ in range(400):
+        fixed = int(rng.choice([0, int(rng.integers(0, 1 << 16)), int(rng.integers(0, 1 << 26))]))
+        per = int(rng.choice([1, int(rng.integers(1, 512)), int(rng.integers(1, 1 << 20)), int(rng.integers(1, 1 << 28))]))
+        cap = int(rng.choice([1, int(rng.integers(1, 20)), 1 << 19, 65535]))
+        # limits around where 1..cap+1 units start to fit, from below the first unit to past the cap
+        marks = [fixed + k * per for k in range(0, min(cap, 40) + 2)] + [fixed + cap * per, fixed + (cap + 1) * per]
+        limits = set(int(x) for x in rng.integers(0, 2 * marks[-1] + 8192, 50))
+        for m in marks:
+            limits.update(max(0, m + d) for d in (-1, 0, 1, 255, 256, 4095, 4096, 4097, 4352, 4353, 8192, 70000))
+        prev = 0
+        for limit in sorted(limits):
+            n = lib.plan_units(limit, fixed, per, cap)
+            assert 1 <= n <= cap, (limit, fixed, per, cap, n)
+            if fits(limit, fixed, per, 1):
+                assert fits(limit, fixed, per, n), (limit, fixed, per, cap, n)
+                assert n == cap or not fits(limit, fixed, per, n + 1), (limit, fixed, per, cap, n)
+            else:
+                assert n == 1, (limit, fixed, per, cap, n)
+            assert n >= prev, (limit, fixed, per, cap, prev, n)
+            prev = n
+
+
 def test_parser_multiframe_triclinic_and_ragged(tmp_path):
     from mdproptools_b200.io import dump as D
     rng = np.random.default_rng(0)
