@@ -106,13 +106,12 @@ int mdp_pair_hist(mdp_ctx *ctx, int nframes,
  * the smallest cell width and |xy|,|xz| <= lx/2, |yz| <= ly/2.  Definition and checker: oracle/oracle.c
  * pair_rsq_tri (parity unpinned by the reference). */
 #define MDP_PAIR_TRICLINIC 4
-/* Uniform-bin histograms: compact the hits into the per-warp queue before binning (the pre-direct-binning path;
- * kept for A/B measurements and as the fallback when the edge table does not fit in shared memory). */
-#define MDP_PAIR_QUEUE_BINNING 8
 /* Uniform-bin histograms are served by the fp32-filtered kernel (csrc/pair_fast.cuh: fp32 distance and bin, every pair
  * within the proven error bound of a bin edge re-evaluated by the reference's fp64 arithmetic; counts identical).  This
  * flag (or the environment variable MDP_PAIR_F64) selects the all-fp64 kernel instead, for A/B measurements and tests. */
 #define MDP_PAIR_F64 16
+/* mdp_pair_hist and mdp_pair_list return MDP_ERR_ARG for any other flag bit (8 selected a binning variant of the
+ * all-fp64 kernel in earlier versions). */
 
 /*
  * out[f][r][b] = sum_rows weights[r][row] * hist[f][row][b]     (all integer)

@@ -86,7 +86,7 @@ _PROTOS = {
 
 EXPORTED_SYMBOLS = tuple(_PROTOS)
 
-PAIR_NO_CULL, PAIR_NO_SORT, PAIR_TRICLINIC, PAIR_QUEUE_BINNING, PAIR_F64 = 1, 2, 4, 8, 16   # flags of mdp_pair_hist / mdp_pair_list
+PAIR_NO_CULL, PAIR_NO_SORT, PAIR_TRICLINIC, PAIR_F64 = 1, 2, 4, 16   # flags of mdp_pair_hist / mdp_pair_list
 
 
 def lib() -> ctypes.CDLL:

@@ -55,7 +55,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     if not force and not needs_build():
         return LIB
     nvcc, cxx = _nvcc(), _host_cxx()
-    extra = os.environ.get("MDP_NVCC_EXTRA", "").split()          # e.g. -DMDP_FAST_CTAS=2 for A/B builds
+    extra = os.environ.get("MDP_NVCC_EXTRA", "").split()          # e.g. -DMDP_FAST_UNROLL=8 for A/B builds
     objdir = os.path.join(HERE, "build")
     os.makedirs(objdir, exist_ok=True)
     objs = []

@@ -20,10 +20,10 @@
 //        k_pair_fast (pair_fast.cuh, the default for uniform bins): distances and bins in fp32 relative to the group
 //          centre, every pair within a proven error bound of a bin edge re-evaluated in the reference's fp64 arithmetic
 //          and corrected -- counts identical to the reference's, 1.6x faster than the all-fp64 kernel;
-//        k_pair (this file): the reference's unfused fp64 chain for every evaluated pair (8-14 FP64-pipe ops), direct
-//          binning (fp32 estimate + one exact fp64 edge compare) or the hit queue.  It serves table bins (coordination
-//          numbers), the neighbour list (clusters, hydration, residence searches), MDP_PAIR_F64 and every shape the fast
-//          kernel declines.
+//        k_pair (this file): the reference's unfused fp64 chain for every evaluated pair (8-14 FP64-pipe ops); the hits
+//          are compacted into a per-warp queue and binned from there (uniform bins: fp32 estimate + one exact fp64 edge
+//          pair).  It serves table bins (coordination numbers), the neighbour list (clusters, hydration, residence
+//          searches), MDP_PAIR_F64, MDP_PAIR_NO_CULL and every shape the fast kernel declines.
 //      The per-CTA uint32 histogram is flushed to the per-frame uint64 global histogram when the CTA leaves a frame (the
 //      only barrier) and whenever the CTA has evaluated 2^30 pairs since the last flush (overflow guard).
 #include <float.h>
@@ -52,19 +52,13 @@ constexpr int CTAS_PER_SM = 2;   // resident CTAs of the pair kernel per SM (reg
 // so that one 32-point chunk is a single contiguous 1 KB block and both halves are bank-conflict free.
 constexpr int GREC = 64;       // double2 per group
 constexpr int RING = 64;       // candidate ring of the pair kernel: entries per warp
-// Scratch words behind the shared histogram: single-row direct binning sends a miss of lane l to word nbins + l, PLUS ONE
-// when rsq >= edge[k + 1] -- which holds for the +inf padding points of a partial chunk against the +inf tail of the edge
-// table.  Lane 31 then reaches word nbins + 32: 33 words are needed (36 keeps what follows 16-byte aligned).  With 32,
-// that increment landed one word past the allocation: harmless while the total was not at an allocation boundary, an
-// illegal-address fault when it was (found by tests/fuzz/fuzz_pair.py: one class, rectangular sets, 88 bins).
-constexpr int HIST_SCRATCH = 36 * 4;
 __host__ __device__ __forceinline__ int64_t rec_xy(int64_t pos) { return (pos >> 5) * GREC + (pos & 31); }
 __host__ __device__ __forceinline__ int64_t rec_zw(int64_t pos) { return (pos >> 5) * GREC + 32 + (pos & 31); }
 constexpr size_t REC_BYTES = 32;   // bytes per point
 
-// MODE_HIST_DIRECT = uniform bins with the edge table in shared memory: every lane bins its own hits inside the pair loop
-// (no compaction queue); the other modes compact the hits into a per-warp queue first.
-enum { MODE_HIST_UNIFORM = 0, MODE_HIST_TABLE = 1, MODE_LIST = 2, MODE_HIST_DIRECT = 3 };
+enum { MODE_HIST_UNIFORM = 0, MODE_HIST_TABLE = 1, MODE_LIST = 2 };
+// the flag bits mdp_pair_hist and mdp_pair_list accept (include/mdprop_b200.h)
+constexpr int PAIR_FLAGS = MDP_PAIR_NO_CULL | MDP_PAIR_NO_SORT | MDP_PAIR_TRICLINIC | MDP_PAIR_F64;
 
 // ---------------------------------------------------------------------------------------------
 // small device helpers
@@ -726,8 +720,6 @@ struct PairParams {
     float inv_ddr;
     unsigned long long *hist;        // device [F][nrows][nbins]
     int edges_in_smem;
-    float inv_ddr_biased;            // MODE_HIST_DIRECT: inv_ddr * (1 - 2^-18)
-    int pipeline;                    // MODE_HIST_DIRECT: dense hits expected, use the software-pipelined pair loop
     // list mode
     double rin2, rout2;
     int shell_mode, exclude_same;
@@ -750,7 +742,6 @@ struct Shared {
     const double2 *edges_s;          // shared-memory copy of the edge table (valid when edges_in_smem)
     const int *cptab;
     unsigned int *hist;
-    unsigned edges_a, cptab_a, hist_a;   // the same three as 32-bit shared-window addresses (MODE_HIST_DIRECT)
 };
 
 // bytes of the warp-private region: two chunk stages + the hit queue (+ its metadata)
@@ -759,11 +750,8 @@ __host__ __device__ constexpr size_t warp_region_bytes(bool meta)
     return 2 * RING * sizeof(double2) + QCAP * sizeof(double) + (meta ? QCAP * sizeof(uint2) : 0);
 }
 
-// shared-memory bytes of the edge table: nbins + 1 (lo, hi) pairs, or direct binning's nbins + 33 plain edges
-__host__ __device__ constexpr size_t edge_region_bytes(int nbins)
-{
-    return (size_t)(nbins + 1) * 16 > (size_t)(nbins + 34) * 8 ? (size_t)(nbins + 1) * 16 : (size_t)(nbins + 34) * 8;
-}
+// shared-memory bytes of the edge table: nbins + 1 (lo, hi) pairs
+__host__ __device__ constexpr size_t edge_region_bytes(int nbins) { return (size_t)(nbins + 1) * 16; }
 
 template <int MODE, bool MULTICLS>
 __device__ __forceinline__ void drain(const PairParams &p, const Shared &sh, int lane, int m, const double *qr,
@@ -800,7 +788,7 @@ __device__ __forceinline__ void drain(const PairParams &p, const Shared &sh, int
             const double r2 = qr[base + lane];
             if (r2 < p.rcut2) {
                 int k;
-                if (MODE == MODE_HIST_UNIFORM || MODE == MODE_HIST_DIRECT) {
+                if (MODE == MODE_HIST_UNIFORM) {
                     // fp32 estimate of sqrt(rsq)/ddr is within +-1 of the reference bin; the exact fp64
                     // edge pair {e[k], e[k+1]} settles it (see mdp_bin_edges)
                     float s;
@@ -841,13 +829,6 @@ struct Shift {
     double x, y, z, xy, xz, yz;
 };
 
-// explicit shared-window accesses (32-bit addresses: no generic-to-shared conversion inside the pair loop)
-__device__ __forceinline__ void lds_f64x2(double &a, double &b, unsigned addr)
-{
-    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(a), "=d"(b) : "r"(addr));
-}
-__device__ __forceinline__ void lds_f64(double &a, unsigned addr) { asm volatile("ld.shared.f64 %0, [%1];" : "=d"(a) : "r"(addr)); }
-
 // squared minimum-image distance of one pair from the raw differences (ax, ay, az) = (xi - xj, ...), in the operation
 // order of the reference (rdf_cn.py:50-56) / of oracle.c pair_rsq_tri for the triclinic variants
 template <int VAR>
@@ -880,71 +861,6 @@ __device__ __forceinline__ double image_r2(double ax, double ay, double az, cons
     return __dadd_rn(__dadd_rn(__dmul_rn(ax, ax), __dmul_rn(ay, ay)), __dmul_rn(az, az));
 }
 
-// ---- direct binning (MODE_HIST_DIRECT) ---------------------------------------------------------------------
-struct DirectBin {
-    unsigned nb, kmax, edges_a, hist_a, cptab_a, dummy_a;
-    uint32_t mi;
-    float inv;
-};
-
-// rsq of my i point against the 4 queued j points at shared address a0 ((x,y) at a0 + 16u, (z,meta) RING entries later)
-template <bool MULTICLS, int VAR>
-__device__ __forceinline__ void direct_eval4(unsigned a0, double xi, double yi, double zi, const Shift &S, double hx, double hy,
-                                             double hz, double (&r2)[4], int (&cj)[4])
-{
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-        double jx, jy, jz, jm = 0.0;
-        lds_f64x2(jx, jy, a0 + u * 16);   // constant offsets after unrolling: folded into the LDS immediates
-        if (MULTICLS)
-            lds_f64x2(jz, jm, a0 + RING * 16 + u * 16);
-        else
-            lds_f64(jz, a0 + RING * 16 + u * 16);
-        r2[u] = image_r2<VAR>(__dsub_rn(xi, jx), __dsub_rn(yi, jy), __dsub_rn(zi, jz), S, hx, hy, hz);
-        cj[u] = MULTICLS ? __double2loint(jm) : 0;
-    }
-}
-
-// Branch-free binning of 4 pairs per lane: float(rsq) (F2F, toward zero; saturates, so rsq beyond the cutoff and the
-// +inf padding need no test of their own: their estimate is >= nbins and the clamp sends them to the invalid bin) ->
-// MUFU.SQRT -> one FFMA.RM whose multiplier is biased DOWN by 2^-18 (more than the fp32 error of the estimate, less
-// than 0.02 bin for nbins <= 4096) with the 2^23 trick, so that k_est = floor(x') is the reference bin or the one
-// below it -> ONE exact fp64 compare against edge[k_est + 1] (mdp_bin_edges: bin(rsq) >= k <=> rsq >= edge[k]) ->
-// unpredicated shared-memory increment.  Misses never reach a histogram word: ptxas wraps every predicated shared
-// atomic in its own branch region (4 extra instructions and a reconvergence point per pair), so they increment words
-// nobody reads instead -- see the two cases in the body (10 instructions per pair single-row, 13 multi-class).
-template <bool MULTICLS>
-__device__ __forceinline__ void direct_bin4(const DirectBin &db, const double (&r2)[4], const int (&cj)[4])
-{
-    unsigned ha[4];
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-        const float f = __double2float_rz(r2[u]);
-        float sq;
-        asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(sq) : "f"(f));
-        unsigned k = __float_as_uint(__fmaf_rd(sq, db.inv, 12582912.0f)) - 0x4b400000u;   // floor(sq*inv), 2^23 trick
-        k = k < db.kmax ? k : db.kmax;
-        double e1;
-        lds_f64(e1, db.edges_a + k * 8u + 8u);
-        if (MULTICLS) {
-            // kmax = nbins: misses (final bin == nbins) increment a per-lane dummy word behind the histogram
-            k += (r2[u] >= e1) ? 1u : 0u;
-            unsigned row;
-            asm volatile("ld.shared.u32 %0, [%1];" : "=r"(row) : "r"(db.cptab_a + (db.mi + (uint32_t)cj[u]) * 4u));
-            ha[u] = k < db.nb ? db.hist_a + (row * db.nb + k) * 4u : db.dummy_a;
-        } else {
-            // kmax = nbins + lane: the single-row histogram is followed by 32 scratch words and the edge table by 33
-            // +inf entries, so a miss needs no select of its own -- it lands in scratch word nbins + lane (its own bank,
-            // like its edge load), which is never zeroed, read or flushed
-            unsigned a = db.hist_a + k * 4u;
-            a += (r2[u] >= e1) ? 4u : 0u;
-            ha[u] = a;
-        }
-    }
-#pragma unroll
-    for (int u = 0; u < 4; ++u) asm volatile("red.shared.add.u32 [%0], 1;" ::"r"(ha[u]) : "memory");
-}
-
 template <int MODE, bool MULTICLS, int VAR, bool TRI>
 __device__ __forceinline__ void chunk_loop(const PairParams &p, const Shared &sh, const double2 *__restrict__ jb, int nj, double xi,
                                            double yi, double zi, uint32_t mi, const Shift S, int rc_hi,
@@ -952,66 +868,6 @@ __device__ __forceinline__ void chunk_loop(const PairParams &p, const Shared &sh
 {
     const double hx = S.x * 0.5, hy = S.y * 0.5, hz = S.z * 0.5;   // VAR_TMIXED only
     constexpr bool META = MULTICLS || MODE == MODE_LIST;
-    if (MODE == MODE_HIST_DIRECT) {
-        // Direct binning: with point-level culling ~30 % of the evaluated pairs are hits, so compacting them first no
-        // longer pays (direct_bin4).  Two loop shapes: the plain one skips the binning of a 4-step round without any hit
-        // (sparse hits: small cutoffs); the pipelined one (p.pipeline, chosen by the host for dense hits) evaluates the
-        // distances of round n+1 in the same basic block as the binning of round n, so that the FP64 chains and the
-        // ALU/MUFU/LSU chains of the binning fill each other's latency slots.
-        const unsigned ja = (unsigned)__cvta_generic_to_shared(jb);
-        DirectBin db;
-        db.nb = (unsigned)p.nbins;
-        db.inv = p.inv_ddr_biased;
-        db.edges_a = sh.edges_a;
-        db.hist_a = sh.hist_a;
-        db.cptab_a = sh.cptab_a;
-        db.kmax = MULTICLS ? db.nb : db.nb + (unsigned)lane;
-        db.dummy_a = sh.hist_a + (unsigned)(p.nrows * p.nbins + lane) * 4u;
-        db.mi = mi;
-        if (!TRI && p.pipeline) {
-            // ping-pong over two register sets (no copies, nothing evaluated twice): round r+1 is evaluated in the
-            // same basic block as round r is binned
-            const int R = nj >> 2;
-            double r2a[4], r2b[4];
-            int cja[4], cjb[4];
-            direct_eval4<MULTICLS, VAR>(ja, xi, yi, zi, S, hx, hy, hz, r2a, cja);
-            int r = 1;
-#pragma unroll 1
-            for (; r + 1 < R; r += 2) {
-                direct_eval4<MULTICLS, VAR>(ja + (unsigned)r * 64u, xi, yi, zi, S, hx, hy, hz, r2b, cjb);
-                direct_bin4<MULTICLS>(db, r2a, cja);
-                direct_eval4<MULTICLS, VAR>(ja + (unsigned)r * 64u + 64u, xi, yi, zi, S, hx, hy, hz, r2a, cja);
-                direct_bin4<MULTICLS>(db, r2b, cjb);
-            }
-            if (r < R) {
-                direct_eval4<MULTICLS, VAR>(ja + (unsigned)r * 64u, xi, yi, zi, S, hx, hy, hz, r2b, cjb);
-                direct_bin4<MULTICLS>(db, r2a, cja);
-                direct_bin4<MULTICLS>(db, r2b, cjb);
-            } else {
-                direct_bin4<MULTICLS>(db, r2a, cja);
-            }
-            return;
-        }
-#pragma unroll 1
-        for (int j0 = 0; j0 < nj; j0 += 4) {
-            double r2[4];
-            int cj[4];
-            direct_eval4<MULTICLS, VAR>(ja + (unsigned)j0 * 16u, xi, yi, zi, S, hx, hy, hz, r2, cj);
-            bool any = false;
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                bool hit = __double2hiint(r2[u]) <= rc_hi;   // superset of rsq < rcut2; edge[nbins] <= rcut2 settles it
-                if (TRI) {
-                    hit = hit && (j0 + u > lane);
-                    if (!hit) r2[u] = INFINITY;              // the lower triangle of the self chunk never counts
-                }
-                any = any || hit;
-            }
-            if (!__any_sync(0xffffffffu, any)) continue;
-            direct_bin4<MULTICLS>(db, r2, cj);
-        }
-        return;
-    }
     const unsigned lt = (1u << lane) - 1u;
 #pragma unroll 1
     for (int j0 = 0; j0 < nj; j0 += 4) {   // nj is a multiple of 4 (candidate batches are padded with +inf points)
@@ -1120,19 +976,11 @@ __global__ void __launch_bounds__(NWARP * 32, CTAS_PER_SM) k_pair(const PairPara
     sh.hist = reinterpret_cast<unsigned int *>(sp);
     sh.edges_s = edges_s;
     sh.cptab = p.cptab;
-    sh.edges_a = (unsigned)__cvta_generic_to_shared(edges_s);
-    sh.cptab_a = (unsigned)__cvta_generic_to_shared(cptab_s);
-    sh.hist_a = (unsigned)__cvta_generic_to_shared(sh.hist);
 
     const int nhist = MODE == MODE_LIST ? 0 : p.nrows * p.nbins;
     if (MODE != MODE_LIST) {
-        if (MODE == MODE_HIST_DIRECT) {
-            // plain edge table e[0..nbins+32] (+inf beyond e[nbins]) in the space reserved for the edge pairs
-            double *e1 = reinterpret_cast<double *>(edges_s);
-            for (int k = tid; k <= p.nbins + 32; k += blockDim.x) e1[k] = k <= p.nbins ? p.edges2[k].x : INFINITY;
-        } else if (p.edges_in_smem) {
+        if (p.edges_in_smem)
             for (int k = tid; k <= p.nbins; k += blockDim.x) edges_s[k] = p.edges2[k];
-        }
         for (int k = tid; k < nhist; k += blockDim.x) sh.hist[k] = 0u;
     }
     if (MODE != MODE_LIST && tid == 0) *evals_s = 0u;
@@ -1494,37 +1342,26 @@ static int sort_set(mdp_ctx *ctx, SetPlan &s, int F, const double *xyz, const in
 
 typedef void (*pair_kernel_t)(const PairParams);
 
-template <int MODE, bool TRICL>
-static pair_kernel_t pick_kernel2(bool multicls, bool symm)
+template <int MODE, bool MULTICLS>
+static pair_kernel_t pick_kernel2(bool symm, bool tric)
 {
-    if (multicls) return symm ? k_pair<MODE, true, true, TRICL> : k_pair<MODE, true, false, TRICL>;
-    return symm ? k_pair<MODE, false, true, TRICL> : k_pair<MODE, false, false, TRICL>;
+    if (tric) return symm ? k_pair<MODE, MULTICLS, true, true> : k_pair<MODE, MULTICLS, false, true>;
+    return symm ? k_pair<MODE, MULTICLS, true, false> : k_pair<MODE, MULTICLS, false, false>;
 }
 template <int MODE>
 static pair_kernel_t pick_kernel(bool multicls, bool symm, bool tric)
 {
-    return tric ? pick_kernel2<MODE, true>(multicls, symm) : pick_kernel2<MODE, false>(multicls, symm);
+    return multicls ? pick_kernel2<MODE, true>(symm, tric) : pick_kernel2<MODE, false>(symm, tric);
 }
 
-template <int NCTA>
-static pair_kernel_t pick_fast_n(bool multicls, bool symm, bool tric)
-{
-    if (tric) {
-        if (multicls) return symm ? k_pair_fast<true, true, true, NCTA> : k_pair_fast<true, false, true, NCTA>;
-        return symm ? k_pair_fast<false, true, true, NCTA> : k_pair_fast<false, false, true, NCTA>;
-    }
-    if (multicls) return symm ? k_pair_fast<true, true, false, NCTA> : k_pair_fast<true, false, false, NCTA>;
-    return symm ? k_pair_fast<false, true, false, NCTA> : k_pair_fast<false, false, false, NCTA>;
-}
-static int fast_ctas()
-{
-    const char *e = getenv("MDP_FAST_CTAS");   // A/B measurements: resident CTAs per SM the kernel is compiled for
-    const int v = e ? atoi(e) : FAST_CTAS_PER_SM;
-    return v == 2 ? 2 : 3;
-}
 static pair_kernel_t pick_fast(bool multicls, bool symm, bool tric)
 {
-    return fast_ctas() == 2 ? pick_fast_n<2>(multicls, symm, tric) : pick_fast_n<3>(multicls, symm, tric);
+    if (tric) {
+        if (multicls) return symm ? k_pair_fast<true, true, true> : k_pair_fast<true, false, true>;
+        return symm ? k_pair_fast<false, true, true> : k_pair_fast<false, false, true>;
+    }
+    if (multicls) return symm ? k_pair_fast<true, true, false> : k_pair_fast<true, false, false>;
+    return symm ? k_pair_fast<false, true, false> : k_pair_fast<false, false, false>;
 }
 
 struct PairCall {
@@ -1582,15 +1419,15 @@ static int run_pair_call(mdp_ctx *ctx, const PairCall &c, cudaStream_t st)
         const size_t edge_bytes = edge_region_bytes(c.nbins);
         if (multicls) smem += (size_t)((ncp * 4 + 15) & ~15);
         const size_t cap = std::min<size_t>(ctx->smem_optin, (216 / CTAS_PER_SM) * 1024);   // keep CTAS_PER_SM CTAs per SM
-        MDP_REQUIRE(smem + hist_bytes + HIST_SCRATCH + 16 <= ctx->smem_optin,
+        MDP_REQUIRE(smem + hist_bytes + 16 <= ctx->smem_optin,
                     "pair: histogram of %d rows x %d bins does not fit in shared memory (%zu B needed); "
                     "reduce the number of distinct classes or bins per call",
                     nrows, c.nbins, smem + hist_bytes);
-        if (smem + hist_bytes + HIST_SCRATCH + 16 + edge_bytes <= cap) {
+        if (smem + hist_bytes + 16 + edge_bytes <= cap) {
             edges_in_smem = 1;
             smem += edge_bytes;
         }
-        smem += hist_bytes + HIST_SCRATCH + 16;   // + the scratch words direct binning sends misses to + the guard counter
+        smem += hist_bytes + 16;   // + the overflow guard's counter
     }
 
     // sub-batching over frames so that scratch stays bounded
@@ -1630,10 +1467,6 @@ static int run_pair_call(mdp_ctx *ctx, const PairCall &c, cudaStream_t st)
         }
     }
 
-    // direct binning needs the edge pairs in shared memory (entries 0..nbins are read)
-    // and rsq >= rcut2 must imply bin >= nbins (edge[nbins] <= rcut2), which holds whenever nbins = int(r_cut/bin_size)
-    const bool direct = c.mode == MODE_HIST_UNIFORM && edges_in_smem && c.nbins <= 4096 && c.edges[c.nbins] <= c.rcut2 &&
-                        !(c.flags & MDP_PAIR_QUEUE_BINNING);
     // the fp32-filtered kernel (pair_fast.cuh) serves the uniform-bin histograms unless the caller asks for the fp64 one
     int f_smax = 0;
     {
@@ -1644,19 +1477,18 @@ static int run_pair_call(mdp_ctx *ctx, const PairCall &c, cudaStream_t st)
     const size_t fast_smem = NWARP * FAST_WARP_BYTES + ((sizeof(FrameConst) + 15) & ~(size_t)15) +
                              (multicls ? (size_t)((ncp * 4 + 15) & ~15) : 0) + 32 + (size_t)nrows * (c.nbins + FAST_XROW) * 4;
     const bool fast = c.mode == MODE_HIST_UNIFORM && !nocull && c.edges[c.nbins] <= c.rcut2 && f_smax >= 6 &&
-                      !(c.flags & (MDP_PAIR_QUEUE_BINNING | MDP_PAIR_F64)) && Bp.npad < ((int64_t)1 << 22) &&
-                      fast_smem <= ctx->smem_optin && !getenv("MDP_PAIR_F64");
+                      !(c.flags & MDP_PAIR_F64) && Bp.npad < ((int64_t)1 << 22) && fast_smem <= ctx->smem_optin &&
+                      !getenv("MDP_PAIR_F64");
     if (fast) smem = fast_smem;
     pair_kernel_t kern = fast                          ? pick_fast(multicls, symm, tric)
-                         : direct                      ? pick_kernel<MODE_HIST_DIRECT>(multicls, symm, tric)
                          : c.mode == MODE_HIST_UNIFORM ? pick_kernel<MODE_HIST_UNIFORM>(multicls, symm, tric)
-                         : c.mode == MODE_HIST_TABLE ? pick_kernel<MODE_HIST_TABLE>(multicls, symm, tric)
-                                                     : pick_kernel<MODE_LIST>(false, symm, tric);
+                         : c.mode == MODE_HIST_TABLE   ? pick_kernel<MODE_HIST_TABLE>(multicls, symm, tric)
+                                                       : pick_kernel2<MODE_LIST, false>(symm, tric);
     MDP_CUDA(cudaFuncSetAttribute((const void *)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int ctas_per_sm = CTAS_PER_SM;
     if (fast) {
         MDP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, (const void *)kern, NWARP * 32, smem));
-        ctas_per_sm = std::max(1, std::min(ctas_per_sm, fast_ctas()));
+        ctas_per_sm = std::max(1, std::min(ctas_per_sm, FAST_CTAS_PER_SM));
     }
 
     MDP_CUDA(cudaMemsetAsync(ctx->d_stats, 0, 4 * sizeof(unsigned long long), st));
@@ -1747,16 +1579,6 @@ static int run_pair_call(mdp_ctx *ctx, const PairCall &c, cudaStream_t st)
         p.inv_ddr = c.uniform_ddr > 0 ? (float)(1.0 / c.uniform_ddr) : 0.f;
         p.hist = (unsigned long long *)c.hist_out;
         p.edges_in_smem = edges_in_smem;
-        p.inv_ddr_biased = p.inv_ddr * (1.0f - 1.0f / 262144.0f);
-        {
-            // expected share of hits among the evaluated pairs: cutoff sphere / (box of a 32-point group dilated by the cutoff)
-            const double vol = c.box[0] * c.box[1] * c.box[2];
-            const double side = cbrt(32.0 * vol / (double)c.n_a), rc = sqrt(c.rcut2);
-            const double dil = side * side * side + 6.0 * side * side * rc + 3.0 * M_PI * side * rc * rc + 4.0 / 3.0 * M_PI * rc * rc * rc;
-            const double hit_share = vol > 0 ? (4.0 / 3.0 * M_PI * rc * rc * rc) / dil : 0.0;
-            p.pipeline = hit_share > 0.08 ? 1 : 0;
-            if (const char *e = getenv("MDP_PAIR_PIPELINE")) p.pipeline = atoi(e) ? 1 : 0;   // A/B measurements
-        }
         p.rin2 = c.rin2;
         p.rout2 = c.rout2;
         p.shell_mode = c.shell_mode;
@@ -1837,6 +1659,7 @@ int mdp_pair_hist(mdp_ctx *ctx, int nframes, int64_t n_a, const double *xyz_a, c
     MDP_REQUIRE(rcut2 > 0, "mdp_pair_hist: rcut2 must be positive");
     MDP_REQUIRE(uniform_ddr == 0.0 || nbins <= (1 << 18), "mdp_pair_hist: uniform binning limited to 2^18 bins");
     MDP_REQUIRE(uniform_ddr > 0.0 || nbins <= 64, "mdp_pair_hist: table binning limited to 64 thresholds");
+    MDP_REQUIRE((flags & ~PAIR_FLAGS) == 0, "mdp_pair_hist: unknown flag bits 0x%x", flags & ~PAIR_FLAGS);
     PairCall c;
     c.mode = uniform_ddr > 0 ? MODE_HIST_UNIFORM : MODE_HIST_TABLE;
     c.nframes = nframes;
@@ -1868,6 +1691,7 @@ int mdp_pair_list(mdp_ctx *ctx, int nframes, int64_t n_a, const double *xyz_a, i
     MDP_REQUIRE(nframes > 0 && n_a > 0 && n_b > 0 && capacity > 0, "mdp_pair_list: sizes must be positive");
     MDP_REQUIRE(n_a < ((int64_t)1 << 30) && n_b < ((int64_t)1 << 30), "mdp_pair_list: point sets limited to 2^30 points");
     MDP_REQUIRE(rout2 > 0, "mdp_pair_list: rout2 must be positive");
+    MDP_REQUIRE((flags & ~PAIR_FLAGS) == 0, "mdp_pair_list: unknown flag bits 0x%x", flags & ~PAIR_FLAGS);
     PairCall c;
     c.mode = MODE_LIST;
     c.nframes = nframes;

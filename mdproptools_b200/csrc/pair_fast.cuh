@@ -13,9 +13,10 @@
 //      the FP32 operations run two candidates at a time as packed FP32x2 instructions (FADD2, FMUL2, FFMA2), each half
 //      rounded exactly as the scalar operation, so nothing below depends on the packing;
 //   3. increments histogram word (Y >> s) unconditionally (misses are clamped to a per-lane scratch word behind the row,
-//      as in k_pair), and flags the pair as UNDECIDED when the fraction bits are all zero or all one, i.e. when x is
-//      within 2^-s of a bin edge.  s is chosen per unit from a rigorous bound E on |x_fp32 - x_exact| (below) such that
-//      2^-s >= 1.5 E: an unflagged pair is provably in the reference's bin;
+//      one of the FAST_XROW words that are never read, so no increment needs a branch), and flags the pair as UNDECIDED
+//      when the fraction bits are all zero or all one, i.e. when x is within 2^-s of a bin edge.  s is chosen per unit
+//      from a rigorous bound E on |x_fp32 - x_exact| (below) such that 2^-s >= 1.5 E: an unflagged pair is provably in
+//      the reference's bin;
 //   4. undecided pairs (about 1 in 1000) go to a per-warp queue and are settled by the exact path: the reference's own
 //      fp64 arithmetic (image_r2, the code k_pair uses) on the fp64 records, the exact edge table (mdp_bin_edges), and
 //      a correction -1/+1 of the shared histogram when the exact bin differs from the one already incremented.
@@ -40,10 +41,7 @@
 
 namespace {
 
-#ifndef MDP_FAST_CTAS
-#define MDP_FAST_CTAS 3
-#endif
-constexpr int FAST_CTAS_PER_SM = MDP_FAST_CTAS;
+constexpr int FAST_CTAS_PER_SM = 3;           // resident CTAs per SM the kernel is compiled for (80 registers)
 #ifndef MDP_FAST_UNROLL
 #define MDP_FAST_UNROLL 4
 #endif
@@ -449,8 +447,8 @@ __device__ __forceinline__ unsigned fast_special(int f_smax, float inv_ddr, cons
     return (unsigned)n;
 }
 
-template <bool MULTICLS, bool SYMM, bool TRICL, int NCTA>
-__global__ void __launch_bounds__(NWARP * 32, NCTA) k_pair_fast(const PairParams p)
+template <bool MULTICLS, bool SYMM, bool TRICL>
+__global__ void __launch_bounds__(NWARP * 32, FAST_CTAS_PER_SM) k_pair_fast(const PairParams p)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;

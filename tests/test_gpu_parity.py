@@ -73,43 +73,57 @@ def test_pair_hist_symmetric_vs_oracle(ops, n, L, rc, ddr, flags):
     assert int(hist.sum().item()) * 2 == int(full.sum())
 
 
-@pytest.mark.parametrize("n,L,rc,ddr,nb,why", [
-    (2500, (40.0, 38.0, 36.0), 7.3, 0.05, None, "direct binning, r_cut/ddr = 146 exactly representable or not"),
-    (2500, (40.0, 38.0, 36.0), 5.03, 0.1, None, "direct: r_cut/ddr not an integer, edge[nbins] < rcut2 (index nbins dropped)"),
-    (2500, (40.0, 38.0, 36.0), 4.99, 0.1, 50, "edge[nbins] > rcut2: the explicit rsq < rcut2 test is needed -> queue path"),
-    (1500, (30.0, 30.0, 30.0), 6.0, 0.001, None, "6000 bins: edge table too large for direct binning -> queue path"),
-    (1500, (30.0, 30.0, 30.0), 6.0, 6.0, None, "a single bin"),
+@pytest.mark.parametrize("n,L,rc,ddr,nb,ncls,why", [
+    (2500, (40.0, 38.0, 36.0), 7.3, 0.05, None, 2, "r_cut/ddr = 146 exactly representable or not"),
+    (2500, (40.0, 38.0, 36.0), 5.03, 0.1, None, 2, "r_cut/ddr not an integer, edge[nbins] < rcut2 (index nbins dropped)"),
+    (2500, (40.0, 38.0, 36.0), 4.99, 0.1, 50, 2, "edge[nbins] > rcut2: the explicit rsq < rcut2 test is needed, all-fp64 kernel"),
+    (1500, (30.0, 30.0, 30.0), 6.0, 0.001, None, 2, "6000 bins: edge table outside shared memory in the all-fp64 kernel"),
+    (1500, (30.0, 30.0, 30.0), 6.0, 6.0, None, 2, "a single bin"),
+    (2500, (40.0, 38.0, 36.0), 6.0, 1.5, None, 64, "2080 rows x 4 bins: the fp32 kernel's histogram does not fit in shared memory"),
 ])
-def test_pair_hist_binning_paths_agree_with_oracle(ops, n, L, rc, ddr, nb, why):
-    """The uniform-bin histogram has two device paths (per-lane direct binning / compacted queue, MDP_PAIR_QUEUE_BINNING);
-    both must give the reference's bin(rsq) = int64(sqrt(rsq)/ddr) (rdf_cn.py:68,85) for every pair, including the
-    cases where the library has to fall back to the queue path by itself."""
-    from mdproptools_b200._lib import PAIR_QUEUE_BINNING, bin_edges
+def test_pair_hist_binning_paths_agree_with_oracle(ops, n, L, rc, ddr, nb, ncls, why):
+    """The uniform-bin histogram has two device paths, the fp32-filtered kernel (flags 0) and the all-fp64 kernel's hit
+    queue (MDP_PAIR_F64); both must give the reference's bin(rsq) = int64(sqrt(rsq)/ddr) (rdf_cn.py:68,85) for every
+    pair, including the shapes where the library has to fall back to the all-fp64 kernel by itself."""
+    from mdproptools_b200._lib import PAIR_F64, bin_edges
     rng = np.random.default_rng(int(rc * 1000) + n)
-    pos, typ = _rand_box(rng, n, L, 2)
+    pos, typ = _rand_box(rng, n, L, ncls)
     # plant pairs exactly ON bin edges and on the cutoff: x-separated partners at k*ddr and at r_cut
     for k in range(1, 40):
         pos[:, 2 * k] = pos[:, 2 * k + 1]
         pos[0, 2 * k] = pos[0, 2 * k + 1] + (k * ddr if k < 38 else rc)
     nb = int(rc / ddr) if nb is None else nb
-    rel = np.array([[1, 1], [1, 2], [2, 2]])
+    rel = np.array([[1, 1], [1, 2], [2, 2]] + ([[ncls, ncls], [3, ncls - 7]] if ncls > 2 else []))
     full, part = O.rdf_loop(typ, pos[0], pos[1], pos[2], rel, L, rc, ddr, nb, nthreads=0)
     cls = (typ.astype(np.int64) - 1).astype(np.int32)
     edges = bin_edges(ddr, nb)
-    w = [np.full(3, 2)]
+    rows = ops.sym_rows(ncls)
+    w = [np.full(rows, 2)]
     for a, b in rel:
-        r = np.zeros(3, dtype=np.int64)
-        r[ops.sym_row(a - 1, b - 1, 2)] = 2 if a == b else 1
+        r = np.zeros(rows, dtype=np.int64)
+        r[ops.sym_row(a - 1, b - 1, ncls)] = 2 if a == b else 1
         w.append(r)
-    for flags in (0, PAIR_QUEUE_BINNING):
-        for c, ncls in ((cls, 2), (None, 1)):                 # multi-class and single-class kernels
-            hist = ops.pair_hist(_dev(pos[None]), None if c is None else _dev(c), ncls, [L], O.rcut_sq(rc), edges, ddr, flags=flags)
+    for flags in (0, PAIR_F64):
+        for c, nc in ((cls, ncls), (None, 1)):                # multi-class and single-class kernels
+            hist = ops.pair_hist(_dev(pos[None]), None if c is None else _dev(c), nc, [L], O.rcut_sq(rc), edges, ddr, flags=flags)
             if c is None:
                 assert np.array_equal(hist.cpu().numpy()[0, 0] * 2, full), (why, flags)
             else:
                 red = ops.hist_reduce(hist, np.stack(w)).cpu().numpy()[0]
                 assert np.array_equal(red[0], full), (why, flags)
                 assert np.array_equal(red[1:], part), (why, flags)
+
+
+@pytest.mark.parametrize("flags", [8, 32])
+def test_pair_calls_reject_unknown_flags(ops, flags):
+    """Flag bits other than NO_CULL | NO_SORT | TRICLINIC | F64 are an error, not a silent choice of another kernel
+    (8 selected a binning variant of the all-fp64 kernel in earlier versions)."""
+    from mdproptools_b200._lib import MdpropError, bin_edges
+    pos = _dev(np.random.default_rng(5).uniform(0, 10.0, (1, 3, 100)))
+    with pytest.raises(MdpropError, match="unknown flag bits"):
+        ops.pair_hist(pos, None, 1, [(10.0, 10.0, 10.0)], 9.0, bin_edges(0.1, 30), 0.1, flags=flags)
+    with pytest.raises(MdpropError, match="unknown flag bits"):
+        ops.pair_list(pos, pos, [(10.0, 10.0, 10.0)], 0.0, 9.0, 0, flags=flags)
 
 
 def test_pair_hist_multiframe_and_per_frame_boxes(ops):
@@ -1117,7 +1131,7 @@ def test_pair_engine_fuzz_fast_equals_f64():
     """The first 400 cases of tests/fuzz/fuzz_pair.py with seed 1 (random sizes, boxes incl. triclinic, cutoffs, bin widths,
     classes, distributions incl. lattices with thousands of pairs exactly on bin edges, symmetric and rectangular sets):
     k_pair_fast == k_pair bit for bit, every 10th case also == the oracle.  Case 118 of this sequence is the one that
-    found the one-word overrun of the all-fp64 kernel's scratch area (an illegal-address fault before the fix); a 240 s
+    found a one-word overrun in the all-fp64 kernel's (since retired) direct binning; a 240 s
     run of the tool (139 220 cases, 2.3e12 pairs) is recorded in profiles/r02b_fuzz_pair.txt."""
     import importlib.util
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))

@@ -54,7 +54,7 @@ def main(tag):
     # SASS of the headline instantiation
     lib = os.path.join(ROOT, "mdproptools_b200", "libmdprop_b200.so")
     names = [l.split()[-1] for l in run(["cuobjdump", "-elf", lib]).splitlines() if ".text." in l and "k_pair_fast" in l]
-    sym = sorted({n.split(".text.")[-1] for n in names if "ILb0ELb1ELb0ELi3" in n})
+    sym = sorted({n.split(".text.")[-1] for n in names if "ILb0ELb1ELb0EE" in n})
     if sym:
         sass = run(["cuobjdump", "-sass", "-fun", sym[0], lib])
         open(os.path.join(PROF, f"{tag}_k_pair_fast_sass.txt"), "w").write(sass)
@@ -63,13 +63,13 @@ def main(tag):
     bf, b64 = last_json(os.path.join(OUT, "ncu_pair_fast.log")), last_json(os.path.join(OUT, "ncu_pair.log"))
     num = lambda d, k: float(d[k].replace(",", ""))
     meta = {
-        "kernel": "k_pair_fast<0,1,0,3>", "capture": "ncu --set full, bench.py --frames 16 (one launch = 16 C2 frames)", "frames": 16,
+        "kernel": "k_pair_fast<0,1,0>", "capture": "ncu --set full, bench.py --frames 16 (one launch = 16 C2 frames)", "frames": 16,
         "evaluated_pairs": bf["evaluated_pair_evals_per_step"], "inst_executed": num(fast, "smsp__inst_executed.sum"),
         "duration_ms": num(fast, "gpu__time_duration.sum") / (1e6 if num(fast, "gpu__time_duration.sum") > 1e4 else 1),
         "issue_active_pct": round(num(fast, "smsp__issue_active.avg.pct_of_peak_sustained_active"), 2),
         "warp_instr_per_32_pairs": round(num(fast, "smsp__inst_executed.sum") / (bf["evaluated_pair_evals_per_step"] / 32.0), 2),
         "all_fp64_kernel": {
-            "kernel": "k_pair<3,0,1,0>", "evaluated_pairs": b64["evaluated_pair_evals_per_step"],
+            "kernel": "k_pair<0,0,1,0>", "evaluated_pairs": b64["evaluated_pair_evals_per_step"],
             "inst_executed": num(f64, "smsp__inst_executed.sum"),
             "duration_ms": num(f64, "gpu__time_duration.sum") / (1e6 if num(f64, "gpu__time_duration.sum") > 1e4 else 1),
             "warp_instr_per_32_pairs": round(num(f64, "smsp__inst_executed.sum") / (b64["evaluated_pair_evals_per_step"] / 32.0), 2)},

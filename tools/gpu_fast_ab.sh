@@ -8,10 +8,9 @@ mkdir -p $OUT
 FR=${2:-256}
 timeout 900 python -m pytest tests -m gpu -q -p no:cacheprovider --timeout 600 -k "pair or rdf or cn or bin or large or smoke or cluster or hydration or residence" > $OUT/pytest_fast.log 2>&1; echo "pytest rc=$?"
 tail -5 $OUT/pytest_fast.log
-for mode in fast3 fast2 f64; do
-  unset MDP_PAIR_F64 MDP_FAST_CTAS
+for mode in fast f64; do
+  unset MDP_PAIR_F64
   if [ $mode = f64 ]; then export MDP_PAIR_F64=1; fi
-  if [ $mode = fast2 ]; then export MDP_FAST_CTAS=2; fi
   timeout 600 python bench.py --steps 6 --warmup 3 --frames $FR --skip-msd --skip-cpu --skip-gk --skip-residence --skip-clusters > $OUT/bench_ab_$mode.json 2> $OUT/bench_ab_$mode.err; echo "bench $mode rc=$?"
   tail -3 $OUT/bench_ab_$mode.err
   python - <<PY
@@ -25,7 +24,7 @@ except Exception as e:
     print('no bench json', e)
 PY
 done
-unset MDP_PAIR_F64 MDP_FAST_CTAS
+unset MDP_PAIR_F64
 if [ "${1:-}" = "ncu" ]; then
   timeout 900 ncu --set full --clock-control none --import-source on -k regex:k_pair -s 3 -c 1 -f -o $OUT/prof_pair_fast \
       python bench.py --steps 1 --warmup 1 --frames 16 --skip-msd --skip-cpu --skip-gk --skip-residence --skip-clusters --skip-triclinic > $OUT/ncu_pair_fast.log 2>&1
