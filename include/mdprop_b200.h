@@ -46,7 +46,7 @@ int64_t mdp_ctx_launch_count(mdp_ctx *ctx);
 /* optional kernel timing for benchmarks: when enabled, the library brackets its main kernels with CUDA events
  * on the launching stream.  tag 0 = pair kernel (k_pair), 1 = pair preparation (sort, boxes, work list),
  * 2 = streaming MSD kernel, 3 = correlation kernel, 4 = charge-flux kernel, 5 = windowed (all-origins) MSD kernel,
- * 6 = bitmask autocorrelation kernel.  mdp_ctx_timing_read synchronises
+ * 6 = bitmask autocorrelation kernel, 7 = FFT all-origins MSD (the whole of mdp_cross_msd_fft).  mdp_ctx_timing_read synchronises
  * on the recorded events, returns the summed milliseconds and the number of launches, and clears them. */
 int mdp_ctx_timing(mdp_ctx *ctx, int enable);
 int mdp_ctx_timing_read(mdp_ctx *ctx, int tag, double *ms_total, int64_t *count);
@@ -238,6 +238,20 @@ int mdp_xcorr_unbiased(mdp_ctx *ctx, int nchan, int64_t T, const double *a, cons
  * round-off of an FFT (~1e-15 of max|C| times log2 N), which is how the reference computes it.  Same arguments. */
 int mdp_xcorr_fft(mdp_ctx *ctx, int nchan, int64_t T, const double *a, const double *b, int64_t nlags, double *out,
                   void *stream);
+/* All-origins (cross) mean-square displacement of channel groups through the FFT of mdp_xcorr_fft (csrc/msd_fft.h, north-star
+ * extension with no reference implementation; defined by the long-double direct sum of tests/native/cross_msd_direct.c):
+ *   out[g][tau] = sum_{c in group g} (1/(T-tau)) sum_{t < T-tau} (a_c(t+tau) - a_c(t)) * (b_c(t+tau) - b_c(t)),  tau < nlags.
+ * a, b = DEVICE [nchan][T]; b == NULL means b = a (the ordinary MSD summed over the group's channels); group_off = HOST int64
+ * [ngroups+1], non-decreasing from 0 to nchan (contiguous channel groups, empty groups allowed, 1 <= ngroups <= 65535);
+ * 1 <= nlags <= T; out = DEVICE [ngroups][nlags], overwritten.  Each channel's mean is subtracted first (the result does not
+ * change; the cancellation of large offsets goes away).  O(nchan N log N) with N = 2^p >= T + nlags, p <= 30.  Agrees with
+ * the direct long-double sum to 1e-10 of max_tau |out[g]| for T <= 10^5; the bound is absolute, so lags where out is small
+ * next to its maximum (the first lags of a long diffusive series) are covered by it and nothing tighter.  Fixed summation
+ * order, no atomics: run-to-run bit-identical, and the same bits under any scratch limit that admits the call.
+ * MDP_ERR_ARG for bad sizes or group offsets, p > 30, or group accumulators (about ngroups * (4 N + 24 T) bytes) above the
+ * context's scratch limit. */
+int mdp_cross_msd_fft(mdp_ctx *ctx, int nchan, int64_t T, const double *a, const double *b, int ngroups, const int64_t *group_off,
+                      int64_t nlags, double *out, void *stream);
 /* cumulative trapezoid along rows (conductivity.py:231 with leading zero, viscosity.py:151 without):
  * in = DEVICE [nrows][T]; out = DEVICE [nrows][T] if leading_zero else [nrows][T-1]; out = scale*integral. */
 int mdp_cumtrapz(mdp_ctx *ctx, int nrows, int64_t T, const double *in, double dx, double scale,

@@ -67,6 +67,8 @@ _PROTOS = {
                                 POINTER(c_int64), c_int, c_double, c_double, c_void_p, c_int64, c_int64, c_void_p]),
     "mdp_xcorr_unbiased": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "mdp_xcorr_fft": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
+    "mdp_cross_msd_fft": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int, POINTER(c_int64), c_int64, c_void_p,
+                                  c_void_p]),
     "mdp_cumtrapz": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_double, c_double, c_int, c_void_p, c_void_p]),
     "mdp_bitmask_fill": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "mdp_bitmask_autocorr": (c_int, [c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p, c_void_p]),

@@ -8,8 +8,14 @@ J = sum q v, _conductivity.py:7-36) as a streaming segmented reduction over ``[T
 correlations and the cumulative trapezoid (:216-232) (csrc/corr.cu).  ``detect_time_range`` (:116-165) is
 discrete window selection and stays on the host, fed with the device results.
 
-Multi-GPU: frames are split round-robin for the flux stage (all-reduce of the zero-padded J), the
-correlation channels are split over ranks and summed with one fp64 all-reduce.
+Einstein (Helfand) and Nernst-Einstein conductivity (``einstein``, ``nernst``; the reference's methods are empty): the
+translational dipole M = sum q_mol r_com per type is the charge-flux reduction applied to unwrapped positions, and
+both the dipole MSD and the per-type centre-of-mass MSD over all time origins go through the FFT kernel
+mdp_cross_msd_fft (csrc/msdfft.cu).  The straight-line fits (with intercept) run on the host.
+
+Multi-GPU: frames are split round-robin for the flux and dipole stages (all-reduce of the zero-padded J or M), the
+correlation channels (or dipole MSD groups) are split over ranks and summed with one fp64 all-reduce; ``nernst`` parses
+every frame on every rank and shards the molecules of each type.
 """
 from __future__ import annotations
 
@@ -24,6 +30,7 @@ from ..common import constants
 from ..common.com_mols import atom_masses, mol_membership
 from ..io import dump as _dump
 from ..io.pipeline import FrameBatches
+from .diffusion import position_columns, unwrapped_positions
 
 
 class Conductivity:
@@ -231,8 +238,207 @@ class Conductivity:
         fig.savefig(f"{self.working_dir}/conductivity.png", bbox_inches="tight", pad_inches=0.1)
         plt.close(fig)
 
-    def einstein(self):
-        pass
+    # -- Einstein and Nernst-Einstein conductivity ------------------------------------------------------------
+    def _fixed_charge_frames(self, frame_select=None):
+        """Unwrapped positions of every (selected) frame, batch by batch: yields (frame indices, timesteps, pos [F,3,N]
+        device) and returns nothing; afterwards ``self._fixed`` holds (q, type, mass) of the first frame seen (host arrays,
+        None when this rank saw no frame).  Charges, types and masses must not change between frames (the Helfand moment of
+        fluctuating charges is not the integral of the flux): ValueError otherwise, also across ranks."""
+        pattern = f"{self.working_dir}/{self.filename}"
+        cols = _dump.available_columns(pattern)
+        if not cols:
+            raise ValueError(f"no dump frames found for {pattern!r}")
+        pos_cols = position_columns(cols)
+        want = ["id", "type", "q"] + pos_cols
+        if not self.mass:
+            assert "mass" in cols, "Missing atom masses in dump file."
+            want.append("mass")
+        _, _, seg_off = mol_membership(self.num_mols, self.num_atoms_per_mol)
+        self._fixed = None
+        for batch in FrameBatches(pattern, want, frame_select=frame_select):
+            d = batch.wait()
+            host = batch.host.numpy()
+            if seg_off[-1] != host.shape[2]:
+                raise ValueError(f"Length of values ({seg_off[-1]}) does not match length of index ({host.shape[2]})")
+            mcol = None if self.mass else batch.col("mass")
+            if self._fixed is None:
+                q0, t0 = host[0, 2].copy(), host[0, 1].copy()
+                self._fixed = (q0, t0, atom_masses(t0, self.mass) if self.mass else host[0, mcol].copy())
+            q0, t0, m0 = self._fixed
+            if not ((host[:, 2] == q0).all() and (host[:, 1] == t0).all() and (mcol is None or (host[:, mcol] == m0).all())):
+                raise ValueError("charges, types and masses must be the same in every frame for the Einstein and "
+                                 "Nernst-Einstein conductivity")
+            yield ([m.index for m in batch.metas], [m.timestep for m in batch.metas],
+                   unwrapped_positions(d, batch.metas, 3, len(pos_cols) == 3).contiguous())
+        if dist.world_size() > 1:                     # the same charges, types and masses on every rank
+            n = int(seg_off[-1])
+            dev = torch.device("cuda", torch.cuda.current_device())
+            ref = (torch.from_numpy(np.concatenate(self._fixed)).to(dev) if self._fixed is not None
+                   else torch.full((3 * n,), -np.inf, dtype=torch.float64, device=dev))
+            hi = dist.all_reduce_max_(ref.clone())
+            lo = dist.all_reduce_max_(torch.where(torch.isinf(ref), ref, -ref))
+            if not torch.equal(hi, -lo):
+                raise ValueError("charges, types and masses must be the same in every frame for the Einstein and "
+                                 "Nernst-Einstein conductivity")
+            if self._fixed is None:
+                h = hi.cpu().numpy()
+                self._fixed = (h[:n], h[n:2 * n], h[2 * n:])
 
-    def nernst(self):
-        pass
+    def _set_even_time(self, steps):
+        """self.time from the timesteps of all frames (in trajectory order); they must be evenly spaced."""
+        steps = np.asarray(steps, dtype=np.float64)
+        if len(steps) == 0:
+            raise ValueError(f"no dump frames found for {self.working_dir}/{self.filename!r}")
+        d = np.diff(steps)
+        if len(d) and not (d[0] > 0 and (d == d[0]).all()):
+            raise ValueError("the Einstein and Nernst-Einstein conductivity need evenly spaced frames (timesteps "
+                             f"{steps[:3].tolist()}...: spacings {sorted(set(d.tolist()))[:4]})")
+        self.time = (steps * constants.TIME_CONVERSION[self.units] * self.timestep).tolist()
+
+    def get_translational_dipole(self):
+        """M[3, ntypes, T] in C m: per type, the sum over molecules of charge x unwrapped centre of mass (SI).  Positions
+        are ``xu yu zu`` or x + ix (xhi - xlo) (as ``Diffusion``); charges, types and masses must be fixed and the frames
+        evenly spaced (ValueError otherwise).  Sets ``self.time``."""
+        _, _, seg_off = mol_membership(self.num_mols, self.num_atoms_per_mol)
+        ntypes = len(self.num_mols)
+        type_off = np.concatenate(([0], np.cumsum(self.num_mols))).astype(np.int64)
+        w, r = dist.world_size(), dist.rank()
+        dev = torch.device("cuda", torch.cuda.current_device())
+        seg_d = torch.from_numpy(seg_off.astype(np.int32)).to(dev)
+        ds, qs = constants.DISTANCE_CONVERSION[self.units], constants.CHARGE_CONVERSION[self.units]
+        pieces, steps = [], {}
+        frames = self._fixed_charge_frames((lambda i: i % w == r) if w > 1 else None)
+        md = qd = None
+        for idxs, ts, pos in frames:
+            if md is None:
+                md = torch.from_numpy(np.ascontiguousarray(self._fixed[2])).to(dev)
+                qd = torch.from_numpy(np.ascontiguousarray(self._fixed[0])).to(dev)
+            # the charge-flux reduction (csrc/reduce.cu) of positions instead of velocities
+            pieces.append((idxs, ops.charge_flux(pos, md, qd, seg_d, type_off, ds, qs)))
+            steps.update(zip(idxs, ts))
+        T = torch.zeros((1,), dtype=torch.float64, device=dev)
+        T[0] = max(steps) + 1 if steps else 0
+        dist.all_reduce_max_(T)
+        T = int(T.item())
+        if T == 0:
+            raise ValueError(f"no dump frames found for {self.working_dir}/{self.filename!r}")
+        M = torch.zeros((3, ntypes, T), dtype=torch.float64, device=dev)
+        st = torch.zeros((T,), dtype=torch.float64, device=dev)
+        for idxs, m in pieces:
+            ii = torch.tensor(idxs, device=dev)
+            M[:, :, ii] = m
+            st[ii] = torch.tensor([float(steps[i]) for i in idxs], dtype=torch.float64, device=dev)
+        dist.all_reduce_sum_(M)
+        dist.all_reduce_sum_(st)
+        self._set_even_time(st.cpu().numpy())
+        return M.cpu().numpy()
+
+    def correlate_translational_dipole(self, dipole, max_lag=None):
+        """[ntypes+1, max_lag] in C^2 m^2: row i = sum_j sum_axes <dM_i(lag) . dM_j(lag)> over all time origins, last row
+        <|dM_tot(lag)|^2> (the row convention of ``correlate_charge_flux``).  By linearity row i is the cross MSD of the
+        three channel pairs (M_i,c , M_tot,c): one mdp_cross_msd_fft call of 3 (ntypes+1) channels.  max_lag defaults to
+        T // 2."""
+        m = torch.as_tensor(np.ascontiguousarray(dipole, dtype=np.float64)).cuda()
+        _, ntypes, T = m.shape
+        max_lag = T // 2 if max_lag is None else min(int(max_lag), T)
+        if max_lag < 1:
+            raise ValueError(f"max_lag must be at least 1 ({T} frames)")
+        tot = m[:, 0].clone()
+        for i in range(1, ntypes):                      # fixed order
+            tot += m[:, i]
+        rows = torch.cat([m.permute(1, 0, 2), tot[None]], dim=0)       # [ntypes+1, 3, T]
+        lo, hi = dist.shard_range(ntypes + 1)
+        out = torch.zeros((ntypes + 1, max_lag), dtype=torch.float64, device=m.device)
+        if hi > lo:
+            a = rows[lo:hi].reshape(-1, T).contiguous()
+            b = tot[None].expand(hi - lo, 3, T).reshape(-1, T).contiguous()
+            out[lo:hi] = ops.cross_msd_fft(a, b, np.arange(0, 3 * (hi - lo) + 1, 3), max_lag)
+        dist.all_reduce_sum_(out)
+        return out.cpu().numpy()
+
+    def _fit_window(self, max_lag, initial_time, final_time):
+        """Lag times l * dt (l < max_lag) and the mask of the fit window: by default the lags max(1, max_lag // 10) to
+        max_lag - 1."""
+        dt = self.time[1] - self.time[0] if len(self.time) > 1 else 0.0
+        t = np.arange(max_lag) * dt
+        lo = t[min(max(1, max_lag // 10), max_lag - 1)] if initial_time is None else initial_time
+        hi = t[max_lag - 1] if final_time is None else final_time
+        mask = (t >= lo) & (t <= hi)
+        if max_lag < 2 or mask.sum() < 2:
+            raise ValueError(f"the fit window [{lo}, {hi}] holds {int(mask.sum()) if max_lag >= 2 else 0} lag times; "
+                             "at least 2 are needed")
+        return t, mask
+
+    @staticmethod
+    def _slope(t, y):
+        """Ordinary least squares with intercept: the slope of y against t."""
+        tc = t - t.mean()
+        return float(np.dot(tc, y - y.mean()) / np.dot(tc, tc))
+
+    def einstein(self, max_lag=None, initial_time=None, final_time=None, save=False):
+        """Einstein (Helfand) conductivity sigma_E[ntypes+1] in S/m: the slope of each row of the translational-dipole
+        MSD (``correlate_translational_dipole``) against the lag time, fitted with intercept over
+        initial_time <= t <= final_time, divided by 6 k_B T V.  Row i is the share of type i, the last row the total.
+        ``save`` writes dipole_msd.csv and einstein_conductivity.csv into ``working_dir``."""
+        dipole = self.get_translational_dipole()
+        msd = self.correlate_translational_dipole(dipole, max_lag)
+        max_lag = msd.shape[1]
+        t, mask = self._fit_window(max_lag, initial_time, final_time)
+        cond = np.array([self._slope(t[mask], row[mask]) for row in msd]) / (
+            6 * constants.BOLTZMANN * self.temp * self.volume)
+        if save and dist.rank() == 0:
+            names = "t," + ",".join(str(i + 1) for i in range(len(msd) - 1)) + ",tot"
+            np.savetxt(f"{self.working_dir}/dipole_msd.csv", np.append(t[None], msd, axis=0).T, delimiter=",", header=names,
+                       comments="")
+            win = np.asarray([[t[mask][0]] * len(cond), [t[mask][-1]] * len(cond), cond])
+            np.savetxt(f"{self.working_dir}/einstein_conductivity.csv", win.T, delimiter=",", header="start_t,end_t,cond",
+                       comments="")
+        return cond
+
+    def nernst(self, max_lag=None, initial_time=None, final_time=None, save=False):
+        """Nernst-Einstein conductivity sigma_NE[ntypes+1] in S/m: row g = D_g sum_{m in g} q_m^2 / (V k_B T), the last
+        row the sum.  D_g is slope / 6 of the all-origins centre-of-mass MSD of type g, fitted as in ``einstein`` (same
+        window defaults, so sigma_NE / sigma_E is the Haven ratio); q_m is the molecule's charge summed in atom order.
+        ``save`` writes nernst_einstein.csv (type, diffusion (m2/s), cond)."""
+        _, _, seg_off = mol_membership(self.num_mols, self.num_atoms_per_mol)
+        ntypes = len(self.num_mols)
+        type_off = np.concatenate(([0], np.cumsum(self.num_mols))).astype(np.int64)
+        dev = torch.device("cuda", torch.cuda.current_device())
+        seg_d = torch.from_numpy(seg_off.astype(np.int32)).to(dev)
+        # every rank parses every frame; the molecules of each type are split in contiguous blocks over the ranks
+        shards = [dist.shard_range(int(n)) for n in self.num_mols]
+        sel = np.concatenate([np.arange(type_off[g] + lo, type_off[g] + hi) for g, (lo, hi) in enumerate(shards)])
+        sel_d = torch.from_numpy(sel.astype(np.int64)).to(dev)
+        coms, steps, md = [], [], None
+        for _, ts, pos in self._fixed_charge_frames():
+            if md is None:
+                md = torch.from_numpy(np.ascontiguousarray(self._fixed[2])).to(dev)
+            com, _, _ = ops.segment_com(pos, md, seg_d)                          # [F, 3, M]
+            coms.append(com.index_select(2, sel_d))
+            steps += ts
+        self._set_even_time(steps)
+        T = len(steps)
+        max_lag = T // 2 if max_lag is None else min(int(max_lag), T)
+        t, mask = self._fit_window(max(max_lag, 1), initial_time, final_time)
+        conv = constants.DISTANCE_CONVERSION[self.units]
+        com = torch.cat(coms, dim=0) * conv                                     # [T, 3, Mloc] in m
+        chans = com.permute(2, 1, 0).reshape(-1, T).contiguous()                # [Mloc * 3, T]
+        goff = 3 * np.concatenate(([0], np.cumsum([hi - lo for lo, hi in shards]))).astype(np.int64)
+        if chans.shape[0]:
+            msd = ops.cross_msd_fft(chans, None, goff, max_lag)
+        else:                                       # a rank without molecules still joins the all-reduce
+            msd = torch.zeros((ntypes, max_lag), dtype=torch.float64, device=dev)
+        dist.all_reduce_sum_(msd)
+        msd = msd.cpu().numpy() / np.asarray(self.num_mols, dtype=np.float64)[:, None]
+        diff = np.array([self._slope(t[mask], row[mask]) for row in msd]) / 6
+        qmol = np.add.reduceat(self._fixed[0], seg_off[:-1]) * constants.CHARGE_CONVERSION[self.units]
+        q2 = np.array([np.sum(qmol[type_off[g]:type_off[g + 1]] ** 2) for g in range(ntypes)])
+        cond = diff * q2 / (self.volume * constants.BOLTZMANN * self.temp)
+        cond = np.append(cond, cond.sum())
+        if save and dist.rank() == 0:
+            with open(f"{self.working_dir}/nernst_einstein.csv", "w") as f:
+                f.write("type,diffusion (m2/s),cond\n")
+                for g in range(ntypes):
+                    f.write(f"{g + 1},{diff[g]!r},{cond[g]!r}\n")
+                f.write(f"tot,,{cond[-1]!r}\n")
+        return cond

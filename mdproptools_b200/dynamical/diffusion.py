@@ -26,6 +26,34 @@ from ..io import dump as _dump
 from ..io.pipeline import ArrayBatches, FrameBatches
 
 
+class MissingCoordinatesError(AssertionError, ValueError):
+    """A dump without unwrapped coordinates and without the image flags to build them (an ``AssertionError``, as in the
+    reference, and a ``ValueError``)."""
+
+
+def position_columns(cols):
+    """Dump columns of the unwrapped positions (_prepare_unwrapped_coords :62-81): ``xu yu zu`` when ``zu`` is present, else
+    ``x y z ix iy iz`` (unwrapped as x + ix * (xhi - xlo) by ``unwrapped_positions``)."""
+    if "zu" in cols:
+        return ["xu", "yu", "zu"]
+    if "z" not in cols:
+        raise MissingCoordinatesError("Missing wrapped and unwrapped coordinates (x y z xu yu zu)")
+    if "iz" not in cols:
+        raise MissingCoordinatesError("Missing unwrapped coordinates (xu yu zu) and box location ("
+                                      "ix iy iz) for converting wrapped coordinates (x y z) into "
+                                      "unwrapped coordinates. ")
+    return ["x", "y", "z", "ix", "iy", "iz"]
+
+
+def unwrapped_positions(dev, metas, k0, have_u):
+    """[F,3,N] unwrapped positions of a parsed batch ``dev`` [F,C,N] whose columns k0.. are those of ``position_columns``
+    (``have_u``: the three ``xu yu zu``; else the six ``x y z ix iy iz``)."""
+    if have_u:
+        return dev[:, k0:k0 + 3, :]
+    L = torch.tensor([m.box.bound_lengths() for m in metas], dtype=torch.float64, device=dev.device)
+    return dev[:, k0:k0 + 3, :] + dev[:, k0 + 3:k0 + 6, :] * L[:, :, None]      # x.add(ix.multiply(L)) (:78-80)
+
+
 class Diffusion:
     """Same constructor and methods as the reference class (:32-60)."""
 
@@ -47,27 +75,15 @@ class Diffusion:
         if not cols:
             raise ValueError(f"no dump frames found for {pattern!r}")
         assert "id" in cols, "Missing atom id's in dump file."
-        have_u = "zu" in cols
-        if have_u:
-            want = ["id", "xu", "yu", "zu"]
-        else:
-            assert "z" in cols, "Missing wrapped and unwrapped coordinates (x y z xu yu zu)"
-            assert "iz" in cols, ("Missing unwrapped coordinates (xu yu zu) and box location ("
-                                  "ix iy iz) for converting wrapped coordinates (x y z) into "
-                                  "unwrapped coordinates. ")
-            want = ["id", "x", "y", "z", "ix", "iy", "iz"]
+        want = ["id"] + position_columns(cols)
+        have_u = len(want) == 4
         want += [c for c in extra_cols if c not in want]
         chunks, metas, first_host = [], [], None
         for batch in FrameBatches(pattern, want):
             dev = batch.wait()
             if first_host is None:
                 first_host = {c: batch.host[0, k].numpy().copy() for k, c in enumerate(want)}
-            if have_u:
-                xyz = dev[:, 1:4, :]
-            else:
-                L = torch.tensor([m.box.bound_lengths() for m in batch.metas], dtype=torch.float64, device=dev.device)
-                xyz = dev[:, 1:4, :] + dev[:, 4:7, :] * L[:, :, None]      # x.add(ix.multiply(L)) (:78-80)
-            chunks.append(xyz.contiguous())
+            chunks.append(unwrapped_positions(dev, batch.metas, 1, have_u).contiguous())
             metas += batch.metas
         coords = torch.cat(chunks, dim=0) if len(chunks) > 1 else chunks[0]
         times = np.array([m.timestep * self.timestep * constants.TIME_CONVERSION[self.units] for m in metas])

@@ -280,6 +280,24 @@ def xcorr_unbiased(a, b, nlags=None):
     return out
 
 
+def cross_msd_fft(a, b, group_off, nlags):
+    """mdp_cross_msd_fft: a, b [C,T] (b None: the self case, b = a), group_off host ints [G+1] ->
+    out [G, nlags] = sum over the group's channels of the all-origins mean of (a(t+tau) - a(t)) * (b(t+tau) - b(t))."""
+    a = _f64(a, "a")
+    C, T = a.shape
+    if b is not None:
+        b = _f64(b, "b")
+        if b.shape != a.shape:
+            raise ValueError(f"b must have the shape of a {tuple(a.shape)}, got {tuple(b.shape)}")
+    garr, gptr = _host_i64(group_off)
+    G = len(garr) - 1
+    ctx = Context.get(a.device.index)
+    out = torch.empty((max(G, 0), max(int(nlags), 0)), dtype=torch.float64, device=a.device)
+    check(lib().mdp_cross_msd_fft(ctx.handle, C, T, ptr(a), ptr(b), G, gptr, int(nlags), ptr(out), stream_ptr()),
+          "mdp_cross_msd_fft")
+    return out
+
+
 def cumtrapz(y, dx, scale=1.0, leading_zero=True):
     y = _f64(y, "y")
     R, T = y.shape
