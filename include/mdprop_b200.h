@@ -46,7 +46,8 @@ int64_t mdp_ctx_launch_count(mdp_ctx *ctx);
 /* optional kernel timing for benchmarks: when enabled, the library brackets its main kernels with CUDA events
  * on the launching stream.  tag 0 = pair kernel (k_pair), 1 = pair preparation (sort, boxes, work list),
  * 2 = streaming MSD kernel, 3 = correlation kernel, 4 = charge-flux kernel, 5 = windowed (all-origins) MSD kernel,
- * 6 = bitmask autocorrelation kernel, 7 = FFT all-origins MSD (the whole of mdp_cross_msd_fft).  mdp_ctx_timing_read synchronises
+ * 6 = bitmask autocorrelation kernel, 7 = FFT all-origins MSD (the whole of mdp_cross_msd_fft), 8 = structure factor (the
+ * whole of mdp_structure_factor: kernels k_sk_sort, k_sk_rho, k_sk_bins).  mdp_ctx_timing_read synchronises
  * on the recorded events, returns the summed milliseconds and the number of launches, and clears them. */
 int mdp_ctx_timing(mdp_ctx *ctx, int enable);
 int mdp_ctx_timing_read(mdp_ctx *ctx, int tag, double *ms_total, int64_t *count);
@@ -256,6 +257,28 @@ int mdp_cross_msd_fft(mdp_ctx *ctx, int nchan, int64_t T, const double *a, const
  * in = DEVICE [nrows][T]; out = DEVICE [nrows][T] if leading_zero else [nrows][T-1]; out = scale*integral. */
 int mdp_cumtrapz(mdp_ctx *ctx, int nrows, int64_t T, const double *in, double dx, double scale,
                  int leading_zero, double *out, void *stream);
+
+/* ---- static structure factor (extension: no reference implementation; defined by tests/sk_oracle.py) -------------------
+ * Direct sum over reciprocal-lattice vectors of the restricted triclinic cell H = [a b c], a = (lx,0,0), b = (xy,ly,0),
+ * c = (xz,yz,lz): cell = HOST double [6] = {lx, ly, lz, xy, xz, yz}, shared by every frame of the call (one call per run of
+ * frames with the same cell).  For Miller triplets n (HOST int32 [nk][3], the caller's k-set, sorted by bin) and classes
+ * c (cls = DEVICE int32 per atom in [0, ncls), cls_stride = n if it differs per frame, 0 if one array serves all frames,
+ * NULL = every atom in class 0; atoms with a class outside [0, ncls) are left out):
+ *   rho_c(n) = sum_{j in c} exp(2 pi i n.s_j),   s_j = H^-1 r_j   (xyz = DEVICE [nframes][3][n]; wrapped or unwrapped
+ *              positions give the same result, n being integer)
+ *   sums_out[f][row(a,b)][bin] = sum_{k = bin_off[bin]}^{bin_off[bin+1]-1} Re(rho_a(n_k) conj(rho_b(n_k)))
+ * one row per unordered class pair a <= b, row(a,b) = a*ncls - a*(a-1)/2 + (b-a) (as mdp_pair_hist's symmetric mode);
+ * bin_off = HOST int64 [nbins+1], non-decreasing from 0 to nk; sums_out = DEVICE double [nframes][ncls(ncls+1)/2][nbins],
+ * overwritten.  nk = 0 and empty classes give zeros.
+ * Accuracy contract (csrc/sk_phase.h, derived in DESIGN 4.5): the phase is the exact integer n.u mod 2^32 of 32-bit fixed-point
+ * fractional coordinates, sin and cos are fp32, terms are summed in fp32 over at most 32 atoms and in fp64 beyond; for every
+ * |h|, |k|, |l| <= 1024:  |rho_c(k)_device - rho_c(k)_exact| <= 1e-5 * N_c.
+ * Fixed summation order, no atomics: run-to-run bit-identical, and the same bits under every scratch limit that admits the call.
+ * MDP_ERR_ARG for negative sizes, n >= 2^31, ncls outside [1, 64], a non-positive or non-finite length, a non-finite tilt,
+ * a Miller component beyond +-1024, or a bin_off that is not non-decreasing from 0 to nk. */
+int mdp_structure_factor(mdp_ctx *ctx, int nframes, int64_t n, const double *xyz, const int32_t *cls, int64_t cls_stride,
+                         int ncls, const double *cell, int64_t nk, const int32_t *miller, int nbins, const int64_t *bin_off,
+                         double *sums_out, void *stream);
 
 /* ---- residence time (residence_time.py:70-148) ---------------------------------------------------
  * Survival correlation from per-pair time bitmasks.  masks = DEVICE uint64 [npairs][nwords], bit t of

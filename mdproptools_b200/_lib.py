@@ -69,6 +69,8 @@ _PROTOS = {
     "mdp_xcorr_fft": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "mdp_cross_msd_fft": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int, POINTER(c_int64), c_int64, c_void_p,
                                   c_void_p]),
+    "mdp_structure_factor": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int64, c_int, POINTER(c_double), c_int64,
+                                     POINTER(c_int32), c_int, POINTER(c_int64), c_void_p, c_void_p]),
     "mdp_cumtrapz": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_double, c_double, c_int, c_void_p, c_void_p]),
     "mdp_bitmask_fill": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "mdp_bitmask_autocorr": (c_int, [c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p, c_void_p]),
@@ -89,6 +91,7 @@ _PROTOS = {
 EXPORTED_SYMBOLS = tuple(_PROTOS)
 
 PAIR_NO_CULL, PAIR_NO_SORT, PAIR_TRICLINIC, PAIR_F64 = 1, 2, 4, 16   # flags of mdp_pair_hist / mdp_pair_list
+SK_NLIM, SK_MAX_CLASSES, SK_EPS = 1024, 64, 1e-5       # mdp_structure_factor: Miller bound, classes, accuracy (csrc/sk_phase.h)
 
 
 def lib() -> ctypes.CDLL:

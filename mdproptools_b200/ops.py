@@ -298,6 +298,30 @@ def cross_msd_fft(a, b, group_off, nlags):
     return out
 
 
+def structure_factor(xyz, cls, ncls, cell, miller, bin_off, nbins):
+    """mdp_structure_factor: xyz float64 [F,3,N]; cls int32 [N] or [F,N] or None (one class); cell host (lx, ly, lz, xy, xz,
+    yz) shared by the F frames; miller host ints [nk,3] sorted by bin; bin_off host ints [nbins+1] ->
+    float64 [F, ncls(ncls+1)/2, nbins]: per class-pair row (ops.sym_row) the sum over each bin's k-vectors of
+    Re(rho_a(k) conj(rho_b(k)))."""
+    xyz = _f64(xyz, "xyz")
+    F, _, n = xyz.shape
+    cell = np.ascontiguousarray(cell, dtype=np.float64).reshape(-1)
+    if cell.size != 6:
+        raise ValueError(f"cell must hold 6 values (lx, ly, lz, xy, xz, yz), got {cell.size}")
+    miller = np.ascontiguousarray(miller, dtype=np.int32).reshape(-1, 3)
+    boff, bptr = _host_i64(bin_off)
+    if boff.shape != (int(nbins) + 1,):
+        raise ValueError(f"bin_off must hold nbins + 1 = {int(nbins) + 1} offsets, got shape {boff.shape}")
+    cls = _i32(cls, "cls")
+    stride = 0 if cls is None or cls.dim() == 1 else n
+    ctx = Context.get(xyz.device.index)
+    out = torch.empty((F, sym_rows(int(ncls)), int(nbins)), dtype=torch.float64, device=xyz.device)
+    check(lib().mdp_structure_factor(ctx.handle, F, n, ptr(xyz), ptr(cls), stride, int(ncls), _lib.dptr(cell), miller.shape[0],
+                                     miller.ctypes.data_as(ctypes.POINTER(c_int32)), int(nbins), bptr, ptr(out), stream_ptr()),
+          "mdp_structure_factor")
+    return out
+
+
 def cumtrapz(y, dx, scale=1.0, leading_zero=True):
     y = _f64(y, "y")
     R, T = y.shape
