@@ -47,7 +47,8 @@ int64_t mdp_ctx_launch_count(mdp_ctx *ctx);
  * on the launching stream.  tag 0 = pair kernel (k_pair), 1 = pair preparation (sort, boxes, work list),
  * 2 = streaming MSD kernel, 3 = correlation kernel, 4 = charge-flux kernel, 5 = windowed (all-origins) MSD kernel,
  * 6 = bitmask autocorrelation kernel, 7 = FFT all-origins MSD (the whole of mdp_cross_msd_fft), 8 = structure factor (the
- * whole of mdp_structure_factor: kernels k_sk_sort, k_sk_rho, k_sk_bins).  mdp_ctx_timing_read synchronises
+ * whole of mdp_structure_factor: kernels k_sk_sort, k_sk_rho, k_sk_bins; and of mdp_sk_rho: k_sk_sort, k_sk_rho), 9 = binned
+ * FFT correlation of complex series (the whole of mdp_isf_fft: kernels k_isf_*).  mdp_ctx_timing_read synchronises
  * on the recorded events, returns the summed milliseconds and the number of launches, and clears them. */
 int mdp_ctx_timing(mdp_ctx *ctx, int enable);
 int mdp_ctx_timing_read(mdp_ctx *ctx, int tag, double *ms_total, int64_t *count);
@@ -279,6 +280,30 @@ int mdp_cumtrapz(mdp_ctx *ctx, int nrows, int64_t T, const double *in, double dx
 int mdp_structure_factor(mdp_ctx *ctx, int nframes, int64_t n, const double *xyz, const int32_t *cls, int64_t cls_stride,
                          int ncls, const double *cell, int64_t nk, const int32_t *miller, int nbins, const int64_t *bin_off,
                          double *sums_out, void *stream);
+/* rho_c(n) itself, per k-vector and frame: the first half of mdp_structure_factor, with the same arguments up to miller, the
+ * same checks, accuracy contract and frame sub-batches, and bit for bit the rho values that mdp_structure_factor bins.
+ * rho_out = DEVICE complex fp64 (re, im) [ncls][nk][out_stride]; frame f of the call goes to column frame0 + f
+ * (0 <= frame0, frame0 + nframes <= out_stride), so that successive calls fill one time series per (class, k) in place;
+ * other columns are left alone.  MDP_ERR_ARG as for mdp_structure_factor, or for frames outside the series. */
+int mdp_sk_rho(mdp_ctx *ctx, int nframes, int64_t n, const double *xyz, const int32_t *cls, int64_t cls_stride, int ncls,
+               const double *cell, int64_t nk, const int32_t *miller, double *rho_out, int64_t out_stride, int64_t frame0,
+               void *stream);
+/* Binned, symmetrised all-origins correlation of complex series (csrc/isf_fft.h; the coherent intermediate scattering function
+ * when rho holds mdp_sk_rho's series; defined by the long-double direct sum of tests/isf_oracle.py):
+ *   out[p][bin][tau] = sum_{k = bin_off[bin]}^{bin_off[bin+1]-1} 1/(T-tau) sum_{t < T-tau}
+ *                      1/2 Re( z_a(k,t+tau) z_b(k,t)* + z_b(k,t+tau) z_a(k,t)* ),   (a, b) = pairs[p],  tau < nlags.
+ * rho = DEVICE complex fp64 (re, im) [nchan][nk][T], z_c(k,t) = rho[c][k][t], not centred; pairs = HOST int32 [npairs][2] of
+ * channels in [0, nchan); bin_off = HOST int64 [nbins+1], non-decreasing from 0 to nk; 1 <= nlags <= T; out = DEVICE double
+ * [npairs][nbins][nlags], overwritten.  Empty bins and nk = 0 give zeros.  One forward transform per (k, channel some pair
+ * uses) of N = 2^p >= T + nlags points (p <= 30); the real, even spectrum of each (pair, bin) is summed over the bin's
+ * k-vectors in k order and two pairs of the same bin share one inverse transform.
+ * Agrees with the direct long-double sum to 1e-10 of max_tau |out[p][bin]| for T <= 10^5.  Fixed summation order, no atomics:
+ * run-to-run bit-identical; the same bits under every scratch limit that admits the call; a bin's bits do not depend on
+ * which other bins share the call; swapping the two channels of a pair gives the same bits.
+ * MDP_ERR_ARG for bad sizes, a pair naming a channel outside [0, nchan), a bad bin_off, p > 30, or accumulators (about
+ * npairs * nbins * (N/2 + 1) * 8 bytes) above the context's scratch limit. */
+int mdp_isf_fft(mdp_ctx *ctx, int nchan, int64_t nk, int64_t T, const double *rho, int npairs, const int32_t *pairs, int nbins,
+                const int64_t *bin_off, int64_t nlags, double *out, void *stream);
 
 /* ---- residence time (residence_time.py:70-148) ---------------------------------------------------
  * Survival correlation from per-pair time bitmasks.  masks = DEVICE uint64 [npairs][nwords], bit t of

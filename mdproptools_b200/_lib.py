@@ -71,6 +71,10 @@ _PROTOS = {
                                   c_void_p]),
     "mdp_structure_factor": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int64, c_int, POINTER(c_double), c_int64,
                                      POINTER(c_int32), c_int, POINTER(c_int64), c_void_p, c_void_p]),
+    "mdp_sk_rho": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int64, c_int, POINTER(c_double), c_int64, POINTER(c_int32),
+                           c_void_p, c_int64, c_int64, c_void_p]),
+    "mdp_isf_fft": (c_int, [c_void_p, c_int, c_int64, c_int64, c_void_p, c_int, POINTER(c_int32), c_int, POINTER(c_int64), c_int64,
+                            c_void_p, c_void_p]),
     "mdp_cumtrapz": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_double, c_double, c_int, c_void_p, c_void_p]),
     "mdp_bitmask_fill": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "mdp_bitmask_autocorr": (c_int, [c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p, c_void_p]),

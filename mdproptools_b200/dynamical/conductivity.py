@@ -33,6 +33,19 @@ from ..io.pipeline import FrameBatches
 from .diffusion import position_columns, unwrapped_positions
 
 
+def even_times(steps, units, timestep, source, who="the Einstein and Nernst-Einstein conductivity need"):
+    """Times in seconds of the frames' timesteps (in trajectory order), which must be evenly spaced: ValueError naming
+    ``who`` otherwise, and naming ``source`` when there is no frame."""
+    steps = np.asarray(steps, dtype=np.float64)
+    if len(steps) == 0:
+        raise ValueError(f"no dump frames found for {source}")
+    d = np.diff(steps)
+    if len(d) and not (d[0] > 0 and (d == d[0]).all()):
+        raise ValueError(f"{who} evenly spaced frames (timesteps "
+                         f"{steps[:3].tolist()}...: spacings {sorted(set(d.tolist()))[:4]})")
+    return steps * constants.TIME_CONVERSION[units] * timestep
+
+
 class Conductivity:
     def __init__(self, filename, num_mols, num_atoms_per_mol, volume, mass=None, temp=298.15, timestep=1, units="real",
                  working_dir=None):
@@ -286,14 +299,7 @@ class Conductivity:
 
     def _set_even_time(self, steps):
         """self.time from the timesteps of all frames (in trajectory order); they must be evenly spaced."""
-        steps = np.asarray(steps, dtype=np.float64)
-        if len(steps) == 0:
-            raise ValueError(f"no dump frames found for {self.working_dir}/{self.filename!r}")
-        d = np.diff(steps)
-        if len(d) and not (d[0] > 0 and (d == d[0]).all()):
-            raise ValueError("the Einstein and Nernst-Einstein conductivity need evenly spaced frames (timesteps "
-                             f"{steps[:3].tolist()}...: spacings {sorted(set(d.tolist()))[:4]})")
-        self.time = (steps * constants.TIME_CONVERSION[self.units] * self.timestep).tolist()
+        self.time = even_times(steps, self.units, self.timestep, f"{self.working_dir}/{self.filename!r}").tolist()
 
     def get_translational_dipole(self):
         """M[3, ntypes, T] in C m: per type, the sum over molecules of charge x unwrapped centre of mass (SI).  Positions

@@ -322,6 +322,48 @@ def structure_factor(xyz, cls, ncls, cell, miller, bin_off, nbins):
     return out
 
 
+def sk_rho(xyz, cls, ncls, cell, miller, out=None, frame0=0):
+    """mdp_sk_rho: xyz float64 [F,3,N]; cls, cell, miller as for ``structure_factor`` -> complex128 [C >= ncls, nk, T]:
+    rho_c(k) of frame f at column frame0 + f of ``out`` for c < ncls (a new [ncls, nk, F] series when None; other columns
+    and channels untouched)."""
+    xyz = _f64(xyz, "xyz")
+    F, _, n = xyz.shape
+    cell = np.ascontiguousarray(cell, dtype=np.float64).reshape(-1)
+    if cell.size != 6:
+        raise ValueError(f"cell must hold 6 values (lx, ly, lz, xy, xz, yz), got {cell.size}")
+    miller = np.ascontiguousarray(miller, dtype=np.int32).reshape(-1, 3)
+    nk = miller.shape[0]
+    if out is None:
+        out = torch.zeros((int(ncls), nk, F), dtype=torch.complex128, device=xyz.device)
+    if not (out.is_cuda and out.dtype == torch.complex128 and out.is_contiguous() and out.dim() == 3
+            and out.shape[0] >= int(ncls) and out.shape[1] == nk):
+        raise ValueError(f"out must be a contiguous complex128 CUDA tensor [>= {int(ncls)}, {nk}, T]")
+    cls = _i32(cls, "cls")
+    stride = 0 if cls is None or cls.dim() == 1 else n
+    ctx = Context.get(xyz.device.index)
+    check(lib().mdp_sk_rho(ctx.handle, F, n, ptr(xyz), ptr(cls), stride, int(ncls), _lib.dptr(cell), nk,
+                           miller.ctypes.data_as(ctypes.POINTER(c_int32)), ptr(out), out.shape[2], int(frame0), stream_ptr()),
+          "mdp_sk_rho")
+    return out
+
+
+def isf_fft(rho, pairs, bin_off, nlags):
+    """mdp_isf_fft: rho complex128 [nchan, nk, T]; pairs host ints [npairs, 2] of channels; bin_off host ints [nbins+1] ->
+    float64 [npairs, nbins, nlags]: per pair and bin the sum over the bin's k-vectors of the symmetrised all-origins
+    correlation 1/2 Re<z_a(t+tau) z_b(t)* + z_b(t+tau) z_a(t)*>."""
+    if not (rho.is_cuda and rho.dtype == torch.complex128 and rho.is_contiguous() and rho.dim() == 3):
+        raise ValueError("rho must be a contiguous complex128 CUDA tensor [nchan, nk, T]")
+    nchan, nk, T = rho.shape
+    pr = np.ascontiguousarray(pairs, dtype=np.int32).reshape(-1, 2)
+    boff, bptr = _host_i64(bin_off)
+    nbins = boff.shape[0] - 1
+    ctx = Context.get(rho.device.index)
+    out = torch.empty((pr.shape[0], max(nbins, 0), max(int(nlags), 0)), dtype=torch.float64, device=rho.device)
+    check(lib().mdp_isf_fft(ctx.handle, nchan, nk, T, ptr(rho), pr.shape[0], pr.ctypes.data_as(ctypes.POINTER(c_int32)), nbins, bptr,
+                            int(nlags), ptr(out), stream_ptr()), "mdp_isf_fft")
+    return out
+
+
 def cumtrapz(y, dx, scale=1.0, leading_zero=True):
     y = _f64(y, "y")
     R, T = y.shape
