@@ -1,5 +1,6 @@
 // fft_corr.h -- unbiased time correlation through a Stockham FFT in fp64: radix-2 butterflies, three stages per pass
-// (host/device shared bodies of the kernels in fftcorr.cu; exercised on the host by tests/native/fft_corr_host.cpp).
+// (host/device shared bodies of fft_pass.cuh and fftcorr.cu, also used by msd_fft.h and isf_fft.h; exercised on the host
+// by tests/native/fft_corr_host.cpp).
 //
 // out[tau] = (sum_{t < T - tau} a[t + tau] * b[t]) / (T - tau)       (conductivity.py:97-114, viscosity.py:86-120)
 //
@@ -66,7 +67,7 @@ MDP_HD void mdp_fft_butterfly(const mdp_c64 *x, mdp_c64 *y, const mdp_c64 *W, lo
 // registers of its two inputs, and the positions they WOULD have in the Stockham array are carried along (pos[]), so the
 // arithmetic is, operation for operation, that of R calls of mdp_fft_butterfly -- bit-identical results (checked on the
 // host by tests/native/fft_corr_host.cpp).  in(pos) reads a point, out(pos, v) writes one: the first pass of a transform
-// can read the real series directly and the last one can write the normalised correlation (fftcorr.cu).
+// can read the real series directly and the last one can write the normalised correlation (fft_pass.cuh).
 // Requires t + R <= log2 n.
 template <int R, class In, class Out>
 MDP_HD void mdp_fft_radix_pass(const In in, const Out out, const mdp_c64 *W, long long i, int t, long long n)
@@ -140,4 +141,45 @@ MDP_HD int mdp_fft_log2_size(long long T, long long nlags)   // smallest p with 
     int p = 1;
     while ((1ll << p) < T + nlags) ++p;
     return p;
+}
+
+// lag tau of the unbiased correlation from element tau of a transform of N points (x = its real or imaginary part)
+MDP_HD double mdp_fft_unbiased(double x, long long n, long long T, long long tau)
+{
+    return x / (double)n / (double)(T - tau);
+}
+
+// element k (0 <= k < n) of a real even spectrum held as its half acc[0 .. n/2]
+MDP_HD long long mdp_fft_fold(long long k, long long n)
+{
+    return k <= n / 2 ? k : n - k;
+}
+
+// the earlier name of mdp_fft_fold (msd_fft.h and isf_fft.h both offered it), kept for host code written against it
+MDP_HD long long mdp_msd_fold(long long k, long long n)
+{
+    return mdp_fft_fold(k, n);
+}
+
+// A real even spectrum transforms to a real series, so one complex inverse transform serves two groups of spectra.
+// Groups come in bins of per_bin (the MSD's groups are one bin, an ISF bin holds one group per pair), and groups of
+// different bins never share a transform, so a bin's bits depend on its own groups only.  A bin takes
+// mdp_fft_transforms_per_bin(per_bin) transforms; its transform j carries group `first` of the bin in its real part and,
+// when `partner`, group first + 1 in its imaginary part (an odd last group is paired with zero).
+MDP_HD long long mdp_fft_transforms_per_bin(long long per_bin)
+{
+    return (per_bin + 1) / 2;
+}
+
+struct mdp_fft_group_pair {
+    long long first;
+    bool partner;
+};
+
+MDP_HD mdp_fft_group_pair mdp_fft_pair_groups(long long j, long long per_bin)
+{
+    mdp_fft_group_pair r;
+    r.first = 2 * j;
+    r.partner = r.first + 1 < per_bin;
+    return r;
 }

@@ -11,7 +11,7 @@
 //     G(w) = 1/2 (Re S(w) + Re S(-w))      (self pair a = b: 1/2 (|Z_a(w)|^2 + |Z_a(-w)|^2)).
 // G is real and even and linear in the k-vector, so it is summed over the bin's k-vectors (in k order) in the frequency
 // domain and one inverse transform serves a (pair, bin) group; two groups of the same bin share one complex transform
-// (mdp_msd_fold and the spectrum load of msdfft.cu).  rho is not centred: its time mean is physical (Bragg peaks).
+// (mdp_fft_pair_groups, mdp_fft_fold).  rho is not centred: its time mean is physical (Bragg peaks).
 //
 // G is computed as 1/2 ((a.re b.re + a.im b.im) + (a'.re b'.re + a'.im b'.im)): products commute, so the pairs (a, b) and
 // (b, a) give the same bits.
@@ -19,7 +19,7 @@
 // Accuracy: agreement with the long-double direct sum (tests/isf_oracle.py) to 1e-10 of max_tau |out[p][bin]| for
 // T <= 10^5 -- the contract of the FFT correlation (fft_corr.h, msd_fft.h).
 #pragma once
-#include "msd_fft.h"
+#include "fft_corr.h"
 
 // G at frequency k of the pair whose spectra are Za, Zb (Za == Zb for a self pair)
 MDP_HD double mdp_isf_spectrum(const mdp_c64 *Za, const mdp_c64 *Zb, long long k, long long n)
@@ -29,16 +29,13 @@ MDP_HD double mdp_isf_spectrum(const mdp_c64 *Za, const mdp_c64 *Zb, long long k
     return 0.5 * ((a.re * b.re + a.im * b.im) + (ac.re * bc.re + ac.im * bc.im));
 }
 
-// groups of a bin are its pairs; transform j of a bin carries pairs 2j (real part) and 2j + 1 (imaginary part, zero when
-// npairs is odd and 2j + 1 = npairs): groups of different bins never share a transform, so a bin's bits depend on its own
-// k-vectors only
+// the earlier names of the shared helpers for the ISF's bins and epilogue, kept for host code written against them
 MDP_HD long long mdp_isf_transforms_per_bin(long long npairs)
 {
-    return (npairs + 1) / 2;
+    return mdp_fft_transforms_per_bin(npairs);
 }
 
-// out[p][bin][tau] from element tau of the inverse transform (x = its real or imaginary part)
 MDP_HD double mdp_isf_epilogue(double x, long long n, long long T, long long tau)
 {
-    return x / (double)n / (double)(T - tau);
+    return mdp_fft_unbiased(x, n, T, tau);
 }

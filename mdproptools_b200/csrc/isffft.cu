@@ -3,23 +3,24 @@
 //
 // One call:
 //   per sub-batch of whole k-vectors (all channels that a pair uses, "units" = (k, channel) series):
-//     k_isf_fft_pass  the forward transform, three butterfly stages per pass (the first pass reads rho[c][k][0..T) and
-//                     zero-pads it);
+//     k_fft_pass      the forward transform, three butterfly stages per pass (fft_pass.cuh; the first pass reads
+//                     rho[c][k][0..T) and zero-pads it through IsfRhoIn);
 //     k_isf_spec_acc  acc_g[w] += G_k(w) of every group g = (bin, pair) over the bin's k-vectors in the sub-batch, in k
 //                     order, w <= N/2 (G is even).  The accumulator lives across sub-batches, so the summation order -- hence
 //                     every bit of the result -- does not depend on the scratch limit;
 //   k_isf_flag        per group: does its half spectrum hold a nonzero value (an empty bin or a pair of empty channels comes
 //                     out exactly zero instead of carrying round-off of its transform partner);
 //   per sub-batch of inverse transforms (two groups of the same bin each):
-//     k_isf_spec_load acc_g + i acc_{g+1} unfolded to N points;
-//     k_isf_fft_pass  the inverse transform (a forward FFT of a real even spectrum); its last pass writes out[p][bin] and
-//                     out[p+1][bin] through mdp_isf_epilogue.
+//     k_fft_spec_load acc_g + i acc_{g+1} unfolded to N points (bins of npairs groups, mdp_fft_pair_groups);
+//     k_fft_pass      the inverse transform (a forward FFT of a real even spectrum); its last pass writes out[p][bin] and
+//                     out[p+1][bin] through IsfEpilogueOut (mdp_fft_unbiased).
 // HBM traffic: 32 B per point and pass of the transforms, plus 16 B per point and pair for the spectrum accumulation.  No
 // atomics: run-to-run bit-identical.
 #include <algorithm>
 #include <vector>
 
 #include "common.cuh"
+#include "fft_pass.cuh"
 #include "isf_fft.h"
 #include "scratch_plan.h"
 
@@ -27,37 +28,20 @@ namespace {
 
 constexpr int IF_THREADS = 256;
 
-__global__ void __launch_bounds__(IF_THREADS) k_isf_twiddle(mdp_c64 *__restrict__ W, long long n)
-{
-    const long long k = (long long)blockIdx.x * IF_THREADS + threadIdx.x;
-    if (k < n / 2) W[k] = mdp_twiddle(k, n);
-}
-
-// IO 0: array -> array; 1: the first forward pass reads unit blockIdx.y = (k0 + u / nused, channel used[u % nused]) of
-// rho; 2: the last inverse pass writes transform j0 + blockIdx.y to out, tau < nlags
-struct IsfIo {
-    const mdp_c64 *x;
-    mdp_c64 *y;
+// the first forward pass reads unit u = (k0 + u / nused, channel used[u % nused]) of rho and zero-pads it
+struct IsfRhoIn {
     const mdp_c64 *rho;
-    const int *used, *flag;
-    double *out;
-    long long T, nk, nlags, n, k0, j0;
-    int nused, npairs, nbins;
-};
-
-template <int IO>
-struct IsfIn {
-    const IsfIo &io;
-    long long u;
-    __device__ __forceinline__ mdp_c64 operator()(long long i) const
+    const int *used;
+    long long T, nk, k0;
+    int nused;
+    __device__ __forceinline__ mdp_c64 operator()(long long u, long long i, long long) const
     {
-        if (IO != 1) return io.x[u * io.n + i];
         mdp_c64 v;
         v.re = 0.0;
         v.im = 0.0;
-        if (i < io.T) {
-            const long long k = io.k0 + u / io.nused, c = io.used[u % io.nused];
-            const double2 z = __ldg((const double2 *)io.rho + (c * io.nk + k) * io.T + i);
+        if (i < T) {
+            const long long k = k0 + u / nused, c = used[u % nused];
+            const double2 z = __ldg((const double2 *)rho + (c * nk + k) * T + i);
             v.re = z.x;
             v.im = z.y;
         }
@@ -65,42 +49,22 @@ struct IsfIn {
     }
 };
 
-template <int IO>
-struct IsfOut {
-    const IsfIo &io;
-    long long u;
-    __device__ __forceinline__ void operator()(long long i, const mdp_c64 &v) const
+// the last inverse pass writes inverse transform j0 + u to out[p][b] and out[p + 1][b], tau < nlags
+struct IsfEpilogueOut {
+    const int *flag;
+    double *out;
+    long long T, nlags, j0;
+    int npairs, nbins;
+    __device__ __forceinline__ void operator()(long long u, long long i, long long n, const mdp_c64 &v) const
     {
-        if (IO != 2) {
-            io.y[u * io.n + i] = v;
-            return;
-        }
-        if (i >= io.nlags) return;
-        const long long tpb = mdp_isf_transforms_per_bin(io.npairs), j = io.j0 + u;
-        const long long b = j / tpb, p = 2 * (j % tpb), g = b * io.npairs + p;
-        io.out[(p * io.nbins + b) * io.nlags + i] = io.flag[g] ? mdp_isf_epilogue(v.re, io.n, io.T, i) : 0.0;
-        if (p + 1 < io.npairs)
-            io.out[((p + 1) * io.nbins + b) * io.nlags + i] = io.flag[g + 1] ? mdp_isf_epilogue(v.im, io.n, io.T, i) : 0.0;
+        if (i >= nlags) return;
+        const long long tpb = mdp_fft_transforms_per_bin(npairs), j = j0 + u, b = j / tpb;
+        const mdp_fft_group_pair gp = mdp_fft_pair_groups(j % tpb, npairs);
+        const long long p = gp.first, g = b * npairs + p;
+        out[(p * nbins + b) * nlags + i] = flag[g] ? mdp_fft_unbiased(v.re, n, T, i) : 0.0;
+        if (gp.partner) out[((p + 1) * nbins + b) * nlags + i] = flag[g + 1] ? mdp_fft_unbiased(v.im, n, T, i) : 0.0;
     }
 };
-
-template <int R, int IO>
-__global__ void __launch_bounds__(IF_THREADS) k_isf_fft_pass(const IsfIo io, const mdp_c64 *__restrict__ W, int t)
-{
-    const long long i = (long long)blockIdx.x * IF_THREADS + threadIdx.x;
-    if (i >= (io.n >> R)) return;
-    const long long u = blockIdx.y;
-    mdp_fft_radix_pass<R>(IsfIn<IO>{io, u}, IsfOut<IO>{io, u}, W, i, t, io.n);
-}
-
-template <int IO>
-void launch_isf_pass(int R, const IsfIo &io, const mdp_c64 *W, int t, int units, cudaStream_t st)
-{
-    const dim3 g((unsigned)ceil_div<long long>(std::max<long long>(io.n >> R, 1), IF_THREADS), (unsigned)units);
-    if (R == 3) k_isf_fft_pass<3, IO><<<g, IF_THREADS, 0, st>>>(io, W, t);
-    else if (R == 2) k_isf_fft_pass<2, IO><<<g, IF_THREADS, 0, st>>>(io, W, t);
-    else k_isf_fft_pass<1, IO><<<g, IF_THREADS, 0, st>>>(io, W, t);
-}
 
 // grid (ceil((n/2 + 1) / IF_THREADS), <= 65535): groups g_lo + blockIdx.y, + gridDim.y, ... below g_hi;
 // acc[g][w] += sum over the k-vectors of g's bin in [k0, k1), in k order, of G_k(w).  Z = [k - k0][nused][n]
@@ -136,20 +100,6 @@ __global__ void __launch_bounds__(IF_THREADS) k_isf_flag(const double *__restric
     if (threadIdx.x == 0) flag[g] = nz;
 }
 
-// grid (ceil(n / IF_THREADS), transforms): x[j][w] = acc[g][fold w] + i acc[g + 1][fold w] for transform j0 + j
-__global__ void __launch_bounds__(IF_THREADS) k_isf_spec_load(const double *__restrict__ acc, long long n, int npairs, long long j0,
-                                                              mdp_c64 *__restrict__ x)
-{
-    const long long w = (long long)blockIdx.x * IF_THREADS + threadIdx.x;
-    if (w >= n) return;
-    const long long H = n / 2 + 1, tpb = mdp_isf_transforms_per_bin(npairs), j = j0 + blockIdx.y;
-    const long long b = j / tpb, p = 2 * (j % tpb), g = b * npairs + p, ww = mdp_msd_fold(w, n);
-    mdp_c64 v;
-    v.re = acc[g * H + ww];
-    v.im = p + 1 < npairs ? acc[(g + 1) * H + ww] : 0.0;
-    x[(long long)blockIdx.y * n + w] = v;
-}
-
 } // namespace
 
 extern "C" {
@@ -183,7 +133,7 @@ int mdp_isf_fft(mdp_ctx *ctx, int nchan, int64_t nk, int64_t T, const double *rh
     std::vector<int> pidx((size_t)2 * npairs);
     for (int q = 0; q < 2 * npairs; ++q) pidx[(size_t)q] = (int)(std::lower_bound(used.begin(), used.end(), pairs[q]) - used.begin());
     const int nused = (int)used.size();
-    const long long ngroups = (long long)npairs * nbins, tpb = mdp_isf_transforms_per_bin(npairs), U2 = nbins * tpb;
+    const long long ngroups = (long long)npairs * nbins, tpb = mdp_fft_transforms_per_bin(npairs), U2 = nbins * tpb;
 
     // group accumulators and everything else that does not scale with the sub-batch; sub-batches of whole k-vectors (nused
     // transforms each, two buffers) sized to 2 GiB of scratch on the whole request (scratch_plan.h).  The inverse transforms
@@ -219,32 +169,20 @@ int mdp_isf_fft(mdp_ctx *ctx, int nchan, int64_t nk, int64_t T, const double *rh
     MDP_CUDA(cudaMemcpyAsync(d_used, used.data(), used.size() * 4, cudaMemcpyHostToDevice, st));
     MDP_CUDA(cudaMemcpyAsync(d_boff, bin_off, (size_t)(nbins + 1) * 8, cudaMemcpyHostToDevice, st));
     MDP_CUDA(cudaMemsetAsync(acc, 0, (size_t)ngroups * H * 8, st));
-    k_isf_twiddle<<<(unsigned)ceil_div<long long>(std::max<long long>(n / 2, 1), IF_THREADS), IF_THREADS, 0, st>>>(W, n);
-    MDP_LAUNCHED(ctx);
+    mdp_fft_twiddles(ctx, W, n, st);
 
-    IsfIo io{nullptr, nullptr, (const mdp_c64 *)rho, d_used, flag, out, T, nk, nlags, n, 0, 0, nused, npairs, nbins};
     int b_lo = 0;
     for (long long k0 = 0; k0 < nk; k0 += batch) {                   // forward transforms and spectrum accumulation
         const long long k1 = std::min<long long>(nk, k0 + batch);
         const int units = (int)((k1 - k0) * nused);
-        io.k0 = k0;
-        mdp_c64 *src = x, *dst = y;
-        for (int t = 0; t < p;) {
-            const int R = mdp_fft_pass_radix(t, p);
-            io.x = src;
-            io.y = dst;
-            if (t == 0) launch_isf_pass<1>(R, io, W, t, units, st);
-            else launch_isf_pass<0>(R, io, W, t, units, st);
-            MDP_LAUNCHED(ctx);
-            std::swap(src, dst);
-            t += R;
-        }
+        const mdp_c64 *Z = mdp_fft_transform(ctx, IsfRhoIn{(const mdp_c64 *)rho, d_used, T, nk, k0, nused}, FftArrayOut{}, x, y, W, p,
+                                             units, st);
         while (bin_off[b_lo + 1] <= k0) ++b_lo;                      // first bin with a k-vector in [k0, k1)
         int b_hi = b_lo;
         while (b_hi + 1 < nbins && bin_off[b_hi + 1] < k1) ++b_hi;   // last one
         const long long g_lo = (long long)b_lo * npairs, g_hi = (long long)(b_hi + 1) * npairs;
         k_isf_spec_acc<<<dim3((unsigned)ceil_div<long long>(H, IF_THREADS), (unsigned)std::min<long long>(g_hi - g_lo, 65535)),
-                         IF_THREADS, 0, st>>>(src, n, nused, d_boff, d_pidx, npairs, g_lo, g_hi, k0, k1, acc);
+                         IF_THREADS, 0, st>>>(Z, n, nused, d_boff, d_pidx, npairs, g_lo, g_hi, k0, k1, acc);
         MDP_LAUNCHED(ctx);
     }
     k_isf_flag<<<(unsigned)ngroups, IF_THREADS, 0, st>>>(acc, H, flag);
@@ -252,23 +190,13 @@ int mdp_isf_fft(mdp_ctx *ctx, int nchan, int64_t nk, int64_t T, const double *rh
     const long long ibatch = batch * nused;
     for (long long j0 = 0; j0 < U2; j0 += ibatch) {                  // inverse transforms, two groups of a bin each
         const int nj = (int)std::min<long long>(ibatch, U2 - j0);
-        k_isf_spec_load<<<dim3((unsigned)ceil_div<long long>(n, IF_THREADS), (unsigned)nj), IF_THREADS, 0, st>>>(acc, n, npairs, j0, x);
+        k_fft_spec_load<<<dim3((unsigned)ceil_div<long long>(n, MDP_FFT_THREADS), (unsigned)nj), MDP_FFT_THREADS, 0, st>>>(acc, n, npairs,
+                                                                                                                     j0, x);
         MDP_LAUNCHED(ctx);
-        io.j0 = j0;
-        mdp_c64 *src = x, *dst = y;
-        for (int t = 0; t < p;) {
-            const int R = mdp_fft_pass_radix(t, p);
-            io.x = src;
-            io.y = dst;
-            if (t + R == p) launch_isf_pass<2>(R, io, W, t, nj, st);
-            else launch_isf_pass<0>(R, io, W, t, nj, st);
-            MDP_LAUNCHED(ctx);
-            std::swap(src, dst);
-            t += R;
-        }
+        mdp_fft_transform(ctx, FftArrayIn{x}, IsfEpilogueOut{flag, out, T, nlags, j0, npairs, nbins}, x, y, W, p, nj, st);
     }
     ctx->timer_end(tk, st);
-    return mdp_check_launch("k_isf_fft_pass");
+    return mdp_check_launch("k_fft_pass");
 }
 
 } // extern "C"

@@ -33,12 +33,6 @@ MDP_HD double mdp_msd_spectrum_cross(const mdp_c64 *Z, long long k, long long n)
     return 2.0 * mdp_cross_spectrum_conj(Z, k, n).re;
 }
 
-// element k of the inverse transform's input, read from the half spectrum acc[0 .. n/2] of a real even spectrum
-MDP_HD long long mdp_msd_fold(long long k, long long n)
-{
-    return k <= n / 2 ? k : n - k;
-}
-
 // out[tau] from the group's suffix sum suf[tau] = sum_{t >= tau} p(t), prefix sum pre[T - tau] = sum_{t < T-tau} p(t) and
 // the bracket xc = xc_ab(tau) + xc_ba(tau) (the inverse transform divided by N)
 MDP_HD double mdp_msd_epilogue(const double *suf, const double *pre, long long T, long long tau, double xc)

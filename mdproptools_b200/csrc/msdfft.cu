@@ -9,20 +9,22 @@
 //                   order: per-thread chunks, a serial scan of the chunk sums, then the chunks);
 //   per sub-batch of transforms ("units": channel a_c + i b_c in the cross case, two channels a_c + i a_c' of the same
 //   group in the self case, an odd last channel paired with zero):
-//     k_msd_fft_pass  the forward transform, three butterfly stages per pass (the first pass reads the centred series);
+//     k_fft_pass      the forward transform, three butterfly stages per pass (fft_pass.cuh; the first pass reads the
+//                     centred series through MsdSeriesIn);
 //     k_msd_spec_acc  acc_g[k] += the unit spectra of group g, units in order, k <= N/2 (the spectrum is even).  The
 //                     accumulator lives across sub-batches, so a group may span several of them and the summation order
 //                     -- hence every bit of the result -- does not depend on the scratch limit;
 //   per sub-batch of group pairs:
-//     k_msd_spec_load acc_g + i acc_{g+1} unfolded to N points;
-//     k_msd_fft_pass  the inverse transform (a forward FFT of a real even spectrum); its last pass writes out[g] and
-//                     out[g+1] through mdp_msd_epilogue.
+//     k_fft_spec_load acc_g + i acc_{g+1} unfolded to N points (the groups are one bin of mdp_fft_pair_groups);
+//     k_fft_pass      the inverse transform (a forward FFT of a real even spectrum); its last pass writes out[g] and
+//                     out[g+1] through MsdEpilogueOut (mdp_msd_epilogue).
 // HBM traffic: 32 B per point and pass of the transforms (as fftcorr.cu), plus 16 B per point for the spectrum
 // accumulation and 8-16 B per series point for the mean and p sums.  No atomics: results are run-to-run identical.
 #include <algorithm>
 #include <vector>
 
 #include "common.cuh"
+#include "fft_pass.cuh"
 #include "msd_fft.h"
 #include "scratch_plan.h"
 
@@ -30,12 +32,6 @@ namespace {
 
 constexpr int MF_THREADS = 256;
 constexpr int MF_SCAN_THREADS = 1024;
-
-__global__ void __launch_bounds__(MF_THREADS) k_msd_twiddle(mdp_c64 *__restrict__ W, long long n)
-{
-    const long long k = (long long)blockIdx.x * MF_THREADS + threadIdx.x;
-    if (k < n / 2) W[k] = mdp_twiddle(k, n);
-}
 
 // grid (nchan, 1 or 2): mean of channel blockIdx.x of a (y = 0) or b (y = 1)
 __global__ void __launch_bounds__(MDP_MSD_MEAN_LANES) k_msd_mean(const double *__restrict__ a, const double *__restrict__ b,
@@ -109,78 +105,47 @@ __global__ void __launch_bounds__(MF_SCAN_THREADS) k_msd_scan(const double *__re
     }
 }
 
-// IO 0: array -> array; 1: the first forward pass reads the centred series of unit blockIdx.y (utab = {c0, c1, group},
-// c1 = -1 for zero); 2: the last inverse pass writes out[g][tau], out[g+1][tau] (g = 2 * (pair0 + blockIdx.y)), tau < nlags
-struct MsdIo {
-    const mdp_c64 *x;
-    mdp_c64 *y;
+// the first forward pass reads the centred series of unit u (utab = {c0, c1, group}, c1 = -1 for zero)
+struct MsdSeriesIn {
     const double *a, *b, *ma, *mb;
     const int *utab;
-    const long long *goff;
-    const double *pre, *suf;
-    double *out;
-    long long T, nlags, n;
-    int self, ngroups, pair0;
-};
-
-template <int IO>
-struct MsdIn {
-    const MsdIo &io;
-    long long u;
-    __device__ __forceinline__ mdp_c64 operator()(long long i) const
+    long long T;
+    int self;
+    __device__ __forceinline__ mdp_c64 operator()(long long u, long long i, long long) const
     {
-        if (IO != 1) return io.x[u * io.n + i];
         mdp_c64 v;
         v.re = 0.0;
         v.im = 0.0;
-        if (i < io.T) {
-            const int c0 = io.utab[3 * u], c1 = io.utab[3 * u + 1];
-            v.re = __ldg(io.a + (long long)c0 * io.T + i) - __ldg(io.ma + c0);
-            if (!io.self) v.im = __ldg(io.b + (long long)c0 * io.T + i) - __ldg(io.mb + c0);
-            else if (c1 >= 0) v.im = __ldg(io.a + (long long)c1 * io.T + i) - __ldg(io.ma + c1);
+        if (i < T) {
+            const int c0 = utab[3 * u], c1 = utab[3 * u + 1];
+            v.re = __ldg(a + (long long)c0 * T + i) - __ldg(ma + c0);
+            if (!self) v.im = __ldg(b + (long long)c0 * T + i) - __ldg(mb + c0);
+            else if (c1 >= 0) v.im = __ldg(a + (long long)c1 * T + i) - __ldg(ma + c1);
         }
         return v;
     }
 };
 
-template <int IO>
-struct MsdOut {
-    const MsdIo &io;
-    long long u;
-    __device__ __forceinline__ void operator()(long long i, const mdp_c64 &v) const
+// the last inverse pass writes out[g][tau], out[g+1][tau] of inverse transform j0 + u, tau < nlags (the groups are one bin
+// of mdp_fft_pair_groups)
+struct MsdEpilogueOut {
+    const long long *goff;
+    const double *pre, *suf;
+    double *out;
+    long long T, nlags;
+    int ngroups, j0;
+    __device__ __forceinline__ void operator()(long long u, long long i, long long n, const mdp_c64 &v) const
     {
-        if (IO != 2) {
-            io.y[u * io.n + i] = v;
-            return;
-        }
-        if (i >= io.nlags) return;
+        if (i >= nlags) return;
         // an empty group is exactly zero (its transform partner would leave round-off in its half of the transform)
-        const long long g = 2 * (io.pair0 + u), T1 = io.T + 1;
-        io.out[g * io.nlags + i] = io.goff[g + 1] == io.goff[g] ? 0.0
-            : mdp_msd_epilogue(io.suf + g * T1, io.pre + g * T1, io.T, i, v.re / (double)io.n);
-        if (g + 1 < io.ngroups)
-            io.out[(g + 1) * io.nlags + i] = io.goff[g + 2] == io.goff[g + 1] ? 0.0
-                : mdp_msd_epilogue(io.suf + (g + 1) * T1, io.pre + (g + 1) * T1, io.T, i, v.im / (double)io.n);
+        const mdp_fft_group_pair gp = mdp_fft_pair_groups(j0 + u, ngroups);
+        const long long g = gp.first, T1 = T + 1;
+        out[g * nlags + i] = goff[g + 1] == goff[g] ? 0.0 : mdp_msd_epilogue(suf + g * T1, pre + g * T1, T, i, v.re / (double)n);
+        if (gp.partner)
+            out[(g + 1) * nlags + i] = goff[g + 2] == goff[g + 1] ? 0.0
+                : mdp_msd_epilogue(suf + (g + 1) * T1, pre + (g + 1) * T1, T, i, v.im / (double)n);
     }
 };
-
-template <int R, int IO>
-__global__ void __launch_bounds__(MF_THREADS) k_msd_fft_pass(const MsdIo io, const mdp_c64 *__restrict__ W, int t)
-{
-    const long long i = (long long)blockIdx.x * MF_THREADS + threadIdx.x;
-    if (i >= (io.n >> R)) return;
-    const long long u = blockIdx.y;
-    mdp_fft_radix_pass<R>(MsdIn<IO>{io, u}, MsdOut<IO>{io, u}, W, i, t, io.n);
-}
-
-template <int IO>
-void launch_msd_pass(int R, const MsdIo &io, const mdp_c64 *W, int t, int units, cudaStream_t st)
-{
-    const dim3 g((unsigned)ceil_div<long long>(std::max<long long>(io.n >> R, 1), MF_THREADS), (unsigned)units);
-    if (R == 3) k_msd_fft_pass<3, IO><<<g, MF_THREADS, 0, st>>>(io, W, t);
-    else if (R == 2) k_msd_fft_pass<2, IO><<<g, MF_THREADS, 0, st>>>(io, W, t);
-    else k_msd_fft_pass<1, IO><<<g, MF_THREADS, 0, st>>>(io, W, t);
-}
 
 // grid (ceil((n/2 + 1) / MF_THREADS), groups g_lo + blockIdx.y): acc[g][k] += spectra of the units of g in [u0, u1)
 __global__ void __launch_bounds__(MF_THREADS) k_msd_spec_acc(const mdp_c64 *__restrict__ Z, long long n, const long long *__restrict__ uoff,
@@ -198,19 +163,6 @@ __global__ void __launch_bounds__(MF_THREADS) k_msd_spec_acc(const mdp_c64 *__re
         s += self ? mdp_msd_spectrum_self(z, k, n) : mdp_msd_spectrum_cross(z, k, n);
     }
     acc[g * H + k] = s;
-}
-
-// grid (ceil(n / MF_THREADS), pairs): x[j][k] = acc[2 (pair0 + j)][fold k] + i acc[2 (pair0 + j) + 1][fold k]
-__global__ void __launch_bounds__(MF_THREADS) k_msd_spec_load(const double *__restrict__ acc, long long n, int ngroups, int pair0,
-                                                              mdp_c64 *__restrict__ x)
-{
-    const long long k = (long long)blockIdx.x * MF_THREADS + threadIdx.x;
-    if (k >= n) return;
-    const long long H = n / 2 + 1, g = 2 * ((long long)pair0 + blockIdx.y), kk = mdp_msd_fold(k, n);
-    mdp_c64 v;
-    v.re = acc[g * H + kk];
-    v.im = g + 1 < ngroups ? acc[(g + 1) * H + kk] : 0.0;
-    x[(long long)blockIdx.y * n + k] = v;
 }
 
 } // namespace
@@ -286,8 +238,7 @@ int mdp_cross_msd_fft(mdp_ctx *ctx, int nchan, int64_t T, const double *a, const
     MDP_CUDA(cudaMemcpyAsync(d_uoff, uoff.data(), uoff.size() * 8, cudaMemcpyHostToDevice, st));
     MDP_CUDA(cudaMemcpyAsync(d_goff, goff.data(), goff.size() * 8, cudaMemcpyHostToDevice, st));
     MDP_CUDA(cudaMemsetAsync(acc, 0, (size_t)ngroups * H * 8, st));
-    k_msd_twiddle<<<(unsigned)ceil_div<long long>(std::max<long long>(n / 2, 1), MF_THREADS), MF_THREADS, 0, st>>>(W, n);
-    MDP_LAUNCHED(ctx);
+    mdp_fft_twiddles(ctx, W, n, st);
     k_msd_mean<<<dim3((unsigned)nchan, self ? 1 : 2), MDP_MSD_MEAN_LANES, 0, st>>>(a, b, T, ma, mb);
     MDP_LAUNCHED(ctx);
     k_msd_psum<<<dim3((unsigned)ceil_div<long long>(T, MF_THREADS), (unsigned)ngroups), MF_THREADS, 0, st>>>(a, b, ma, mb, d_goff, T,
@@ -296,49 +247,28 @@ int mdp_cross_msd_fft(mdp_ctx *ctx, int nchan, int64_t T, const double *a, const
     k_msd_scan<<<(unsigned)ngroups, MF_SCAN_THREADS, 0, st>>>(psum, T, pre, suf);
     MDP_LAUNCHED(ctx);
 
-    MsdIo io{nullptr, nullptr, a, b, ma, mb, d_utab, d_goff, pre, suf, out, T, nlags, n, self, ngroups, 0};
     int g_lo = 0;
     for (long long u0 = 0; u0 < U; u0 += batch) {                    // forward transforms and spectrum accumulation
         const long long u1 = std::min(U, u0 + batch);
-        io.utab = d_utab + 3 * u0;
-        mdp_c64 *src = x, *dst = y;
-        for (int t = 0; t < p;) {
-            const int R = mdp_fft_pass_radix(t, p);
-            io.x = src;
-            io.y = dst;
-            if (t == 0) launch_msd_pass<1>(R, io, W, t, (int)(u1 - u0), st);
-            else launch_msd_pass<0>(R, io, W, t, (int)(u1 - u0), st);
-            MDP_LAUNCHED(ctx);
-            std::swap(src, dst);
-            t += R;
-        }
+        const mdp_c64 *Z = mdp_fft_transform(ctx, MsdSeriesIn{a, b, ma, mb, d_utab + 3 * u0, T, self}, FftArrayOut{}, x, y, W, p,
+                                             (int)(u1 - u0), st);
         while (uoff[(size_t)g_lo + 1] <= u0) ++g_lo;                 // first group with a unit in [u0, u1)
         int g_hi = g_lo;
         while (uoff[(size_t)g_hi + 1] < u1) ++g_hi;                  // last one
         k_msd_spec_acc<<<dim3((unsigned)ceil_div<long long>(H, MF_THREADS), (unsigned)(g_hi - g_lo + 1)), MF_THREADS, 0, st>>>(
-            src, n, d_uoff, g_lo, u0, u1, self, acc);
+            Z, n, d_uoff, g_lo, u0, u1, self, acc);
         MDP_LAUNCHED(ctx);
     }
-    const int pairs = (ngroups + 1) / 2;
+    const int pairs = (int)mdp_fft_transforms_per_bin(ngroups);
     for (int j0 = 0; j0 < pairs; j0 += (int)batch) {                 // inverse transforms, two groups each
         const int nj = (int)std::min<long long>(batch, pairs - j0);
-        k_msd_spec_load<<<dim3((unsigned)ceil_div<long long>(n, MF_THREADS), (unsigned)nj), MF_THREADS, 0, st>>>(acc, n, ngroups, j0, x);
+        k_fft_spec_load<<<dim3((unsigned)ceil_div<long long>(n, MDP_FFT_THREADS), (unsigned)nj), MDP_FFT_THREADS, 0, st>>>(acc, n, ngroups,
+                                                                                                                     j0, x);
         MDP_LAUNCHED(ctx);
-        io.pair0 = j0;
-        mdp_c64 *src = x, *dst = y;
-        for (int t = 0; t < p;) {
-            const int R = mdp_fft_pass_radix(t, p);
-            io.x = src;
-            io.y = dst;
-            if (t + R == p) launch_msd_pass<2>(R, io, W, t, nj, st);
-            else launch_msd_pass<0>(R, io, W, t, nj, st);
-            MDP_LAUNCHED(ctx);
-            std::swap(src, dst);
-            t += R;
-        }
+        mdp_fft_transform(ctx, FftArrayIn{x}, MsdEpilogueOut{d_goff, pre, suf, out, T, nlags, ngroups, j0}, x, y, W, p, nj, st);
     }
     ctx->timer_end(tk, st);
-    return mdp_check_launch("k_msd_fft_pass");
+    return mdp_check_launch("k_fft_pass");
 }
 
 } // extern "C"

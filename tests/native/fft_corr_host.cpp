@@ -3,36 +3,7 @@
 #include <stdint.h>
 #include <vector>
 
-#include "../../mdproptools_b200/csrc/fft_corr.h"
-
-namespace {
-
-struct HostIn {
-    const mdp_c64 *x;
-    mdp_c64 operator()(long long i) const { return x[i]; }
-};
-struct HostOut {
-    mdp_c64 *y;
-    void operator()(long long i, const mdp_c64 &v) const { y[i] = v; }
-};
-
-// one transform in fused passes, with the pass schedule of mdp_xcorr_fft; returns the array that holds the result
-mdp_c64 *fft_fused(mdp_c64 *src, mdp_c64 *dst, const mdp_c64 *W, int p, long long n)
-{
-    for (int t = 0; t < p;) {
-        const int R = mdp_fft_pass_radix(t, p);
-        for (long long i = 0; i < (n >> R); ++i) {
-            if (R == 3) mdp_fft_radix_pass<3>(HostIn{src}, HostOut{dst}, W, i, t, n);
-            else if (R == 2) mdp_fft_radix_pass<2>(HostIn{src}, HostOut{dst}, W, i, t, n);
-            else mdp_fft_radix_pass<1>(HostIn{src}, HostOut{dst}, W, i, t, n);
-        }
-        mdp_c64 *tmp = src; src = dst; dst = tmp;
-        t += R;
-    }
-    return src;
-}
-
-} // namespace
+#include "fft_host.h"
 
 // the fused passes against p single radix-2 stages on the same data: number of values that differ in any bit
 extern "C" long long fft_fused_vs_radix2(const double *re, const double *im, int p)
@@ -73,6 +44,6 @@ extern "C" int emulate_fft_xcorr(const double *a, const double *b, long long T, 
     for (long long k = 0; k < n; ++k) dst[k] = mdp_cross_spectrum_conj(src, k, n);
     src = fft_fused(dst, src, W.data(), p, n);
     // src = FFT(conj(P)) = N * conj(corr); corr is real
-    for (long long tau = 0; tau < nlags; ++tau) out[tau] = src[tau].re / (double)n / (double)(T - tau);
+    for (long long tau = 0; tau < nlags; ++tau) out[tau] = mdp_fft_unbiased(src[tau].re, n, T, tau);
     return p;
 }

@@ -5,34 +5,7 @@
 #include <vector>
 
 #include "../../mdproptools_b200/csrc/isf_fft.h"
-
-namespace {
-
-struct HostIn {
-    const mdp_c64 *x;
-    mdp_c64 operator()(long long i) const { return x[i]; }
-};
-struct HostOut {
-    mdp_c64 *y;
-    void operator()(long long i, const mdp_c64 &v) const { y[i] = v; }
-};
-
-mdp_c64 *fft_fused(mdp_c64 *src, mdp_c64 *dst, const mdp_c64 *W, int p, long long n)
-{
-    for (int t = 0; t < p;) {
-        const int R = mdp_fft_pass_radix(t, p);
-        for (long long i = 0; i < (n >> R); ++i) {
-            if (R == 3) mdp_fft_radix_pass<3>(HostIn{src}, HostOut{dst}, W, i, t, n);
-            else if (R == 2) mdp_fft_radix_pass<2>(HostIn{src}, HostOut{dst}, W, i, t, n);
-            else mdp_fft_radix_pass<1>(HostIn{src}, HostOut{dst}, W, i, t, n);
-        }
-        mdp_c64 *tmp = src; src = dst; dst = tmp;
-        t += R;
-    }
-    return src;
-}
-
-} // namespace
+#include "fft_host.h"
 
 // rho = (re, im) [nchan][nk][T]; pairs [npairs][2]; bin_off [nbins+1]; out [npairs][nbins][nlags].  Returns log2 N.
 extern "C" int emulate_isf_fft(const double *rho, int nchan, long long nk, long long T, const int *pairs, int npairs,
@@ -59,19 +32,19 @@ extern "C" int emulate_isf_fft(const double *rho, int nchan, long long nk, long 
                 for (long long w = 0; w < H; ++w) a[w] += mdp_isf_spectrum(&Z[(size_t)(pairs[2 * q] * n)], &Z[(size_t)(pairs[2 * q + 1] * n)], w, n);
             }
         }
-    const long long tpb = mdp_isf_transforms_per_bin(npairs);
     for (int b = 0; b < nbins; ++b)
-        for (long long j = 0; j < tpb; ++j) {
-            const long long q = 2 * j, g = b * (long long)npairs + q;
+        for (long long j = 0; j < mdp_fft_transforms_per_bin(npairs); ++j) {
+            const mdp_fft_group_pair gp = mdp_fft_pair_groups(j, npairs);
+            const long long q = gp.first, g = b * (long long)npairs + q;
             for (long long w = 0; w < n; ++w) {
-                const long long ww = mdp_msd_fold(w, n);
+                const long long ww = mdp_fft_fold(w, n);
                 x[(size_t)w].re = acc[(size_t)(g * H + ww)];
-                x[(size_t)w].im = q + 1 < npairs ? acc[(size_t)((g + 1) * H + ww)] : 0.0;
+                x[(size_t)w].im = gp.partner ? acc[(size_t)((g + 1) * H + ww)] : 0.0;
             }
             const mdp_c64 *r = fft_fused(x.data(), y.data(), W.data(), p, n);
             for (long long tau = 0; tau < nlags; ++tau) {
-                out[(q * nbins + b) * nlags + tau] = mdp_isf_epilogue(r[tau].re, n, T, tau);
-                if (q + 1 < npairs) out[((q + 1) * nbins + b) * nlags + tau] = mdp_isf_epilogue(r[tau].im, n, T, tau);
+                out[(q * nbins + b) * nlags + tau] = mdp_fft_unbiased(r[tau].re, n, T, tau);
+                if (gp.partner) out[((q + 1) * nbins + b) * nlags + tau] = mdp_fft_unbiased(r[tau].im, n, T, tau);
             }
         }
     return p;

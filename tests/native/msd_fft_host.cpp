@@ -5,32 +5,9 @@
 #include <vector>
 
 #include "../../mdproptools_b200/csrc/msd_fft.h"
+#include "fft_host.h"
 
 namespace {
-
-struct HostIn {
-    const mdp_c64 *x;
-    mdp_c64 operator()(long long i) const { return x[i]; }
-};
-struct HostOut {
-    mdp_c64 *y;
-    void operator()(long long i, const mdp_c64 &v) const { y[i] = v; }
-};
-
-mdp_c64 *fft_fused(mdp_c64 *src, mdp_c64 *dst, const mdp_c64 *W, int p, long long n)
-{
-    for (int t = 0; t < p;) {
-        const int R = mdp_fft_pass_radix(t, p);
-        for (long long i = 0; i < (n >> R); ++i) {
-            if (R == 3) mdp_fft_radix_pass<3>(HostIn{src}, HostOut{dst}, W, i, t, n);
-            else if (R == 2) mdp_fft_radix_pass<2>(HostIn{src}, HostOut{dst}, W, i, t, n);
-            else mdp_fft_radix_pass<1>(HostIn{src}, HostOut{dst}, W, i, t, n);
-        }
-        mdp_c64 *tmp = src; src = dst; dst = tmp;
-        t += R;
-    }
-    return src;
-}
 
 double mean(const double *x, long long T)
 {
@@ -78,17 +55,19 @@ extern "C" int emulate_cross_msd(const double *a, const double *b, long long T, 
                 acc[(size_t)(g * H + k)] += self ? mdp_msd_spectrum_self(Z, k, n) : mdp_msd_spectrum_cross(Z, k, n);
         }
     }
-    for (int g = 0; g < ngroups; g += 2) {
+    for (long long j = 0; j < mdp_fft_transforms_per_bin(ngroups); ++j) {
+        const mdp_fft_group_pair gp = mdp_fft_pair_groups(j, ngroups);
+        const long long g = gp.first;
         for (long long k = 0; k < n; ++k) {
-            const long long kk = mdp_msd_fold(k, n);
+            const long long kk = mdp_fft_fold(k, n);
             x[(size_t)k].re = acc[(size_t)(g * H + kk)];
-            x[(size_t)k].im = g + 1 < ngroups ? acc[(size_t)((g + 1) * H + kk)] : 0.0;
+            x[(size_t)k].im = gp.partner ? acc[(size_t)((g + 1) * H + kk)] : 0.0;
         }
         const mdp_c64 *r = fft_fused(x.data(), y.data(), W.data(), p, n);
         for (long long tau = 0; tau < nlags; ++tau) {
             out[g * nlags + tau] = group_off[g + 1] == group_off[g] ? 0.0
                 : mdp_msd_epilogue(&suf[(size_t)(g * (T + 1))], &pre[(size_t)(g * (T + 1))], T, tau, r[tau].re / (double)n);
-            if (g + 1 < ngroups)
+            if (gp.partner)
                 out[(g + 1) * nlags + tau] = group_off[g + 2] == group_off[g + 1] ? 0.0
                     : mdp_msd_epilogue(&suf[(size_t)((g + 1) * (T + 1))], &pre[(size_t)((g + 1) * (T + 1))], T, tau,
                                        r[tau].im / (double)n);

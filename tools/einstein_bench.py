@@ -13,7 +13,7 @@ are integrated chunk by chunk, so the [T][3][50 000] trajectory (120 GB at 10^5 
   * nernst_msd     the Nernst-Einstein MSD: mdp_cross_msd_fft on [M][3] = 15 000 self channels grouped by type,
              max_lag = T/2 (CUDA events), against mdp_msd_all_origins on the same centres (CUDA events), results compared
              to the accuracy contract (1e-10 of the maximum); in a separate torch.profiler pass the kernel time of the
-             FFT passes (k_msd_fft_pass) and their rate at 32 B per point and pass.
+             FFT passes (k_fft_pass) and their rate at 32 B per point and pass.
 
 Achieved GB/s are bytes computed here over measured time; the card's name and power limit are read in the same run.
 Writes nothing unless --out is given.  Needs a GPU: there is no CPU path.
@@ -155,16 +155,16 @@ def main():
         torch.cuda.synchronize()
     kt = {}
     for e in prof.key_averages():
-        m = re.search(r"(k_msd_\w+)", e.key)
+        m = re.search(r"(k_(?:msd|fft)_\w+)", e.key)
         if m:
             kt[m.group(1)] = kt.get(m.group(1), 0.0) + e.device_time_total / 1e3
     res["nernst_msd"]["kernel_ms"] = kt
-    if "k_msd_fft_pass" in kt:
+    if "k_fft_pass" in kt:
         peak = json.load(open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "profiles",
                                            "peaks_b200.json")))["stream_read_gbs"]
         p = int(np.ceil(np.log2(T + T // 2)))
         inv = 32.0 * (1 << p) * (-(-p // 3)) * 1                        # one inverse transform (two groups)
-        g = (fwd + inv) / kt["k_msd_fft_pass"] / 1e6
+        g = (fwd + inv) / kt["k_fft_pass"] / 1e6
         res["nernst_msd"]["fft_pass_gbs"] = g
         res["nernst_msd"]["fft_pass_share_of_stream_read"] = g / peak
         res["nernst_msd"]["stream_read_gbs"] = peak
