@@ -48,7 +48,8 @@ int64_t mdp_ctx_launch_count(mdp_ctx *ctx);
  * 2 = streaming MSD kernel, 3 = correlation kernel, 4 = charge-flux kernel, 5 = windowed (all-origins) MSD kernel,
  * 6 = bitmask autocorrelation kernel, 7 = FFT all-origins MSD (the whole of mdp_cross_msd_fft), 8 = structure factor (the
  * whole of mdp_structure_factor: kernels k_sk_sort, k_sk_rho, k_sk_bins; and of mdp_sk_rho: k_sk_sort, k_sk_rho), 9 = binned
- * FFT correlation of complex series (the whole of mdp_isf_fft: kernels k_isf_*).  mdp_ctx_timing_read synchronises
+ * FFT correlation of complex series (the whole of mdp_isf_fft: kernels k_isf_*), 10 = grouped FFT autocorrelation (the
+ * whole of mdp_group_acf_fft: kernels k_fft_*, k_msd_spec_acc).  mdp_ctx_timing_read synchronises
  * on the recorded events, returns the summed milliseconds and the number of launches, and clears them. */
 int mdp_ctx_timing(mdp_ctx *ctx, int enable);
 int mdp_ctx_timing_read(mdp_ctx *ctx, int tag, double *ms_total, int64_t *count);
@@ -254,6 +255,20 @@ int mdp_xcorr_fft(mdp_ctx *ctx, int nchan, int64_t T, const double *a, const dou
  * context's scratch limit. */
 int mdp_cross_msd_fft(mdp_ctx *ctx, int nchan, int64_t T, const double *a, const double *b, int ngroups, const int64_t *group_off,
                       int64_t nlags, double *out, void *stream);
+/* Grouped all-origins autocorrelation through the same FFT pipeline (csrc/msd_fft.h: mdp_acf_epilogue; the velocity
+ * autocorrelation of Diffusion.get_vacf; defined by the long-double direct sum of tests/vacf_oracle.py):
+ *   out[g][tau] = sum_{c in group g} (1/(T-tau)) sum_{t < T-tau} a_c(t+tau) * a_c(t),   tau < nlags.
+ * a = DEVICE [nchan][T], not centred (a mean, such as a velocity drift, is part of the result); group_off, nlags and out as
+ * for mdp_cross_msd_fft (b = NULL): group_off = HOST int64 [ngroups+1], non-decreasing from 0 to nchan, empty groups
+ * allowed (written as exactly 0), 1 <= ngroups <= 65535; 1 <= nlags <= T; out = DEVICE [ngroups][nlags], overwritten.  Two
+ * channels of a group per forward transform, the spectra summed per group in the frequency domain, one inverse transform
+ * per two groups: O(nchan N log N) with N = 2^p >= T + nlags, p <= 30, and no [nchan][nlags] intermediate.  Agrees with the
+ * direct long-double sum to 1e-10 of max_tau |out[g]| (= out[g][0]) for T <= 10^5.  Fixed summation order, no atomics:
+ * run-to-run bit-identical, and the same bits under any scratch limit that admits the call.  Scratch: group accumulators of
+ * ngroups * (N/2 + 1) * 8 bytes plus the sub-batch work arrays.  MDP_ERR_ARG for every argument mdp_cross_msd_fft rejects
+ * and for accumulators above the context's scratch limit. */
+int mdp_group_acf_fft(mdp_ctx *ctx, int nchan, int64_t T, const double *a, int ngroups, const int64_t *group_off, int64_t nlags,
+                      double *out, void *stream);
 /* cumulative trapezoid along rows (conductivity.py:231 with leading zero, viscosity.py:151 without):
  * in = DEVICE [nrows][T]; out = DEVICE [nrows][T] if leading_zero else [nrows][T-1]; out = scale*integral. */
 int mdp_cumtrapz(mdp_ctx *ctx, int nrows, int64_t T, const double *in, double dx, double scale,

@@ -69,6 +69,7 @@ _PROTOS = {
     "mdp_xcorr_fft": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "mdp_cross_msd_fft": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int, POINTER(c_int64), c_int64, c_void_p,
                                   c_void_p]),
+    "mdp_group_acf_fft": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_int, POINTER(c_int64), c_int64, c_void_p, c_void_p]),
     "mdp_structure_factor": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int64, c_int, POINTER(c_double), c_int64,
                                      POINTER(c_int32), c_int, POINTER(c_int64), c_void_p, c_void_p]),
     "mdp_sk_rho": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int64, c_int, POINTER(c_double), c_int64, POINTER(c_int32),

@@ -1,5 +1,5 @@
 // msd_fft.h -- mean-square displacement over all time origins through the Stockham FFT of fft_corr.h (host/device shared
-// bodies of the kernels in msdfft.cu; exercised on the host by tests/native/msd_fft_host.cpp).
+// bodies of the kernels in msdfft.cu; exercised on the host by tests/native/msd_fft_host.cpp and acf_fft_host.cpp).
 //
 // out[g][tau] = sum_{c in group g} (1/(T-tau)) sum_{t < T-tau} (a_c(t+tau) - a_c(t)) * (b_c(t+tau) - b_c(t)),  tau < nlags
 //
@@ -38,6 +38,17 @@ MDP_HD double mdp_msd_spectrum_cross(const mdp_c64 *Z, long long k, long long n)
 MDP_HD double mdp_msd_epilogue(const double *suf, const double *pre, long long T, long long tau, double xc)
 {
     return ((suf[tau] + pre[T - tau]) - xc) / (double)(T - tau);
+}
+
+// Grouped autocorrelation (mdp_group_acf_fft, the self case without centring; emulated by tests/native/acf_fft_host.cpp):
+//   out[g][tau] = sum_{c in group g} (1/(T-tau)) sum_{t < T-tau} a_c(t+tau) * a_c(t)
+// The group's summed self spectrum is 2 sum_c |A_c|^2 (mdp_msd_spectrum_self), whose inverse transform is N times twice
+// the lag-tau sum: out = 0.5 * x / N / (T - tau) of element tau (x = its real or imaginary part).  The series are not
+// centred: a mean (a velocity drift) is part of this result.  Same contract as the MSD: 1e-10 of max_tau |out[g]|, which
+// is out[g][0], for T <= 10^5.
+MDP_HD double mdp_acf_epilogue(double x, long long n, long long T, long long tau)
+{
+    return 0.5 * x / (double)n / (double)(T - tau);
 }
 
 // the mean of a channel in a fixed order: lane l of MDP_MSD_MEAN_LANES sums t = l, l + lanes, ... (mdp_msd_lane_sum),

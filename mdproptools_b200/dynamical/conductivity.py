@@ -30,7 +30,7 @@ from ..common import constants
 from ..common.com_mols import atom_masses, mol_membership
 from ..io import dump as _dump
 from ..io.pipeline import FrameBatches
-from .diffusion import position_columns, unwrapped_positions
+from .diffusion import fit_window, position_columns, unwrapped_positions
 
 
 def even_times(steps, units, timestep, source, who="the Einstein and Nernst-Einstein conductivity need"):
@@ -363,17 +363,11 @@ class Conductivity:
         return out.cpu().numpy()
 
     def _fit_window(self, max_lag, initial_time, final_time):
-        """Lag times l * dt (l < max_lag) and the mask of the fit window: by default the lags max(1, max_lag // 10) to
-        max_lag - 1."""
+        """Lag times l * dt (l < max_lag) and the mask of the fit window (``fit_window``: by default the lags
+        max(1, max_lag // 10) to max_lag - 1)."""
         dt = self.time[1] - self.time[0] if len(self.time) > 1 else 0.0
         t = np.arange(max_lag) * dt
-        lo = t[min(max(1, max_lag // 10), max_lag - 1)] if initial_time is None else initial_time
-        hi = t[max_lag - 1] if final_time is None else final_time
-        mask = (t >= lo) & (t <= hi)
-        if max_lag < 2 or mask.sum() < 2:
-            raise ValueError(f"the fit window [{lo}, {hi}] holds {int(mask.sum()) if max_lag >= 2 else 0} lag times; "
-                             "at least 2 are needed")
-        return t, mask
+        return t, fit_window(t, initial_time, final_time)
 
     @staticmethod
     def _slope(t, y):

@@ -6,6 +6,9 @@ Device work (csrc/reduce.cu): molecule centres of mass of unwrapped coordinates 
 displacements from the Time==0 frame and their per-group sums (:212-218) as a streaming fp64 reduction over
 ``[T][3][N]`` SoA frames, the strided-interval MSD (:225-237), the OLS sums of calc_diff (:323-329), and --
 beyond the reference -- the windowed MSD over all time origins (``get_msd_all_origins``).
+Green-Kubo route (``get_vacf``, ``calc_diff_green_kubo``, ``get_vdos``; no reference counterpart): the velocity
+autocorrelation over all time origins per (type, axis) group through the grouped FFT autocorrelation mdp_group_acf_fft
+(csrc/msdfft.cu) and its running integral (mdp_cumtrapz); the vibrational density of states is a DCT-I of each VACF.
 Host work: unit tables, DataFrame shaping/column names (:211-222), artefact files.
 
 Multi-GPU: atoms (or molecules) are split in contiguous blocks over the ranks; per-frame partial sums are
@@ -52,6 +55,39 @@ def unwrapped_positions(dev, metas, k0, have_u):
         return dev[:, k0:k0 + 3, :]
     L = torch.tensor([m.box.bound_lengths() for m in metas], dtype=torch.float64, device=dev.device)
     return dev[:, k0:k0 + 3, :] + dev[:, k0 + 3:k0 + 6, :] * L[:, :, None]      # x.add(ix.multiply(L)) (:78-80)
+
+
+def fit_window(t, initial_time=None, final_time=None):
+    """Mask of the lag times ``t`` (l * dt, l < L) inside [initial_time, final_time]; by default the lags max(1, L // 10)
+    to L - 1, which leaves out the first tenth of the curve.  ValueError when the window holds fewer than 2 lag times."""
+    L = len(t)
+    lo = t[min(max(1, L // 10), L - 1)] if initial_time is None else initial_time
+    hi = t[L - 1] if final_time is None else final_time
+    mask = (t >= lo) & (t <= hi)
+    if L < 2 or mask.sum() < 2:
+        raise ValueError(f"the fit window [{lo}, {hi}] holds {int(mask.sum()) if L >= 2 else 0} lag times; "
+                         "at least 2 are needed")
+    return mask
+
+
+VDOS_WINDOWS = ("hann", "none")
+
+
+def vdos_transform(c, dt, window="hann"):
+    """(nu [L], S [L]) of one autocorrelation c [L] (a float64 torch tensor on any device) with lag step dt, L >= 2:
+    the DCT-I  X_k = w_0 c_0 + (-1)^k w_{L-1} c_{L-1} + 2 sum_{l=1}^{L-2} w_l c_l cos(pi k l / (L-1)),
+    S(nu_k) = 2 dt X_k / c_0 at nu_k = k / (2 (L-1) dt), with w_l = 0.5 (1 + cos(pi l / (L-1))) ("hann") or 1 ("none").
+    The DCT-I is the real part of the FFT of the even extension (c_0 .. c_{L-1} .. c_1).  The trapezoid area of S over nu
+    is w_0 = 1, and S(0) c_0 / 4 is the trapezoid integral of w c."""
+    if window not in VDOS_WINDOWS:
+        raise ValueError(f"window must be one of {VDOS_WINDOWS}, got {window!r}")
+    L = c.shape[0]
+    lag = torch.arange(L, dtype=torch.float64, device=c.device)
+    w = 0.5 * (1.0 + torch.cos(np.pi * lag / (L - 1))) if window == "hann" else torch.ones_like(lag)
+    y = w * c
+    ext = torch.cat([y, y[1:L - 1].flip(0)])                             # length 2 (L - 1)
+    X = torch.fft.rfft(ext).real                                         # L values
+    return lag / (2 * (L - 1) * dt), 2.0 * dt * X / c[0]
 
 
 class Diffusion:
@@ -365,3 +401,152 @@ class Diffusion:
             fig.savefig(f"{self.diff_dir}/diff_dist.png", bbox_inches="tight", pad_inches=0.1)
             plt.close(fig)
         return msd_int
+
+    # ------------------------------------------------------------------------------------------
+    def get_vacf(self, filename, max_lag=None, vacf_type="allatom", num_mols=None, num_atoms_per_mol=None, mass=None):
+        """Velocity autocorrelation over all time origins, C(lag) = < v_i(t0 + lag) . v_i(t0) >_{i, t0}, in m^2/s^2 for
+        lags 0 .. max_lag - 1 (default T // 2) of evenly spaced frames with ``vx vy vz`` columns.
+
+        ``allatom``: one group per atom type (ascending type id; the types must not change between frames), columns
+        ``vxvx{t} vyvy{t} vzvz{t} vacf{t}`` (means over the type's atoms) and ``vacf``, the mean over all atoms.
+        ``com``: mass-weighted centre-of-mass velocities of the molecules (``num_mols``, ``num_atoms_per_mol``; masses from
+        ``mass`` by type, else the dump's ``mass`` column), one group per molecule type labelled 1..ntypes.
+        The first column is ``Time (s)``, the lag times from 0.  Velocities are not centred: a drift is part of C.
+        All (type, axis) groups go through one mdp_group_acf_fft call.  Multi-GPU: every rank parses every frame and
+        keeps a contiguous block of each group's atoms (or molecules); the sums are merged with one fp64 all-reduce."""
+        from .conductivity import even_times
+
+        if vacf_type not in ("allatom", "com"):
+            raise ValueError("vacf_type must be 'allatom' or 'com'.")
+        if max_lag is not None and int(max_lag) < 1:
+            raise ValueError(f"max_lag must be at least 1, got {max_lag}")
+        pattern = f"{self.outputs_dir}/{filename}"
+        cols = _dump.available_columns(pattern)
+        if not cols:
+            raise ValueError(f"no dump frames found for {pattern!r}")
+        if not {"vx", "vy", "vz"} <= set(cols):
+            raise ValueError(f"the velocity autocorrelation needs the dump columns vx vy vz ({pattern!r} has {sorted(cols)})")
+        want = ["id", "type", "vx", "vy", "vz"]
+        com = vacf_type == "com"
+        if com and not mass:
+            assert "mass" in cols, "Missing atom masses in dump file."
+            want.append("mass")
+        dev = torch.device("cuda", torch.cuda.current_device())
+        vs = constants.VELOCITY_CONVERSION[self.units]
+        types0 = sel_d = md = seg_d = None
+        pieces, steps = [], []
+        for batch in FrameBatches(pattern, want):
+            d = batch.wait()
+            host = batch.host.numpy()
+            if types0 is None:
+                types0 = host[0, 1].copy()
+                if com:
+                    _, _, seg_off = mol_membership(num_mols, num_atoms_per_mol)
+                    if seg_off[-1] != len(types0):
+                        raise ValueError(f"Length of values ({seg_off[-1]}) does not match length of index ({len(types0)})")
+                    m_atom = atom_masses(types0, mass) if mass else host[0, batch.col("mass")]
+                    md = torch.from_numpy(np.ascontiguousarray(m_atom, dtype=np.float64)).to(dev)
+                    seg_d = torch.from_numpy(seg_off.astype(np.int32)).to(dev)
+                    labels = [str(k + 1) for k in range(len(num_mols))]
+                    first = np.concatenate(([0], np.cumsum(num_mols))).astype(np.int64)
+                    members = [np.arange(first[g], first[g + 1]) for g in range(len(num_mols))]
+                else:
+                    tids = np.unique(types0)
+                    labels = [str(int(t)) for t in tids]
+                    members = [np.nonzero(types0 == t)[0] for t in tids]
+                # this rank's contiguous block of every group, gathered into group order once per batch
+                local = [idx[slice(*dist.shard_range(len(idx)))] for idx in members]
+                sel_d = torch.from_numpy(np.concatenate(local).astype(np.int64)).to(dev)
+                nloc = [len(idx) for idx in local]
+                counts = np.array([len(idx) for idx in members], dtype=np.float64)
+            if not (host[:, 1] == types0).all():
+                raise ValueError("atom types must be the same in every frame for the velocity autocorrelation")
+            vel = d[:, 2:5, :]
+            if com:
+                vel, _, _ = ops.segment_com(vel.contiguous(), md, seg_d)                 # [F, 3, M]
+            pieces.append(vel.index_select(2, sel_d) * vs)                               # [F, 3, local]
+            steps += [m.timestep for m in batch.metas]
+        times = even_times(steps, self.units, self.timestep, repr(pattern), who="the velocity autocorrelation needs")
+        T = len(steps)
+        max_lag = T // 2 if max_lag is None else min(int(max_lag), T)
+        if max_lag < 1:
+            raise ValueError(f"max_lag must be at least 1 ({T} frames)")
+        v = torch.cat(pieces, dim=0) if len(pieces) > 1 else pieces[0]                   # [T, 3, local]
+        del pieces
+        # channels [group][axis][atom] (groups are (type, axis)), one row per series
+        G = len(nloc)
+        goff = np.concatenate(([0], np.cumsum(np.repeat(nloc, 3)))).astype(np.int64)
+        chans = torch.empty((int(goff[-1]), T), dtype=torch.float64, device=dev)
+        s0 = 0
+        for g in range(G):
+            chans[3 * s0:3 * (s0 + nloc[g])].view(3, nloc[g], T).copy_(v[:, :, s0:s0 + nloc[g]].permute(1, 2, 0))
+            s0 += nloc[g]
+        del v
+        if chans.shape[0]:
+            sums = ops.group_acf_fft(chans, goff, max_lag)                               # [3 G, max_lag]
+        else:                                       # a rank without atoms still joins the all-reduce
+            sums = torch.zeros((3 * G, max_lag), dtype=torch.float64, device=dev)
+        del chans
+        dist.all_reduce_sum_(sums)
+        sums = sums.cpu().numpy().reshape(G, 3, max_lag)
+        out = {"Time (s)": times[:max_lag] - times[0]}
+        for g, lab in enumerate(labels):
+            for k, name in enumerate(["vxvx", "vyvy", "vzvz"]):
+                out[f"{name}{lab}"] = sums[g, k] / counts[g]
+            out[f"vacf{lab}"] = sums[g].sum(axis=0) / counts[g]
+        if not com:
+            out["vacf"] = sums.sum(axis=(0, 1)) / counts.sum()
+        return pd.DataFrame(out)
+
+    def calc_diff_green_kubo(self, vacf, initial_time=None, final_time=None, dimension=3, diff_names=None, save=False):
+        """Green-Kubo self-diffusion D = (1/dimension) integral of the VACF, for every ``vacf*`` column of ``get_vacf``.
+        The running integral (trapezoid, leading zero) is formed on the device; D is its mean over the fit window divided
+        by ``dimension`` and ``std`` its standard deviation (ddof 0) over the window divided by ``dimension``.  The window of
+        column ``ind`` runs from ``initial_time[ind]`` to ``final_time[ind]`` (dicts keyed by column index, as in
+        ``calc_diff``), by default over the lags max(1, L // 10) to L - 1.  ``save`` writes vacf_integral.csv and
+        diffusion_gk.csv into ``diff_dir``."""
+        initial_time = initial_time or {}
+        final_time = final_time or {}
+        names = [col for col in vacf.columns if "vacf" in col.lower()]
+        t = vacf["Time (s)"].to_numpy(dtype=np.float64)
+        if len(t) < 2:
+            raise ValueError(f"the Green-Kubo integral needs at least 2 lag times, got {len(t)}")
+        y = torch.from_numpy(np.array(vacf[names].to_numpy(dtype=np.float64).T, order="C")).cuda()
+        integral = ops.cumtrapz(y, float(t[1] - t[0]), 1.0, leading_zero=True).cpu().numpy()     # [columns, L]
+        diff = np.zeros((len(names), 2))
+        for ind, row in enumerate(integral):
+            win = row[fit_window(t, initial_time.get(ind), final_time.get(ind))]
+            diff[ind] = [win.mean() / dimension, win.std() / dimension]
+        diffusion = pd.DataFrame(diff, columns=["diffusion (m2/s)", "std"],
+                                 index=diff_names or [i + 1 for i in range(len(names))])
+        if save and dist.rank() == 0:
+            run = pd.DataFrame(integral.T, columns=names)
+            run.insert(0, "Time (s)", t)
+            run.to_csv(f"{self.diff_dir}/vacf_integral.csv", index=False)
+            diffusion.to_csv(f"{self.diff_dir}/diffusion_gk.csv")
+        return diffusion
+
+    def get_vdos(self, vacf, window="hann", save=False):
+        """Vibrational density of states of every ``vacf*`` column of ``get_vacf``: ``vdos*`` = S(nu) of
+        ``vdos_transform`` (normalised to unit area over nu), with ``Frequency (Hz)`` and ``Wavenumber (cm^-1)`` columns.
+        ValueError for fewer than 2 lags or a column with C(0) = 0.  ``save`` writes vdos.csv into ``diff_dir``."""
+        names = [col for col in vacf.columns if "vacf" in col.lower()]
+        t = vacf["Time (s)"].to_numpy(dtype=np.float64)
+        dt = float(t[1] - t[0]) if len(t) > 1 else 0.0
+        dev = torch.device("cuda", torch.cuda.current_device())
+        out = {}
+        for col in names:
+            c = vacf[col].to_numpy(dtype=np.float64)
+            if len(c) < 2 or c[0] == 0:
+                raise ValueError(f"the VDOS of {col!r} needs at least 2 lags and a nonzero C(0) "
+                                 f"({len(c)} lags, C(0) = {c[0] if len(c) else None})")
+            nu, S = vdos_transform(torch.from_numpy(np.ascontiguousarray(c)).to(dev), dt, window)
+            if not out:
+                nu = nu.cpu().numpy()
+                out["Frequency (Hz)"] = nu
+                out["Wavenumber (cm^-1)"] = nu / constants.LIGHT_SPEED / 100
+            out["vdos" + col[len("vacf"):]] = S.cpu().numpy()
+        vdos = pd.DataFrame(out)
+        if save and dist.rank() == 0:
+            vdos.to_csv(f"{self.diff_dir}/vdos.csv", index=False)
+        return vdos

@@ -298,6 +298,19 @@ def cross_msd_fft(a, b, group_off, nlags):
     return out
 
 
+def group_acf_fft(a, group_off, nlags):
+    """mdp_group_acf_fft: a [C,T], group_off host ints [G+1] -> out [G, nlags] = sum over the group's channels of the
+    all-origins mean of a(t+tau) * a(t) (not centred)."""
+    a = _f64(a, "a")
+    C, T = a.shape
+    garr, gptr = _host_i64(group_off)
+    G = len(garr) - 1
+    ctx = Context.get(a.device.index)
+    out = torch.empty((max(G, 0), max(int(nlags), 0)), dtype=torch.float64, device=a.device)
+    check(lib().mdp_group_acf_fft(ctx.handle, C, T, ptr(a), G, gptr, int(nlags), ptr(out), stream_ptr()), "mdp_group_acf_fft")
+    return out
+
+
 def structure_factor(xyz, cls, ncls, cell, miller, bin_off, nbins):
     """mdp_structure_factor: xyz float64 [F,3,N]; cls int32 [N] or [F,N] or None (one class); cell host (lx, ly, lz, xy, xz,
     yz) shared by the F frames; miller host ints [nk,3] sorted by bin; bin_off host ints [nbins+1] ->
