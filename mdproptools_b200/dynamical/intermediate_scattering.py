@@ -31,9 +31,9 @@ import torch
 from .. import dist, ops
 from .._lib import SK_MAX_CLASSES
 from ..common import constants
+from ..common.frames import _ClassMap, _value_counts, calc_atom_type_ids
 from ..io.dump import dump_files
 from ..io.pipeline import FrameBatches
-from ..structural.rdf_cn import _ClassMap, _value_counts, calc_atom_type_ids
 from ..structural.structure_factor import _cell, kset
 from .conductivity import even_times
 

@@ -27,9 +27,9 @@ import pandas as pd
 import torch
 
 from .. import dist, ops
+from ..common.frames import calc_atom_type_ids
 from ..io import dump as _dump
 from ..io.pipeline import FrameBatches
-from ..structural.rdf_cn import calc_atom_type_ids
 
 
 class ResidenceTime:

@@ -29,9 +29,10 @@ import pandas as pd
 import torch
 
 from .. import _lib, dist, ops
+from ..common.frames import calc_atom_type_ids
 from ..io import dump as _dump
 from ..io.pipeline import FrameBatches
-from .rdf_cn import _mol_segments, calc_atom_type_ids
+from .rdf_cn import _mol_segments
 
 FORCE_CONSTANT = 0.043363 / 16.0  # :28
 

@@ -21,8 +21,9 @@ import numpy as np
 import torch
 
 from .. import dist, ops
+from ..common.frames import _merge_frames, calc_atom_type_ids
 from ..io.pipeline import FrameBatches
-from .rdf_cn import _log, _merge_frames, _num_bins, _save_rdf, calc_atom_type_ids
+from .rdf_cn import _log, _num_bins, _save_rdf
 
 _AXES = {"x": 2, "y": 3, "z": 4}
 

@@ -36,7 +36,9 @@ import torch
 
 from .. import dist, ops
 from .._lib import PAIR_TRICLINIC, bin_edges
-from ..io.pipeline import ArrayBatches, FrameBatches
+from ..common.frames import _ClassMap, _frame_batches, _value_counts, file_sharded, merge_results, typed_batches
+from ..common.frames import calc_atom_type_ids  # noqa: F401  (public under this module's path, as in the reference)
+from ..io.pipeline import ArrayBatches
 
 CON_CONSTANT = 1.660538921  # :30
 
@@ -68,99 +70,6 @@ def _rcut_sq(r_cut) -> float:
         return float(int(r_cut) ** 2)
     r = float(r_cut)
     return r * r
-
-
-def calc_atom_type_ids(ids, num_mols, num_atoms):
-    """_calc_atom_type (:197-215) vectorised: atom id -> 1-based position inside its molecule type block,
-    offset by the atoms-per-molecule of the earlier molecule types.  ids beyond the last block are left as is."""
-    ids = np.asarray(ids, dtype=np.float64)
-    cut = np.cumsum(np.multiply(num_mols, num_atoms))
-    out = ids.copy()
-    which = np.searchsorted(cut, ids, side="left")          # first block with id <= cutoff
-    for i in range(len(cut)):
-        sel = which == i
-        if not sel.any():
-            continue
-        v = np.mod(ids[sel] - cut[i], num_atoms[i])
-        v[v == 0] = num_atoms[i]
-        if i > 0:
-            v = v + np.sum(num_atoms[:i])
-        out[sel] = v
-    return out
-
-
-def _same_values(a, b):
-    """a == b element for element.  Contiguous arrays of one dtype and shape are compared with one memcmp (ctypes releases
-    the GIL; 10^5 doubles take ~50 us, where ``np.array_equal`` builds a temporary and holds the GIL next to the pipeline's
-    reader threads)."""
-    if a is b:
-        return True
-    if a.shape != b.shape:
-        return False
-    if a.dtype == b.dtype and a.flags.c_contiguous and b.flags.c_contiguous:
-        import ctypes
-
-        return _memcmp()(ctypes.c_void_p(a.ctypes.data), ctypes.c_void_p(b.ctypes.data), ctypes.c_size_t(a.nbytes)) == 0
-    return bool(np.array_equal(a, b))
-
-
-def _memcmp():
-    import ctypes
-
-    fn = getattr(_memcmp, "fn", None)
-    if fn is None:
-        fn = ctypes.CDLL(None).memcmp
-        fn.restype = ctypes.c_int
-        fn.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t]
-        _memcmp.fn = fn
-    return fn
-
-
-class _TypeCache:
-    """Per-frame host work that depends only on the frame's id/type column: the altered types, the {type: count} table and
-    the class of every atom.  Trajectories almost always repeat the same column frame after frame; one comparison (tens
-    of microseconds for 10^5 atoms) then replaces ~1 ms of recomputation per frame, which is what the consumer thread of
-    the file pipeline spent next to a pair kernel that needs 0.1 ms per frame."""
-
-    def __init__(self):
-        self.key = None
-        self.val = None
-        self.src = None            # the object last asked about (an identical object needs no comparison at all)
-
-    def get(self, column, make):
-        if column is self.src:
-            return self.val
-        if self.key is None or not _same_values(self.key, column):
-            self.key = np.array(column, copy=True)
-            self.val = make(column)
-        self.src = column if column.base is None else None      # (a view into a staging buffer is not an identity)
-        return self.val
-
-
-class _DeviceCache:
-    """The class vector on the device: uploaded again only when the host vector is another object than last time (a
-    pageable H2D copy waits for the stream -- the consumer would stall behind its own kernels once per batch)."""
-
-    def __init__(self):
-        self.src, self.dev = None, None
-
-    def get(self, arr, device):
-        if arr is not self.src or self.dev is None or self.dev.device != device:
-            self.dev = torch.from_numpy(arr).to(device)
-            self.src = arr
-        return self.dev
-
-
-def _value_counts(typ):
-    """{type: count}, keys ascending.  Types are small non-negative integers in practice: one bincount pass instead of
-    np.unique's sort (this runs once per frame on the host, next to a pair kernel that takes 0.16 ms per frame)."""
-    t = np.asarray(typ).astype(np.int64)
-    if t.size and t.min() >= 0 and t.max() < (1 << 20):
-        c = np.bincount(t)
-        u = np.flatnonzero(c)
-        return dict(zip(u.tolist(), c[u].tolist()))
-    u, c = np.unique(t, return_counts=True)
-    return dict(zip(u.tolist(), c.tolist()))
 
 
 def _calc_props(box_lengths, n_objects, atom_types, object_types, num_types, mass, partial_relations, atom_types_col,
@@ -260,41 +169,6 @@ def _save_cn(relation_matrix, path_or_buff, cn_sum, save_mode):
     return final_df
 
 
-# ------------------------------------------------------------------------------------------------
-# class maps: relation types -> small dense class ids for the device histogram
-# ------------------------------------------------------------------------------------------------
-class _ClassMap:
-    """Types named by the relations get their own class; everything else shares the class 'other'."""
-
-    def __init__(self, named_types, present_types=None):
-        self.named = sorted(set(int(t) for t in named_types))
-        self.index = {t: k for k, t in enumerate(self.named)}
-        # the class 'other' is only materialised when some point actually has an unnamed type (one class fewer
-        # keeps single-species runs on the kernel variant without per-pair class bookkeeping)
-        self.has_other = present_types is None or bool(set(int(t) for t in present_types) - set(self.named))
-        self.ncls = len(self.named) + (1 if self.has_other else 0)
-        self.other = self.ncls - 1 if self.has_other else -1
-
-    def classes_of(self, typ: np.ndarray) -> np.ndarray:
-        t = np.asarray(typ).astype(np.int64)
-        if t.size and t.min() >= 0 and t.max() < (1 << 20):      # one table lookup instead of a mask per named type
-            lut = np.full(int(t.max()) + 1, self.other, dtype=np.int32)
-            for ty, k in self.index.items():
-                if 0 <= ty < len(lut):
-                    lut[ty] = k
-            cls = lut[t]
-        else:
-            cls = np.full(t.shape, self.other, dtype=np.int32)
-            for ty, k in self.index.items():
-                cls[t == ty] = k
-        if not self.has_other and (cls < 0).any():
-            raise ValueError("a frame contains atom types that were absent from the first frame")
-        return cls
-
-    def cls(self, t):
-        return self.index.get(int(t), self.other)
-
-
 def _sym_weights(cmap: _ClassMap, relation_matrix, with_full: bool):
     """hist_reduce weights for the symmetric kernel: g_full counts every pair twice (:85-86); relation (a,b)
     counts a pair once per matching role order (:89-96) -> 2 on the like row, 1 on the unlike row."""
@@ -370,65 +244,6 @@ class _PropsCache:
         return self.val[1:]
 
 
-# ------------------------------------------------------------------------------------------------
-# frame iteration shared by all entry points
-# ------------------------------------------------------------------------------------------------
-class _RetryUnsharded(Exception):
-    """Some rank met a dump file with more than one frame while reading only its share of the files."""
-
-
-_SHARD_FILES = [True]
-
-
-def _frame_batches(filename, columns):
-    """This rank's frames.  With several ranks every rank READS only every world-th file (frame index = file index for the
-    usual one-frame-per-file dumps); ``_agree_sharding`` then checks collectively that no rank met a multi-frame file --
-    otherwise the call is repeated with every rank reading everything and selecting its frames (``file_sharded``)."""
-    w, r = dist.world_size(), dist.rank()
-    if w > 1 and _SHARD_FILES[0]:
-        return FrameBatches(filename, columns, file_shard=(r, w))
-    sel = (lambda i: i % w == r) if w > 1 else None
-    return FrameBatches(filename, columns, frame_select=sel)
-
-
-def _agree_sharding(batches, device):
-    """Call after the batch loop and before the merge collective: all ranks learn whether the sharded read held."""
-    if getattr(batches, "file_shard", None) is None:
-        return
-    flag = torch.tensor([1 if batches.multi_frame_seen else 0], dtype=torch.int64, device=device)
-    dist.all_reduce_max_(flag)
-    if int(flag.item()):
-        raise _RetryUnsharded()
-
-
-def file_sharded(fn):
-    """Decorator of the file-based entry points: run with sharded file reads, fall back (on every rank at once) when a
-    multi-frame file was met."""
-    import functools
-
-    @functools.wraps(fn)
-    def wrapper(*args, **kwargs):
-        try:
-            return fn(*args, **kwargs)
-        except _RetryUnsharded:
-            _SHARD_FILES[0] = False
-            try:
-                return fn(*args, **kwargs)
-            finally:
-                _SHARD_FILES[0] = True
-
-    return wrapper
-
-
-def _merge_frames(per_frame: dict, total_frames: int, shape, device):
-    """Place this rank's per-frame integer results into [T, *shape] and all-reduce (int64, exact)."""
-    out = torch.zeros((total_frames,) + tuple(shape), dtype=torch.int64, device=device)
-    for idx, t in per_frame.items():
-        out[idx] = t
-    dist.all_reduce_sum_(out)
-    return out
-
-
 def _mol_segments(num_mols, num_atoms_per_mol):
     """Molecule membership implied by id order (:222-230): (mol_type[M], seg_off[M+1])."""
     mt = np.repeat(np.arange(1, len(num_mols) + 1), num_mols)
@@ -438,68 +253,103 @@ def _mol_segments(num_mols, num_atoms_per_mol):
 
 
 # ------------------------------------------------------------------------------------------------
-# public API
+# frame loops of the file-based entry points
 # ------------------------------------------------------------------------------------------------
-@file_sharded
-def calc_atomic_rdf(r_cut, bin_size, num_types, mass, partial_relations, filename, num_mols=None, num_atoms_per_mol=None,
-                    path_or_buff="rdf.csv", save_mode=True, mic="reference"):
-    """Full and partial atom-atom RDF; see the reference docstring (:397-452) for the arguments."""
-    flags = _mic_flags(mic)
-    num_bins, radii = _num_bins(r_cut, bin_size)
-    num_relations = len(partial_relations[0])
+def _atomic_counts(filename, num_types, mass, partial_relations, num_mols, num_atoms_per_mol, flags, shard_files, rcut2, edges,
+                   ddr, cumulative):
+    """The frame loop of calc_atomic_rdf (``cumulative=False``: rows g_full and the relations; props (at, rho, rho_pairs,
+    natoms) per frame) and calc_atomic_cn (``cumulative=True``: the relations, cumulative over the cutoff table; props at
+    per frame) -> (counts [T, rows, bins], props of every frame, T)."""
     relation_matrix = np.asarray(partial_relations).transpose()
     altered = bool(num_mols and num_atoms_per_mol)
-    named = list(partial_relations[0]) + list(partial_relations[1])
-    cmap = weights = None          # fixed by the types present in this rank's first frame
-    edges = bin_edges(bin_size, num_bins)
-    rcut2 = _rcut_sq(r_cut)
-
-    batches = _frame_batches(filename, ["id", "type", "x", "y", "z"])
-    counts, props = {}, {}
-    device = torch.device("cuda", torch.cuda.current_device())   # a rank that receives no frames still joins the merge
-    tcache, ccache, dcache = _TypeCache(), _TypeCache(), _DeviceCache()
     pcache = _PropsCache(flags, num_types, mass, partial_relations, "id" if altered else "type", num_atoms_per_mol)
 
-    def _typ_and_counts(col):
-        typ_ = calc_atom_type_ids(col, num_mols, num_atoms_per_mol) if altered else np.array(col, copy=True)
-        return typ_, _value_counts(typ_)
+    def frame_props(meta, at):
+        if not cumulative:
+            _log("The timestep of the current file is: " + str(meta.timestep))
+        return pcache.get(meta, at)
 
+    batches = _frame_batches(filename, ["id", "type", "x", "y", "z"], shard_files)
+    named = list(partial_relations[0]) + list(partial_relations[1])
+    counts, props = {}, {}
+    weights = None          # fixed by the types present in this rank's first frame
+    for b in typed_batches(batches, num_mols, num_atoms_per_mol, frame_props, named=named):
+        if weights is None:
+            weights = _sym_weights(b.cmap, relation_matrix, with_full=not cumulative)
+        boxes = np.array([p[0] for p in b.props], dtype=np.float64)
+        xyz = b.dev[:, 2:5, :].contiguous()
+        hist = ops.pair_hist(xyz, b.classes(0, len(b.metas)), b.cmap.ncls, boxes, rcut2, edges, ddr, flags=flags)
+        red = ops.hist_reduce(hist, weights, cumulative=cumulative)
+        for k, meta in enumerate(b.metas):
+            counts[meta.index] = red[k]
+            props[meta.index] = b.atom_types[k] if cumulative else (b.atom_types[k], *b.props[k][1:], meta.natoms)
+    rows = len(partial_relations[0]) + (0 if cumulative else 1)
+    return merge_results(batches, counts, props, filename, (rows, len(edges) - 1))
+
+
+def _molecular_counts(filename, num_types, mass, partial_relations, num_mols, num_atoms_per_mol, inter, flags, shard_files,
+                      rcut2, edges, ddr, cumulative):
+    """The frame loop of the atom/molecule-COM entry points (:654-902): relation counts between the atoms (with ``inter``
+    the molecule centres) of the types partial_relations[0] and the centres of the molecule types partial_relations[1],
+    cumulative over the cutoff table with ``cumulative`` -> (counts [T, R, bins], props (at, rho_pairs) of every frame, T)."""
+    relation_matrix = np.asarray(partial_relations).transpose()
+    mol_type, seg_off = _mol_segments(num_mols, num_atoms_per_mol)
+    cmap_a = _ClassMap(partial_relations[0])
+    cmap_b = _ClassMap(partial_relations[1])
+    weights = _rect_weights(cmap_a, cmap_b, relation_matrix)
+    mol_types_count = _value_counts(mol_type)
+    batches = _frame_batches(filename, ["id", "type", "x", "y", "z"], shard_files)
+    counts, props = {}, {}
     for batch in batches:
         dev = batch.wait()
         device = dev.device
         F = len(batch.metas)
         host = batch.host.numpy()
-        cls_rows = []
+        n = host.shape[2]
+        if seg_off[-1] != n:
+            raise ValueError(f"Length of values ({seg_off[-1]}) does not match length of index ({n})")
         boxes = np.empty((F, 6 if flags else 3))
-        same_cls, cls_first = True, None
+        cls_a = np.empty((F, n), dtype=np.int32)
         for k, meta in enumerate(batch.metas):
-            _log("The timestep of the current file is: " + str(meta.timestep))
-            typ, at = tcache.get(host[k, 0] if altered else host[k, 1], _typ_and_counts)
-            boxrow, rho, rho_pairs = pcache.get(meta, at)
-            props[meta.index] = (at, rho, rho_pairs, meta.natoms)
-            if cmap is None:
-                cmap = _ClassMap(named, present_types=at.keys())
-                weights = _sym_weights(cmap, relation_matrix, with_full=True)
-            cls_k = ccache.get(typ, cmap.classes_of)
-            same_cls = same_cls and (k == 0 or cls_k is cls_first)
-            cls_first = cls_k if k == 0 else cls_first
-            cls_rows.append(cls_k)
-            boxes[k] = boxrow
+            lengths, boxes[k] = _frame_box(meta.box, flags)
+            at = mol_types_count if inter else _value_counts(host[k, 1])
+            if not inter:
+                cls_a[k] = cmap_a.classes_of(host[k, 1])
+            rho, rho_pairs = _calc_props(lengths, len(mol_type), at, mol_types_count, num_types, mass, partial_relations, "type",
+                                         num_atoms_per_mol)
+            props[meta.index] = (at, rho_pairs)
         xyz = dev[:, 2:5, :].contiguous()
-        # one [N] vector when the batch shares its classes (and no upload at all when it is the previous batch's)
-        cls_d = dcache.get(cls_first, device) if same_cls else torch.from_numpy(np.stack(cls_rows)).to(device)
-        hist = ops.pair_hist(xyz, cls_d, cmap.ncls, boxes, rcut2, edges, bin_size, flags=flags)
-        red = ops.hist_reduce(hist, weights)                      # [F, 1+R, nb]
+        # masses per atom from the type column of the first frame of the batch (:231); types are static per id
+        m_atom = torch.from_numpy(np.array([mass[int(t - 1)] for t in host[0, 1]], dtype=np.float64)).to(device)
+        com, _, _ = ops.segment_com(xyz, m_atom, torch.from_numpy(seg_off.astype(np.int32)).to(device))   # [F,3,M]
+        cls_m = torch.from_numpy(cmap_b.classes_of(mol_type)).to(device)
+        if inter:
+            xyz_a, cls_a_d = com, torch.from_numpy(cmap_a.classes_of(mol_type)).to(device)
+        else:
+            xyz_a, cls_a_d = xyz, torch.from_numpy(cls_a).to(device)
+        hist = ops.pair_hist(xyz_a, cls_a_d, cmap_a.ncls, boxes, rcut2, edges, ddr, xyz_b=com, cls_b=cls_m, ncls_b=cmap_b.ncls,
+                             flags=flags)
+        red = ops.hist_reduce(hist, weights, cumulative=cumulative)
         for k, meta in enumerate(batch.metas):
             counts[meta.index] = red[k]
-    _agree_sharding(batches, device)
-    T = batches.total_frames or 0
-    if T == 0:
-        raise ValueError(f"no dump frames found for {filename!r}")
-    allc = _merge_frames(counts, T, (1 + num_relations, num_bins), device).cpu().numpy()
-    if dist.world_size() > 1:
-        props = _gather_props(props, T)
+    return merge_results(batches, counts, props, filename, (len(partial_relations[0]), len(edges) - 1))
 
+
+# ------------------------------------------------------------------------------------------------
+# public API
+# ------------------------------------------------------------------------------------------------
+@file_sharded
+def calc_atomic_rdf(r_cut, bin_size, num_types, mass, partial_relations, filename, num_mols=None, num_atoms_per_mol=None,
+                    path_or_buff="rdf.csv", save_mode=True, mic="reference", *, shard_files=True):
+    """Full and partial atom-atom RDF; see the reference docstring (:397-452) for the arguments."""
+    flags = _mic_flags(mic)
+    num_bins, radii = _num_bins(r_cut, bin_size)
+    num_relations = len(partial_relations[0])
+    relation_matrix = np.asarray(partial_relations).transpose()
+    edges = bin_edges(bin_size, num_bins)
+    rcut2 = _rcut_sq(r_cut)
+    allc, props, T = _atomic_counts(filename, num_types, mass, partial_relations, num_mols, num_atoms_per_mol, flags,
+                                    shard_files, rcut2, edges, bin_size, cumulative=False)
     rdf_full_sum = np.zeros(num_bins)
     rdf_part_sum = np.zeros((num_relations, num_bins))
     den_cache = {}   # frames of one composition and volume share the divisors of _normalize_rdf (the NVT case: one entry)
@@ -517,76 +367,17 @@ def calc_atomic_rdf(r_cut, bin_size, num_types, mass, partial_relations, filenam
     return _save_rdf(radii, relation_matrix, path_or_buff, save_mode, rdf_part_sum, rdf_full_sum=rdf_full_sum)
 
 
-def _gather_props(props: dict, total_frames: int) -> dict:
-    """Every rank needs every frame's host-side normalisation inputs (tiny python objects)."""
-    import torch.distributed as d
-
-    gathered = [None] * d.get_world_size()
-    d.all_gather_object(gathered, props)
-    out = {}
-    for g in gathered:
-        out.update(g)
-    assert len(out) == total_frames
-    return out
-
-
 @file_sharded
 def calc_atomic_cn(r_cut, bin_size, num_types, mass, partial_relations, filename, num_mols=None, num_atoms_per_mol=None,
-                   path_or_buff="cn.csv", save_mode=True, mic="reference"):
+                   path_or_buff="cn.csv", save_mode=True, mic="reference", *, shard_files=True):
     """Atom-atom coordination numbers, one cutoff per relation (:533-651)."""
     flags = _mic_flags(mic)
     _num_bins(r_cut, bin_size)
     num_relations = len(partial_relations[0])
     relation_matrix = np.asarray(partial_relations).transpose()
-    altered = bool(num_mols and num_atoms_per_mol)
-    named = list(partial_relations[0]) + list(partial_relations[1])
-    cmap = weights = None
     edges, rcut2_max, upto = _cn_edges(r_cut)
-    nthr = len(edges) - 1
-
-    batches = _frame_batches(filename, ["id", "type", "x", "y", "z"])
-    counts, props = {}, {}
-    device = torch.device("cuda", torch.cuda.current_device())   # a rank that receives no frames still joins the merge
-    tcache, ccache, dcache = _TypeCache(), _TypeCache(), _DeviceCache()
-    pcache = _PropsCache(flags, num_types, mass, partial_relations, "id" if altered else "type", num_atoms_per_mol)
-
-    def _typ_and_counts(col):
-        typ_ = calc_atom_type_ids(col, num_mols, num_atoms_per_mol) if altered else np.array(col, copy=True)
-        return typ_, _value_counts(typ_)
-
-    for batch in batches:
-        dev = batch.wait()
-        device = dev.device
-        F = len(batch.metas)
-        host = batch.host.numpy()
-        cls_rows = []
-        boxes = np.empty((F, 6 if flags else 3))
-        same_cls, cls_first = True, None
-        for k, meta in enumerate(batch.metas):
-            typ, at = tcache.get(host[k, 0] if altered else host[k, 1], _typ_and_counts)
-            boxrow = pcache.get(meta, at)[0]
-            props[meta.index] = at
-            if cmap is None:
-                cmap = _ClassMap(named, present_types=at.keys())
-                weights = _sym_weights(cmap, relation_matrix, with_full=False)
-            cls_k = ccache.get(typ, cmap.classes_of)
-            same_cls = same_cls and (k == 0 or cls_k is cls_first)
-            cls_first = cls_k if k == 0 else cls_first
-            cls_rows.append(cls_k)
-            boxes[k] = boxrow
-        xyz = dev[:, 2:5, :].contiguous()
-        cls_d = dcache.get(cls_first, device) if same_cls else torch.from_numpy(np.stack(cls_rows)).to(device)
-        hist = ops.pair_hist(xyz, cls_d, cmap.ncls, boxes, rcut2_max, edges, 0.0, flags=flags)
-        red = ops.hist_reduce(hist, weights, cumulative=True)     # [F, R, nthr] cumulative over thresholds
-        for k, meta in enumerate(batch.metas):
-            counts[meta.index] = red[k]
-    _agree_sharding(batches, device)
-    T = batches.total_frames or 0
-    if T == 0:
-        raise ValueError(f"no dump frames found for {filename!r}")
-    allc = _merge_frames(counts, T, (num_relations, nthr), device).cpu().numpy()
-    if dist.world_size() > 1:
-        props = _gather_props(props, T)
+    allc, props, T = _atomic_counts(filename, num_types, mass, partial_relations, num_mols, num_atoms_per_mol, flags,
+                                    shard_files, rcut2_max, edges, 0.0, cumulative=True)
     cn_sum = np.zeros(num_relations)
     for idx in range(T):
         cn = np.array([allc[idx, kl, upto[kl]] for kl in range(num_relations)], dtype=np.float64)
@@ -595,115 +386,43 @@ def calc_atomic_cn(r_cut, bin_size, num_types, mass, partial_relations, filename
     return _save_cn(relation_matrix, path_or_buff, cn_sum, save_mode)
 
 
-def _molecular_common(filename, num_types, mass, partial_relations, num_mols, num_atoms_per_mol, inter, run_pairs, flags=0):
-    """Shared frame loop of the atom/molecule-COM entry points (:654-902).  ``run_pairs`` gets the device
-    tensors of one batch and returns per-frame integer results [F, R, *]."""
-    num_relations = len(partial_relations[0])
-    relation_matrix = np.asarray(partial_relations).transpose()
-    mol_type, seg_off = _mol_segments(num_mols, num_atoms_per_mol)
-    cmap_a = _ClassMap(partial_relations[0])
-    cmap_b = _ClassMap(partial_relations[1])
-    weights = _rect_weights(cmap_a, cmap_b, relation_matrix)
-    mol_types_count = _value_counts(mol_type)
-    batches = _frame_batches(filename, ["id", "type", "x", "y", "z"])
-    counts, props = {}, {}
-    device = torch.device("cuda", torch.cuda.current_device())   # a rank that receives no frames still joins the merge
-    for batch in batches:
-        dev = batch.wait()
-        device = dev.device
-        F = len(batch.metas)
-        host = batch.host.numpy()
-        n = host.shape[2]
-        if seg_off[-1] != n:
-            raise ValueError(f"Length of values ({seg_off[-1]}) does not match length of index ({n})")
-        boxes = np.empty((F, 6 if flags else 3))
-        cls_a = np.empty((F, n), dtype=np.int32)
-        for k, meta in enumerate(batch.metas):
-            lengths, boxes[k] = _frame_box(meta.box, flags)
-            if inter:
-                at = mol_types_count
-                n_objects = len(mol_type)
-                atc = "type"
-            else:
-                at = _value_counts(host[k, 1])
-                n_objects = len(mol_type)
-                atc = "type"
-                cls_a[k] = cmap_a.classes_of(host[k, 1])
-            rho, rho_pairs = _calc_props(lengths, n_objects, at, mol_types_count, num_types, mass, partial_relations, atc,
-                                         num_atoms_per_mol)
-            props[meta.index] = (at, rho_pairs)
-        xyz = dev[:, 2:5, :].contiguous()
-        # masses per atom from the type column of the first frame of the batch (:231); types are static per id
-        m_atom = torch.from_numpy(np.array([mass[int(t - 1)] for t in host[0, 1]], dtype=np.float64)).to(device)
-        com, _, _ = ops.segment_com(xyz, m_atom, torch.from_numpy(seg_off.astype(np.int32)).to(device))   # [F,3,M]
-        cls_m = torch.from_numpy(cmap_b.classes_of(mol_type)).to(device)
-        if inter:
-            cm_a = _ClassMap(partial_relations[0])
-            res = run_pairs(com, torch.from_numpy(cm_a.classes_of(mol_type)).to(device), cm_a.ncls, com, cls_m,
-                            cmap_b.ncls, boxes, _rect_weights(cm_a, cmap_b, relation_matrix))
-        else:
-            res = run_pairs(xyz, torch.from_numpy(cls_a).to(device), cmap_a.ncls, com, cls_m, cmap_b.ncls, boxes, weights)
-        for k, meta in enumerate(batch.metas):
-            counts[meta.index] = res[k]
-    _agree_sharding(batches, device)
-    T = batches.total_frames or 0
-    if T == 0:
-        raise ValueError(f"no dump frames found for {filename!r}")
-    return counts, props, T, device, relation_matrix, num_relations
-
-
 @file_sharded
 def calc_molecular_rdf(r_cut, bin_size, num_types, mass, partial_relations, filename, num_mols, num_atoms_per_mol,
-                       path_or_buff="rdf_mol.csv", save_mode=True, _inter=False, mic="reference"):
+                       path_or_buff="rdf_mol.csv", save_mode=True, _inter=False, mic="reference", *, shard_files=True):
     """Partial RDF between atoms and molecule centres of mass (:654-756)."""
     flags = _mic_flags(mic)
     num_bins, radii = _num_bins(r_cut, bin_size)
     edges = bin_edges(bin_size, num_bins)
     rcut2 = _rcut_sq(r_cut)
-
-    def run(xa, ca, na, xb, cb, nb_, boxes, w):
-        hist = ops.pair_hist(xa, ca, na, boxes, rcut2, edges, bin_size, xyz_b=xb, cls_b=cb, ncls_b=nb_, flags=flags)
-        return ops.hist_reduce(hist, w)
-
-    counts, props, T, device, relation_matrix, R = _molecular_common(filename, num_types, mass, partial_relations, num_mols,
-                                                                      num_atoms_per_mol, _inter, run, flags)
-    allc = _merge_frames(counts, T, (R, num_bins), device).cpu().numpy()
-    if dist.world_size() > 1:
-        props = _gather_props(props, T)
+    allc, props, T = _molecular_counts(filename, num_types, mass, partial_relations, num_mols, num_atoms_per_mol, _inter,
+                                       flags, shard_files, rcut2, edges, bin_size, cumulative=False)
+    R = len(partial_relations[0])
     rdf_part_sum = np.zeros((R, num_bins))
     for idx in range(T):
         at, rho_pairs = props[idx]
         _, rdf_part = _normalize_rdf(bin_size, rho_pairs, at, partial_relations, R, num_bins, allc[idx].astype(np.float64))
         rdf_part_sum += rdf_part
     rdf_part_sum = rdf_part_sum / T
-    return _save_rdf(radii, relation_matrix, path_or_buff, save_mode, rdf_part_sum)
+    return _save_rdf(radii, np.asarray(partial_relations).transpose(), path_or_buff, save_mode, rdf_part_sum)
 
 
 @file_sharded
 def calc_molecular_cn(r_cut, bin_size, num_types, mass, partial_relations, filename, num_mols, num_atoms_per_mol,
-                      path_or_buff="cn_mol.csv", save_mode=True, mic="reference"):
+                      path_or_buff="cn_mol.csv", save_mode=True, mic="reference", *, shard_files=True):
     """Coordination numbers between atoms and molecule centres of mass (:759-854)."""
     flags = _mic_flags(mic)
     _num_bins(r_cut, bin_size)
     edges, rcut2_max, upto = _cn_edges(r_cut)
-    nthr = len(edges) - 1
-
-    def run(xa, ca, na, xb, cb, nb_, boxes, w):
-        hist = ops.pair_hist(xa, ca, na, boxes, rcut2_max, edges, 0.0, xyz_b=xb, cls_b=cb, ncls_b=nb_, flags=flags)
-        return ops.hist_reduce(hist, w, cumulative=True)
-
-    counts, props, T, device, relation_matrix, R = _molecular_common(filename, num_types, mass, partial_relations, num_mols,
-                                                                      num_atoms_per_mol, False, run, flags)
-    allc = _merge_frames(counts, T, (R, nthr), device).cpu().numpy()
-    if dist.world_size() > 1:
-        props = _gather_props(props, T)
+    allc, props, T = _molecular_counts(filename, num_types, mass, partial_relations, num_mols, num_atoms_per_mol, False, flags,
+                                       shard_files, rcut2_max, edges, 0.0, cumulative=True)
+    R = len(partial_relations[0])
     cn_sum = np.zeros(R)
     for idx in range(T):
         at, _ = props[idx]
         cn = np.array([allc[idx, kl, upto[kl]] for kl in range(R)], dtype=np.float64)
         cn_sum += _normalize_cn(at, partial_relations, cn)
     cn_sum = cn_sum / T
-    return _save_cn(relation_matrix, path_or_buff, cn_sum, save_mode)
+    return _save_cn(np.asarray(partial_relations).transpose(), path_or_buff, cn_sum, save_mode)
 
 
 def calc_atomic_rdf_from_arrays(positions, types, box_lengths, r_cut, bin_size, partial_relations, batch_frames=64,

@@ -29,10 +29,9 @@ import numpy as np
 import pandas as pd
 import torch
 
-from .. import dist, ops
+from .. import ops
 from .._lib import SK_MAX_CLASSES, SK_NLIM
-from .rdf_cn import (_agree_sharding, _ClassMap, _DeviceCache, _frame_batches, _gather_props, _TypeCache, _value_counts,
-                     calc_atom_type_ids, file_sharded)
+from ..common.frames import _ClassMap, _frame_batches, file_sharded, merge_results, typed_batches
 
 
 # ------------------------------------------------------------------------------------------------
@@ -168,7 +167,7 @@ def _save_sk(k, relation_matrix, path_or_buff, save_mode, s_tot, s_part, nk_mean
 # ------------------------------------------------------------------------------------------------
 @file_sharded
 def calc_structure_factor(k_max, bin_size, partial_relations, filename, k_min=None, max_k_per_bin=None, seed=0, num_mols=None,
-                          num_atoms_per_mol=None, path_or_buff="sk.csv", save_mode=True):
+                          num_atoms_per_mol=None, path_or_buff="sk.csv", save_mode=True, *, shard_files=True):
     """Total and partial static structure factor of the frames of ``filename`` (LAMMPS dump(s) with id type x y z).
 
     k_max, bin_size   bins [b bin_size, (b+1) bin_size) for b < int(k_max / bin_size), in 1/A
@@ -182,7 +181,6 @@ def calc_structure_factor(k_max, bin_size, partial_relations, filename, k_min=No
     if nbins < 1:
         raise ValueError(f"k_max = {k_max} is below one bin of {bin_size}")
     relation_matrix = np.asarray(partial_relations).transpose()
-    altered = bool(num_mols and num_atoms_per_mol)
     named = list(partial_relations[0]) + list(partial_relations[1])
     cmap = _ClassMap(named)                 # 'other' always present: the same class rows on every rank
     if cmap.ncls > SK_MAX_CLASSES:
@@ -190,56 +188,32 @@ def calc_structure_factor(k_max, bin_size, partial_relations, filename, k_min=No
     rows = ops.sym_rows(cmap.ncls)
     kcache = _KSetCache(k_max, bin_size, k_min, max_k_per_bin, seed)
 
-    batches = _frame_batches(filename, ["id", "type", "x", "y", "z"])
+    def frame_cell(meta, at):
+        for t in named:
+            if at.get(int(t), 0) == 0:
+                raise ValueError(f"no atom of type {t} in frame {meta.index} (timestep {meta.timestep})")
+        return _cell(meta.box)
+
+    batches = _frame_batches(filename, ["id", "type", "x", "y", "z"], shard_files)
     sums, props = {}, {}
-    device = torch.device("cuda", torch.cuda.current_device())   # a rank that receives no frames still joins the merge
-    tcache, ccache, dcache = _TypeCache(), _TypeCache(), _DeviceCache()
-
-    def _typ_and_counts(col):
-        typ_ = calc_atom_type_ids(col, num_mols, num_atoms_per_mol) if altered else np.array(col, copy=True)
-        return typ_, _value_counts(typ_)
-
-    for batch in batches:
-        dev = batch.wait()
-        device = dev.device
-        host = batch.host.numpy()
-        F = len(batch.metas)
-        cells, cls_rows, ats = [], [], []
-        for k, meta in enumerate(batch.metas):
-            typ, at = tcache.get(host[k, 0] if altered else host[k, 1], _typ_and_counts)
-            for t in named:
-                if at.get(int(t), 0) == 0:
-                    raise ValueError(f"no atom of type {t} in frame {meta.index} (timestep {meta.timestep})")
-            cells.append(_cell(meta.box))
-            cls_rows.append(ccache.get(typ, cmap.classes_of))
-            ats.append(at)
-        xyz = dev[:, 2:5, :]
+    for b in typed_batches(batches, num_mols, num_atoms_per_mol, frame_cell, cmap=cmap):
+        cells, F = b.props, len(b.metas)
+        xyz = b.dev[:, 2:5, :]
         k0 = 0
         while k0 < F:                       # one call per run of frames sharing a cell (all of an NVT batch)
             k1 = k0 + 1
             while k1 < F and cells[k1] == cells[k0]:
                 k1 += 1
             miller, bin_off = kcache.get(cells[k0])
-            same = all(c is cls_rows[k0] for c in cls_rows[k0:k1])
-            cls_d = dcache.get(cls_rows[k0], device) if same else torch.from_numpy(np.stack(cls_rows[k0:k1])).to(device)
+            cls_d = b.classes(k0, k1)
             out = ops.structure_factor(xyz[k0:k1].contiguous(), cls_d, cmap.ncls, cells[k0], miller, bin_off, nbins)
             nk = np.diff(bin_off)
             for j in range(k0, k1):
-                meta = batch.metas[j]
+                meta = b.metas[j]
                 sums[meta.index] = out[j - k0]
-                props[meta.index] = (ats[j], meta.natoms, nk)
+                props[meta.index] = (b.atom_types[j], meta.natoms, nk)
             k0 = k1
-    _agree_sharding(batches, device)
-    T = batches.total_frames or 0
-    if T == 0:
-        raise ValueError(f"no dump frames found for {filename!r}")
-    allp = torch.zeros((T, rows, nbins), dtype=torch.float64, device=device)
-    for idx, t in sums.items():
-        allp[idx] = t
-    dist.all_reduce_sum_(allp)
-    allp = allp.cpu().numpy()
-    if dist.world_size() > 1:
-        props = _gather_props(props, T)
+    allp, props, T = merge_results(batches, sums, props, filename, (rows, nbins), torch.float64)
 
     w = np.array([1.0 if a == b else 2.0 for a in range(cmap.ncls) for b in range(a, cmap.ncls)])
     prow = [ops.sym_row(cmap.cls(a), cmap.cls(b), cmap.ncls) for a, b in relation_matrix]

@@ -539,7 +539,8 @@ def test_calc_atom_type_ids_matches_oracle():
 def test_class_maps_and_weights_reproduce_reference_counting():
     """Derive full/partial histograms from a class-pair histogram built on the CPU and compare with _rdf_loop."""
     from mdproptools_b200 import ops
-    from mdproptools_b200.structural.rdf_cn import _ClassMap, _sym_weights
+    from mdproptools_b200.common.frames import _ClassMap
+    from mdproptools_b200.structural.rdf_cn import _sym_weights
     rng = np.random.default_rng(3)
     n, L = 400, (12.0, 13.0, 11.0)
     pos = rng.uniform(0, 1, (3, n)) * np.asarray(L)[:, None]
@@ -570,11 +571,12 @@ def test_class_maps_and_weights_reproduce_reference_counting():
 
 def test_host_normalisation_is_bit_identical_to_reference(sample_dir, gold_structural):
     """Feed the reference's own raw counts through the product's host normalisation."""
+    from mdproptools_b200.common.frames import _value_counts
     from mdproptools_b200.io import dump as D
     from mdproptools_b200.structural import rdf_cn as R
     fr = next(D.read_dumps(os.path.join(sample_dir, "dump.nvt.0.dump"), ["id", "type"]))
     rel = [[9, 9, 9, 9], [1, 4, 6, 9]]
-    at = R._value_counts(fr.data["type"])
+    at = _value_counts(fr.data["type"])
     L = fr.box.lattice_lengths()
     rho, rho_pairs = R._calc_props(L, fr.natoms, at, at, 9, MASS, rel, "type")
     full, part = R._normalize_rdf(0.05, rho_pairs, at, rel, 4, 400, gold_structural["rdf_raw_part_f0"].astype(np.float64),
@@ -725,14 +727,15 @@ def test_per_frame_host_caches():
     """The caches that keep the consumer thread of the file pipeline off the critical path: _same_values (memcmp of
     contiguous arrays, element comparison otherwise), _TypeCache (recompute only when the column changes; an identical
     object needs no comparison), _PropsCache (box / density work once per kind of frame, consistency error on the first)."""
+    from mdproptools_b200.common.frames import _same_values, _TypeCache
     from mdproptools_b200.io.dump import Box
     from mdproptools_b200.io.pipeline import FrameMeta
     from mdproptools_b200.structural import rdf_cn as R
     a = np.arange(10, dtype=np.float64)
-    assert R._same_values(a, a.copy()) and not R._same_values(a, a + 1) and not R._same_values(a, a[:5])
-    assert R._same_values(a[::2], a[::2].copy()) and not R._same_values(a[::2], a[1::2])       # non-contiguous: element-wise
+    assert _same_values(a, a.copy()) and not _same_values(a, a + 1) and not _same_values(a, a[:5])
+    assert _same_values(a[::2], a[::2].copy()) and not _same_values(a[::2], a[1::2])       # non-contiguous: element-wise
     calls = []
-    tc = R._TypeCache()
+    tc = _TypeCache()
     make = lambda col: (calls.append(1), col.sum())[1]
     buf = np.stack([a, a, a + 1])
     assert tc.get(buf[0], make) == 45 and tc.get(buf[1], make) == 45 and len(calls) == 1     # equal rows of a staging buffer
@@ -775,7 +778,7 @@ sys.path.insert(0, {root!r})
 import numpy as np, torch, torch.distributed as d
 d.init_process_group("gloo", rank=int(os.environ["RANK"]), world_size=2)
 from mdproptools_b200 import dist
-from mdproptools_b200.structural.rdf_cn import _merge_frames, _gather_props
+from mdproptools_b200.common.frames import _merge_frames, _gather_props
 r = dist.rank()
 assert dist.world_size() == 2
 # frames round-robin: rank r owns frames r, r+2, ...; integer histograms merge exactly
@@ -808,7 +811,7 @@ whole = dist.all_gather_blocks(blk, 7)
 assert whole.shape == (7, 2, 3) and whole[:, 1, 2].tolist() == list(range(7))
 # sharded file reads: every rank reads only its files; frame index = file index; total = number of files
 from mdproptools_b200.io.pipeline import FrameBatches
-from mdproptools_b200.structural.rdf_cn import _agree_sharding, _RetryUnsharded
+from mdproptools_b200.common.frames import _agree_sharding, _RetryUnsharded
 def write(path, step, n=4):
     rows = "\n".join("%d 1 %g %g %g" % (i + 1, 0.5 * i + step, 1.0 * i, 2.0 * i) for i in range(n))
     return "ITEM: TIMESTEP\n%d\nITEM: NUMBER OF ATOMS\n%d\nITEM: BOX BOUNDS pp pp pp\n0 9\n0 9\n0 9\nITEM: ATOMS id type x y z\n%s\n" % (step, n, rows)
@@ -849,6 +852,33 @@ def test_two_rank_gloo_merge(tmp_path):
     res = subprocess.run(cmd, capture_output=True, text=True, timeout=300)
     assert res.returncode == 0, res.stdout + res.stderr
     assert res.stdout.count("ok") == 2
+
+
+def test_file_sharded_retries_one_call_unsharded():
+    """file_sharded runs a call with sharded reads and repeats only that call with shard_files=False when it meets a
+    multi-frame file; the next call reads sharded again, also after a retried call raised."""
+    from mdproptools_b200.common.frames import _RetryUnsharded, file_sharded
+    calls = []
+
+    @file_sharded
+    def entry(kind, scale=1, *, shard_files=True):
+        calls.append((kind, scale, shard_files))
+        if shard_files and kind != "one":
+            raise _RetryUnsharded()
+        if kind == "bad":
+            raise ValueError("no dump frames found")
+        return kind * scale
+
+    assert entry("one", 2) == "oneone" and calls == [("one", 2, True)]
+    calls.clear()
+    assert entry("multi", scale=3) == "multi" * 3 and calls == [("multi", 3, True), ("multi", 3, False)]
+    calls.clear()
+    with pytest.raises(ValueError, match="no dump frames"):
+        entry("bad")
+    assert calls == [("bad", 1, True), ("bad", 1, False)]
+    calls.clear()
+    assert entry("one") == "one" and calls == [("one", 1, True)]
+    assert entry.__name__ == "entry"
 
 
 def test_utilities_mirror_reference_import_paths(tmp_path):
