@@ -237,10 +237,11 @@ def file_sharded(fn):
 
 
 def _merge_frames(per_frame: dict, total_frames: int, shape, device, dtype=torch.int64):
-    """Place this rank's per-frame results into [T, *shape] and all-reduce (exact: every other rank adds zeros)."""
+    """Place this rank's per-frame results into [T, *shape] and all-reduce (exact: every other rank adds zeros).  ``per_frame``
+    maps a frame index to its [*shape] result, or a tuple of frame indices (a batch) to their [len(indices), *shape] results."""
     out = torch.zeros((total_frames,) + tuple(shape), dtype=dtype, device=device)
     for idx, t in per_frame.items():
-        out[idx] = t
+        out[torch.tensor(idx, device=device) if isinstance(idx, tuple) else idx] = t
     dist.all_reduce_sum_(out)
     return out
 

@@ -27,23 +27,10 @@ import torch
 
 from .. import dist, ops
 from ..common import constants
-from ..common.com_mols import atom_masses, mol_membership
-from ..io import dump as _dump
+from ..common.frames import _frame_batches, _merge_frames
 from ..io.pipeline import FrameBatches
-from .diffusion import fit_window, position_columns, unwrapped_positions
-
-
-def even_times(steps, units, timestep, source, who="the Einstein and Nernst-Einstein conductivity need"):
-    """Times in seconds of the frames' timesteps (in trajectory order), which must be evenly spaced: ValueError naming
-    ``who`` otherwise, and naming ``source`` when there is no frame."""
-    steps = np.asarray(steps, dtype=np.float64)
-    if len(steps) == 0:
-        raise ValueError(f"no dump frames found for {source}")
-    d = np.diff(steps)
-    if len(d) and not (d[0] > 0 and (d == d[0]).all()):
-        raise ValueError(f"{who} evenly spaced frames (timesteps "
-                         f"{steps[:3].tolist()}...: spacings {sorted(set(d.tolist()))[:4]})")
-    return steps * constants.TIME_CONVERSION[units] * timestep
+from .series import (DumpColumns, MoleculeLayout, all_reduce_groups, even_times, fit_window, lag_count, rank_blocks,
+                     unwrapped_positions)
 
 
 class Conductivity:
@@ -107,31 +94,20 @@ class Conductivity:
     def get_charge_flux(self):
         """J[3, ntypes, T] (:167-195)."""
         pattern = f"{self.working_dir}/{self.filename}"
-        cols = _dump.available_columns(pattern)
-        want = ["id", "type", "q", "vx", "vy", "vz"]
-        if not self.mass:
-            assert "mass" in cols, "Missing atom masses in dump file."
-            want.append("mass")
-        mol_type, _, seg_off = mol_membership(self.num_mols, self.num_atoms_per_mol)
-        ntypes = len(self.num_mols)
-        type_off = np.concatenate(([0], np.cumsum(self.num_mols))).astype(np.int64)
-        w, r = dist.world_size(), dist.rank()
-        sel = (lambda i: i % w == r) if w > 1 else None
-        batches = FrameBatches(pattern, want, frame_select=sel)
-        pieces, times = [], {}
+        want = DumpColumns(pattern).select(["id", "type", "q", "vx", "vy", "vz"], masses=not self.mass)
+        layout = MoleculeLayout(self.num_mols, self.num_atoms_per_mol, self.mass)
+        batches = _frame_batches(pattern, want, shard_files=False)
+        fluxes, times = {}, {}
         dev = torch.device("cuda", torch.cuda.current_device())    # a rank without frames still joins the collectives
-        seg_d = torch.from_numpy(seg_off.astype(np.int32)).to(dev)
         vs, qs = constants.VELOCITY_CONVERSION[self.units], constants.CHARGE_CONVERSION[self.units]
         for batch in batches:
             d = batch.wait()
             host = batch.host.numpy()
-            n = host.shape[2]
-            if seg_off[-1] != n:
-                raise ValueError(f"Length of values ({seg_off[-1]}) does not match length of index ({n})")
+            layout.check(host.shape[2])
             mcol = None if self.mass else batch.col("mass")
 
             def masses(k):
-                return atom_masses(host[k, 1], self.mass) if self.mass else host[k, mcol]
+                return layout.masses(host[k, 1], None if mcol is None else host[k, mcol], dev)
 
             vel = d[:, 3:6, :].contiguous()
             # the kernel sums each molecule's charge and mass once per call; the reference does it per frame
@@ -140,27 +116,17 @@ class Conductivity:
             static = bool((host[:, 2] == host[0, 2]).all() and (host[:, 1] == host[0, 1]).all()
                           and (mcol is None or (host[:, mcol] == host[0, mcol]).all()))
             if static:
-                j = ops.charge_flux(vel, torch.from_numpy(np.ascontiguousarray(masses(0))).to(dev), d[0, 2].contiguous(),
-                                    seg_d, type_off, vs, qs)
+                j = ops.charge_flux(vel, masses(0), d[0, 2].contiguous(), layout.seg_d, layout.type_off, vs, qs)
             else:
-                j = torch.cat([ops.charge_flux(vel[k:k + 1], torch.from_numpy(np.ascontiguousarray(masses(k))).to(dev),
-                                               d[k, 2].contiguous(), seg_d, type_off, vs, qs)
-                               for k in range(vel.shape[0])], dim=2)
-            pieces.append(([m.index for m in batch.metas], j))
-            for m in batch.metas:
-                times[m.index] = m.timestep * constants.TIME_CONVERSION[self.units] * self.timestep
-        T = batches.total_frames or 0
-        if T == 0:
-            raise ValueError(f"no dump frames found for {pattern!r}")
-        J = torch.zeros((3, ntypes, T), dtype=torch.float64, device=dev)
-        tt = torch.zeros((T,), dtype=torch.float64, device=dev)
-        for idxs, j in pieces:
-            ii = torch.tensor(idxs, device=dev)
-            J[:, :, ii] = j
-            tt[ii] = torch.tensor([times[i] for i in idxs], dtype=torch.float64, device=dev)
-        dist.all_reduce_sum_(J)
-        dist.all_reduce_sum_(tt)
-        self.time = tt.cpu().tolist()
+                j = torch.cat([ops.charge_flux(vel[k:k + 1], masses(k), d[k, 2].contiguous(), layout.seg_d, layout.type_off,
+                                               vs, qs) for k in range(vel.shape[0])], dim=2)
+            idxs = tuple(m.index for m in batch.metas)
+            fluxes[idxs] = j.permute(2, 0, 1)                                            # [F, 3, ntypes]
+            times[idxs] = torch.tensor([m.timestep * constants.TIME_CONVERSION[self.units] * self.timestep
+                                        for m in batch.metas], dtype=torch.float64, device=dev)
+        J = _merge_frames(fluxes, batches.total_frames, (3, len(self.num_mols)), dev, torch.float64)     # [T, 3, ntypes]
+        self.time = _merge_frames(times, batches.total_frames, (), dev, torch.float64).cpu().tolist()
+        J = J.permute(1, 2, 0).contiguous()
         self._flux_dev = J
         return J.cpu().numpy()
 
@@ -252,39 +218,35 @@ class Conductivity:
         plt.close(fig)
 
     # -- Einstein and Nernst-Einstein conductivity ------------------------------------------------------------
-    def _fixed_charge_frames(self, frame_select=None):
-        """Unwrapped positions of every (selected) frame, batch by batch: yields (frame indices, timesteps, pos [F,3,N]
-        device) and returns nothing; afterwards ``self._fixed`` holds (q, type, mass) of the first frame seen (host arrays,
-        None when this rank saw no frame).  Charges, types and masses must not change between frames (the Helfand moment of
-        fluctuating charges is not the integral of the flux): ValueError otherwise, also across ranks."""
+    def _fixed_charge_frames(self, layout, round_robin=False):
+        """Unwrapped positions of every frame (``round_robin``: of this rank's frames) of the molecules ``layout``, batch by
+        batch: yields (frame indices, timesteps, pos [F,3,N], atom masses [N], charges [N]; on the device) and returns
+        nothing; afterwards ``self._fixed`` holds (q, type, mass) of the first frame seen (host arrays, None when this rank
+        saw no frame) and ``self._total_frames`` the number of frames of the trajectory.  Charges, types and masses must not
+        change between frames (the Helfand moment of fluctuating charges is not the integral of the flux): ValueError
+        otherwise, also across ranks."""
         pattern = f"{self.working_dir}/{self.filename}"
-        cols = _dump.available_columns(pattern)
-        if not cols:
-            raise ValueError(f"no dump frames found for {pattern!r}")
-        pos_cols = position_columns(cols)
-        want = ["id", "type", "q"] + pos_cols
-        if not self.mass:
-            assert "mass" in cols, "Missing atom masses in dump file."
-            want.append("mass")
-        _, _, seg_off = mol_membership(self.num_mols, self.num_atoms_per_mol)
+        want = DumpColumns(pattern).select(["id", "type", "q"], positions=True, masses=not self.mass)
         self._fixed = None
-        for batch in FrameBatches(pattern, want, frame_select=frame_select):
+        batches = _frame_batches(pattern, want, shard_files=False) if round_robin else FrameBatches(pattern, want)
+        for batch in batches:
             d = batch.wait()
             host = batch.host.numpy()
-            if seg_off[-1] != host.shape[2]:
-                raise ValueError(f"Length of values ({seg_off[-1]}) does not match length of index ({host.shape[2]})")
+            layout.check(host.shape[2])
             mcol = None if self.mass else batch.col("mass")
             if self._fixed is None:
                 q0, t0 = host[0, 2].copy(), host[0, 1].copy()
-                self._fixed = (q0, t0, atom_masses(t0, self.mass) if self.mass else host[0, mcol].copy())
+                self._fixed = (q0, t0, layout.masses(t0, None if mcol is None else host[0, mcol]))
+                md, qd = torch.from_numpy(self._fixed[2]).to(d.device), torch.from_numpy(q0).to(d.device)
             q0, t0, m0 = self._fixed
             if not ((host[:, 2] == q0).all() and (host[:, 1] == t0).all() and (mcol is None or (host[:, mcol] == m0).all())):
                 raise ValueError("charges, types and masses must be the same in every frame for the Einstein and "
                                  "Nernst-Einstein conductivity")
-            yield ([m.index for m in batch.metas], [m.timestep for m in batch.metas],
-                   unwrapped_positions(d, batch.metas, 3, len(pos_cols) == 3).contiguous())
+            yield (tuple(m.index for m in batch.metas), [m.timestep for m in batch.metas],
+                   unwrapped_positions(d, batch.metas, 3, want[3] == "xu").contiguous(), md, qd)
+        self._total_frames = batches.total_frames
         if dist.world_size() > 1:                     # the same charges, types and masses on every rank
-            n = int(seg_off[-1])
+            n = int(layout.seg_off[-1])
             dev = torch.device("cuda", torch.cuda.current_device())
             ref = (torch.from_numpy(np.concatenate(self._fixed)).to(dev) if self._fixed is not None
                    else torch.full((3 * n,), -np.inf, dtype=torch.float64, device=dev))
@@ -305,39 +267,18 @@ class Conductivity:
         """M[3, ntypes, T] in C m: per type, the sum over molecules of charge x unwrapped centre of mass (SI).  Positions
         are ``xu yu zu`` or x + ix (xhi - xlo) (as ``Diffusion``); charges, types and masses must be fixed and the frames
         evenly spaced (ValueError otherwise).  Sets ``self.time``."""
-        _, _, seg_off = mol_membership(self.num_mols, self.num_atoms_per_mol)
-        ntypes = len(self.num_mols)
-        type_off = np.concatenate(([0], np.cumsum(self.num_mols))).astype(np.int64)
-        w, r = dist.world_size(), dist.rank()
+        layout = MoleculeLayout(self.num_mols, self.num_atoms_per_mol, self.mass)
         dev = torch.device("cuda", torch.cuda.current_device())
-        seg_d = torch.from_numpy(seg_off.astype(np.int32)).to(dev)
         ds, qs = constants.DISTANCE_CONVERSION[self.units], constants.CHARGE_CONVERSION[self.units]
-        pieces, steps = [], {}
-        frames = self._fixed_charge_frames((lambda i: i % w == r) if w > 1 else None)
-        md = qd = None
-        for idxs, ts, pos in frames:
-            if md is None:
-                md = torch.from_numpy(np.ascontiguousarray(self._fixed[2])).to(dev)
-                qd = torch.from_numpy(np.ascontiguousarray(self._fixed[0])).to(dev)
+        dipoles, steps = {}, {}
+        for idxs, ts, pos, md, qd in self._fixed_charge_frames(layout, round_robin=True):
             # the charge-flux reduction (csrc/reduce.cu) of positions instead of velocities
-            pieces.append((idxs, ops.charge_flux(pos, md, qd, seg_d, type_off, ds, qs)))
-            steps.update(zip(idxs, ts))
-        T = torch.zeros((1,), dtype=torch.float64, device=dev)
-        T[0] = max(steps) + 1 if steps else 0
-        dist.all_reduce_max_(T)
-        T = int(T.item())
-        if T == 0:
-            raise ValueError(f"no dump frames found for {self.working_dir}/{self.filename!r}")
-        M = torch.zeros((3, ntypes, T), dtype=torch.float64, device=dev)
-        st = torch.zeros((T,), dtype=torch.float64, device=dev)
-        for idxs, m in pieces:
-            ii = torch.tensor(idxs, device=dev)
-            M[:, :, ii] = m
-            st[ii] = torch.tensor([float(steps[i]) for i in idxs], dtype=torch.float64, device=dev)
-        dist.all_reduce_sum_(M)
-        dist.all_reduce_sum_(st)
-        self._set_even_time(st.cpu().numpy())
-        return M.cpu().numpy()
+            m = ops.charge_flux(pos, md, qd, layout.seg_d, layout.type_off, ds, qs)
+            dipoles[idxs] = m.permute(2, 0, 1)                                           # [F, 3, ntypes]
+            steps[idxs] = torch.tensor([float(s) for s in ts], dtype=torch.float64, device=dev)
+        M = _merge_frames(dipoles, self._total_frames, (3, len(self.num_mols)), dev, torch.float64)      # [T, 3, ntypes]
+        self._set_even_time(_merge_frames(steps, self._total_frames, (), dev, torch.float64).cpu().numpy())
+        return M.permute(1, 2, 0).contiguous().cpu().numpy()
 
     def correlate_translational_dipole(self, dipole, max_lag=None):
         """[ntypes+1, max_lag] in C^2 m^2: row i = sum_j sum_axes <dM_i(lag) . dM_j(lag)> over all time origins, last row
@@ -346,9 +287,7 @@ class Conductivity:
         T // 2."""
         m = torch.as_tensor(np.ascontiguousarray(dipole, dtype=np.float64)).cuda()
         _, ntypes, T = m.shape
-        max_lag = T // 2 if max_lag is None else min(int(max_lag), T)
-        if max_lag < 1:
-            raise ValueError(f"max_lag must be at least 1 ({T} frames)")
+        max_lag = lag_count(max_lag, T)
         tot = m[:, 0].clone()
         for i in range(1, ntypes):                      # fixed order
             tot += m[:, i]
@@ -400,39 +339,29 @@ class Conductivity:
         row the sum.  D_g is slope / 6 of the all-origins centre-of-mass MSD of type g, fitted as in ``einstein`` (same
         window defaults, so sigma_NE / sigma_E is the Haven ratio); q_m is the molecule's charge summed in atom order.
         ``save`` writes nernst_einstein.csv (type, diffusion (m2/s), cond)."""
-        _, _, seg_off = mol_membership(self.num_mols, self.num_atoms_per_mol)
+        layout = MoleculeLayout(self.num_mols, self.num_atoms_per_mol, self.mass)
         ntypes = len(self.num_mols)
-        type_off = np.concatenate(([0], np.cumsum(self.num_mols))).astype(np.int64)
         dev = torch.device("cuda", torch.cuda.current_device())
-        seg_d = torch.from_numpy(seg_off.astype(np.int32)).to(dev)
         # every rank parses every frame; the molecules of each type are split in contiguous blocks over the ranks
-        shards = [dist.shard_range(int(n)) for n in self.num_mols]
-        sel = np.concatenate([np.arange(type_off[g] + lo, type_off[g] + hi) for g, (lo, hi) in enumerate(shards)])
-        sel_d = torch.from_numpy(sel.astype(np.int64)).to(dev)
-        coms, steps, md = [], [], None
-        for _, ts, pos in self._fixed_charge_frames():
-            if md is None:
-                md = torch.from_numpy(np.ascontiguousarray(self._fixed[2])).to(dev)
-            com, _, _ = ops.segment_com(pos, md, seg_d)                          # [F, 3, M]
+        sel_d, nloc = rank_blocks(layout.type_members(), dev)
+        coms, steps = [], []
+        for _, ts, pos, md, _ in self._fixed_charge_frames(layout):
+            com, _, _ = ops.segment_com(pos, md, layout.seg_d)                 # [F, 3, M]
             coms.append(com.index_select(2, sel_d))
             steps += ts
         self._set_even_time(steps)
         T = len(steps)
-        max_lag = T // 2 if max_lag is None else min(int(max_lag), T)
-        t, mask = self._fit_window(max(max_lag, 1), initial_time, final_time)
+        max_lag = lag_count(max_lag, T)
+        t, mask = self._fit_window(max_lag, initial_time, final_time)
         conv = constants.DISTANCE_CONVERSION[self.units]
         com = torch.cat(coms, dim=0) * conv                                     # [T, 3, Mloc] in m
         chans = com.permute(2, 1, 0).reshape(-1, T).contiguous()                # [Mloc * 3, T]
-        goff = 3 * np.concatenate(([0], np.cumsum([hi - lo for lo, hi in shards]))).astype(np.int64)
-        if chans.shape[0]:
-            msd = ops.cross_msd_fft(chans, None, goff, max_lag)
-        else:                                       # a rank without molecules still joins the all-reduce
-            msd = torch.zeros((ntypes, max_lag), dtype=torch.float64, device=dev)
-        dist.all_reduce_sum_(msd)
+        goff = 3 * np.concatenate(([0], np.cumsum(nloc))).astype(np.int64)
+        msd = all_reduce_groups(lambda c: ops.cross_msd_fft(c, None, goff, max_lag), chans, ntypes, max_lag)
         msd = msd.cpu().numpy() / np.asarray(self.num_mols, dtype=np.float64)[:, None]
         diff = np.array([self._slope(t[mask], row[mask]) for row in msd]) / 6
-        qmol = np.add.reduceat(self._fixed[0], seg_off[:-1]) * constants.CHARGE_CONVERSION[self.units]
-        q2 = np.array([np.sum(qmol[type_off[g]:type_off[g + 1]] ** 2) for g in range(ntypes)])
+        qmol = np.add.reduceat(self._fixed[0], layout.seg_off[:-1]) * constants.CHARGE_CONVERSION[self.units]
+        q2 = np.array([np.sum(qmol[a:b] ** 2) for a, b in zip(layout.type_off[:-1], layout.type_off[1:])])
         cond = diff * q2 / (self.volume * constants.BOLTZMANN * self.temp)
         cond = np.append(cond, cond.sum())
         if save and dist.rank() == 0:

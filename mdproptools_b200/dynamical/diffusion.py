@@ -24,50 +24,11 @@ import torch
 
 from .. import dist, ops
 from ..common import constants
-from ..common.com_mols import atom_masses, mol_membership
-from ..io import dump as _dump
+from ..io.log import concat_log
 from ..io.pipeline import ArrayBatches, FrameBatches
-
-
-class MissingCoordinatesError(AssertionError, ValueError):
-    """A dump without unwrapped coordinates and without the image flags to build them (an ``AssertionError``, as in the
-    reference, and a ``ValueError``)."""
-
-
-def position_columns(cols):
-    """Dump columns of the unwrapped positions (_prepare_unwrapped_coords :62-81): ``xu yu zu`` when ``zu`` is present, else
-    ``x y z ix iy iz`` (unwrapped as x + ix * (xhi - xlo) by ``unwrapped_positions``)."""
-    if "zu" in cols:
-        return ["xu", "yu", "zu"]
-    if "z" not in cols:
-        raise MissingCoordinatesError("Missing wrapped and unwrapped coordinates (x y z xu yu zu)")
-    if "iz" not in cols:
-        raise MissingCoordinatesError("Missing unwrapped coordinates (xu yu zu) and box location ("
-                                      "ix iy iz) for converting wrapped coordinates (x y z) into "
-                                      "unwrapped coordinates. ")
-    return ["x", "y", "z", "ix", "iy", "iz"]
-
-
-def unwrapped_positions(dev, metas, k0, have_u):
-    """[F,3,N] unwrapped positions of a parsed batch ``dev`` [F,C,N] whose columns k0.. are those of ``position_columns``
-    (``have_u``: the three ``xu yu zu``; else the six ``x y z ix iy iz``)."""
-    if have_u:
-        return dev[:, k0:k0 + 3, :]
-    L = torch.tensor([m.box.bound_lengths() for m in metas], dtype=torch.float64, device=dev.device)
-    return dev[:, k0:k0 + 3, :] + dev[:, k0 + 3:k0 + 6, :] * L[:, :, None]      # x.add(ix.multiply(L)) (:78-80)
-
-
-def fit_window(t, initial_time=None, final_time=None):
-    """Mask of the lag times ``t`` (l * dt, l < L) inside [initial_time, final_time]; by default the lags max(1, L // 10)
-    to L - 1, which leaves out the first tenth of the curve.  ValueError when the window holds fewer than 2 lag times."""
-    L = len(t)
-    lo = t[min(max(1, L // 10), L - 1)] if initial_time is None else initial_time
-    hi = t[L - 1] if final_time is None else final_time
-    mask = (t >= lo) & (t <= hi)
-    if L < 2 or mask.sum() < 2:
-        raise ValueError(f"the fit window [{lo}, {hi}] holds {int(mask.sum()) if L >= 2 else 0} lag times; "
-                         "at least 2 are needed")
-    return mask
+from .series import (DumpColumns, MoleculeLayout, all_reduce_groups, even_times, fit_window, lag_count, rank_blocks,
+                     unwrapped_positions)
+from .series import MissingCoordinatesError, position_columns  # noqa: F401  (public under this path)
 
 
 VDOS_WINDOWS = ("hann", "none")
@@ -102,24 +63,22 @@ class Diffusion:
         self.timestep = timestep
 
     # ------------------------------------------------------------------------------------------
-    def _load_unwrapped(self, filename, extra_cols=()):
-        """Read every frame; returns (times[T], metas, coords device [T,3,N], host columns of frame 0).
+    def _load_unwrapped(self, filename, extra_cols=(), masses=False):
+        """Read every frame; returns (times[T], metas, coords device [T,3,N], host columns of frame 0).  ``masses``: the
+        dump's ``mass`` column is read too (``DumpColumns.select``).
 
         _prepare_unwrapped_coords (:62-81): when ``zu`` is absent, xu = x + ix * (xhi - xlo) etc."""
         pattern = f"{self.outputs_dir}/{filename}"
-        cols = _dump.available_columns(pattern)
-        if not cols:
-            raise ValueError(f"no dump frames found for {pattern!r}")
-        assert "id" in cols, "Missing atom id's in dump file."
-        want = ["id"] + position_columns(cols)
-        have_u = len(want) == 4
-        want += [c for c in extra_cols if c not in want]
+        plan = DumpColumns(pattern)
+        assert "id" in plan.available, "Missing atom id's in dump file."
+        want = plan.select(["id", *extra_cols], positions=True, masses=masses)
+        k0 = 1 + len(extra_cols)
         chunks, metas, first_host = [], [], None
         for batch in FrameBatches(pattern, want):
             dev = batch.wait()
             if first_host is None:
                 first_host = {c: batch.host[0, k].numpy().copy() for k, c in enumerate(want)}
-            chunks.append(unwrapped_positions(dev, batch.metas, 1, have_u).contiguous())
+            chunks.append(unwrapped_positions(dev, batch.metas, k0, want[k0] == "xu").contiguous())
             metas += batch.metas
         coords = torch.cat(chunks, dim=0) if len(chunks) > 1 else chunks[0]
         times = np.array([m.timestep * self.timestep * constants.TIME_CONVERSION[self.units] for m in metas])
@@ -136,6 +95,14 @@ class Diffusion:
         if len(z) == 0:
             raise KeyError(0)      # msd_all.xs(0, 0) in the reference (:213)
         return int(z[0])
+
+    def _com_series(self, filename, num_mols, num_atoms_per_mol, mass):
+        """Unwrapped molecule centres of mass of every frame: (times[T], com device [T,3,M], mol_mass [M], layout)."""
+        times, _, coords, h0 = self._load_unwrapped(filename, extra_cols=["type"], masses=not mass)
+        layout = MoleculeLayout(num_mols, num_atoms_per_mol, mass)
+        layout.check(coords.shape[2])                 # before segment_com, which reads seg_off unchecked
+        com, mol_mass, _ = ops.segment_com(coords, layout.masses(h0["type"], h0.get("mass"), coords.device), layout.seg_d)
+        return times, com, mol_mass, layout
 
     def get_msd_from_dump(self, filename, msd_type="com", num_mols=None, num_atoms_per_mol=None, mass=None, com_drift=False,
                           avg_interval=False, tao_coeff=4):
@@ -178,33 +145,20 @@ class Diffusion:
             return msd, msd_all
 
         # ---- centre-of-mass MSD per molecule type -------------------------------------------------
-        extra = ["type"] if mass else ["type", "mass"]
-        times, metas, coords, h0 = self._load_unwrapped(filename, extra_cols=extra)
-        if not mass:
-            assert "mass" in h0, "Missing atom masses in dump file."
-            m_atom = h0["mass"]
-        else:
-            m_atom = atom_masses(h0["type"], mass)
-        mol_type, mol_id, seg_off = mol_membership(num_mols, num_atoms_per_mol)
-        T, _, N = coords.shape
-        if seg_off[-1] != N:
-            raise ValueError(f"Length of values ({seg_off[-1]}) does not match length of index ({N})")
-        dev = coords.device
-        com, mol_mass, _ = ops.segment_com(coords, torch.from_numpy(m_atom).to(dev),
-                                           torch.from_numpy(seg_off.astype(np.int32)).to(dev))          # [T,3,M]
-        M = com.shape[2]
+        times, com, mol_mass, layout = self._com_series(filename, num_mols, num_atoms_per_mol, mass)   # com [T,3,M]
+        T, _, M = com.shape
+        dev = com.device
         com = com * conv                                                  # SI before anything else (:201-203)
         mol_mass = mol_mass * constants.MASS_CONVERSION[self.units]       # (:193)
         ntypes = len(num_mols)
-        type_off = np.concatenate(([0], np.cumsum(num_mols))).astype(np.int64)
         t0 = self._time_zero_index(times)
         if com_drift:
             # _modify_dump_coordinates (:91-96): subtract the drift of each type's centre of mass
-            tcom, _, _ = ops.segment_com(com, mol_mass, torch.from_numpy(type_off.astype(np.int32)).to(dev))   # [T,3,ntypes]
+            tcom, _, _ = ops.segment_com(com, mol_mass, torch.from_numpy(layout.type_off.astype(np.int32)).to(dev))  # [T,3,G]
             drift = tcom - tcom[t0:t0 + 1]
             tidx = torch.from_numpy(np.repeat(np.arange(ntypes), num_mols)).to(dev)
             com = (com - drift.index_select(2, tidx)).contiguous()
-        sums, per_mol = ops.msd_single_origin(com, com[t0].contiguous(), 1.0, group_off=type_off, per_atom=True)
+        sums, per_mol = ops.msd_single_origin(com, com[t0].contiguous(), 1.0, group_off=layout.type_off, per_atom=True)
         counts = torch.tensor(np.asarray(num_mols, dtype=np.float64), device=dev)
         mean = (sums / counts[None, :, None]).cpu().numpy()              # [T, ntypes, 4]
         cols, data = [], []
@@ -216,14 +170,14 @@ class Diffusion:
         msd.insert(0, "Time (s)", times)
         pm = per_mol.permute(0, 2, 1).reshape(T * M, 4).cpu().numpy()
         msd_all = pd.DataFrame(pm, columns=disps + ["msd"])
-        msd_all.insert(0, "mol_id", np.tile(mol_id, T))
-        msd_all.insert(0, "type", np.tile(mol_type, T))
+        msd_all.insert(0, "mol_id", np.tile(layout.mol_id, T))
+        msd_all.insert(0, "type", np.tile(layout.mol_type, T))
         msd_all.insert(0, "Time (s)", np.repeat(times, M))
         if avg_interval:
             mi = ops.msd_interval(com[::tao_coeff].contiguous(), 1.0, 1).cpu().numpy()
             msd_int = pd.DataFrame(mi.T, columns=disps + ["msd"])
-            msd_int.insert(0, "mol_id", mol_id)
-            msd_int.insert(0, "type", mol_type)
+            msd_int.insert(0, "mol_id", layout.mol_id)
+            msd_int.insert(0, "type", layout.mol_type)
             return msd, msd_all, msd_int
         return msd, msd_all
 
@@ -263,14 +217,8 @@ class Diffusion:
             times, metas, coords, h0 = self._load_unwrapped(filename)
             group_off, counts, labels = None, np.array([coords.shape[2]], dtype=np.float64), [""]
         else:
-            extra = ["type"] if mass else ["type", "mass"]
-            times, metas, coords, h0 = self._load_unwrapped(filename, extra_cols=extra)
-            m_atom = atom_masses(h0["type"], mass) if mass else h0["mass"]
-            _, _, seg_off = mol_membership(num_mols, num_atoms_per_mol)
-            coords, _, _ = ops.segment_com(coords, torch.from_numpy(m_atom).to(coords.device),
-                                           torch.from_numpy(seg_off.astype(np.int32)).to(coords.device))
-            group_off = np.concatenate(([0], np.cumsum(num_mols))).astype(np.int64)
-            counts = np.asarray(num_mols, dtype=np.float64)
+            times, coords, _, layout = self._com_series(filename, num_mols, num_atoms_per_mol, mass)
+            group_off, counts = layout.type_off, np.asarray(num_mols, dtype=np.float64)
             labels = [str(k + 1) for k in range(len(num_mols))]
         T, _, N = coords.shape
         max_lag = T if max_lag is None else min(int(max_lag), T)
@@ -354,8 +302,6 @@ class Diffusion:
 
     def get_msd_from_log(self, log_pattern):
         """MSD columns of LAMMPS thermo logs converted to SI (:241-265)."""
-        from ..io.log import concat_log
-
         full_log = concat_log(log_pattern, step=None, working_dir=self.outputs_dir)
         msd = full_log.filter(regex="msd").copy()
         for col in msd:
@@ -414,26 +360,20 @@ class Diffusion:
         The first column is ``Time (s)``, the lag times from 0.  Velocities are not centred: a drift is part of C.
         All (type, axis) groups go through one mdp_group_acf_fft call.  Multi-GPU: every rank parses every frame and
         keeps a contiguous block of each group's atoms (or molecules); the sums are merged with one fp64 all-reduce."""
-        from .conductivity import even_times
-
         if vacf_type not in ("allatom", "com"):
             raise ValueError("vacf_type must be 'allatom' or 'com'.")
         if max_lag is not None and int(max_lag) < 1:
             raise ValueError(f"max_lag must be at least 1, got {max_lag}")
         pattern = f"{self.outputs_dir}/{filename}"
-        cols = _dump.available_columns(pattern)
-        if not cols:
-            raise ValueError(f"no dump frames found for {pattern!r}")
-        if not {"vx", "vy", "vz"} <= set(cols):
-            raise ValueError(f"the velocity autocorrelation needs the dump columns vx vy vz ({pattern!r} has {sorted(cols)})")
-        want = ["id", "type", "vx", "vy", "vz"]
+        plan = DumpColumns(pattern)
+        if not {"vx", "vy", "vz"} <= set(plan.available):
+            raise ValueError(f"the velocity autocorrelation needs the dump columns vx vy vz "
+                             f"({pattern!r} has {sorted(plan.available)})")
         com = vacf_type == "com"
-        if com and not mass:
-            assert "mass" in cols, "Missing atom masses in dump file."
-            want.append("mass")
+        want = plan.select(["id", "type", "vx", "vy", "vz"], masses=com and not mass)
         dev = torch.device("cuda", torch.cuda.current_device())
         vs = constants.VELOCITY_CONVERSION[self.units]
-        types0 = sel_d = md = seg_d = None
+        types0 = sel_d = md = layout = None
         pieces, steps = [], []
         for batch in FrameBatches(pattern, want):
             d = batch.wait()
@@ -441,36 +381,27 @@ class Diffusion:
             if types0 is None:
                 types0 = host[0, 1].copy()
                 if com:
-                    _, _, seg_off = mol_membership(num_mols, num_atoms_per_mol)
-                    if seg_off[-1] != len(types0):
-                        raise ValueError(f"Length of values ({seg_off[-1]}) does not match length of index ({len(types0)})")
-                    m_atom = atom_masses(types0, mass) if mass else host[0, batch.col("mass")]
-                    md = torch.from_numpy(np.ascontiguousarray(m_atom, dtype=np.float64)).to(dev)
-                    seg_d = torch.from_numpy(seg_off.astype(np.int32)).to(dev)
+                    layout = MoleculeLayout(num_mols, num_atoms_per_mol, mass)
+                    layout.check(len(types0))
+                    md = layout.masses(types0, None if mass else host[0, batch.col("mass")], dev)
                     labels = [str(k + 1) for k in range(len(num_mols))]
-                    first = np.concatenate(([0], np.cumsum(num_mols))).astype(np.int64)
-                    members = [np.arange(first[g], first[g + 1]) for g in range(len(num_mols))]
+                    members = layout.type_members()
                 else:
                     tids = np.unique(types0)
                     labels = [str(int(t)) for t in tids]
                     members = [np.nonzero(types0 == t)[0] for t in tids]
-                # this rank's contiguous block of every group, gathered into group order once per batch
-                local = [idx[slice(*dist.shard_range(len(idx)))] for idx in members]
-                sel_d = torch.from_numpy(np.concatenate(local).astype(np.int64)).to(dev)
-                nloc = [len(idx) for idx in local]
+                sel_d, nloc = rank_blocks(members, dev)
                 counts = np.array([len(idx) for idx in members], dtype=np.float64)
             if not (host[:, 1] == types0).all():
                 raise ValueError("atom types must be the same in every frame for the velocity autocorrelation")
             vel = d[:, 2:5, :]
             if com:
-                vel, _, _ = ops.segment_com(vel.contiguous(), md, seg_d)                 # [F, 3, M]
+                vel, _, _ = ops.segment_com(vel.contiguous(), md, layout.seg_d)       # [F, 3, M]
             pieces.append(vel.index_select(2, sel_d) * vs)                               # [F, 3, local]
             steps += [m.timestep for m in batch.metas]
         times = even_times(steps, self.units, self.timestep, repr(pattern), who="the velocity autocorrelation needs")
         T = len(steps)
-        max_lag = T // 2 if max_lag is None else min(int(max_lag), T)
-        if max_lag < 1:
-            raise ValueError(f"max_lag must be at least 1 ({T} frames)")
+        max_lag = lag_count(max_lag, T)
         v = torch.cat(pieces, dim=0) if len(pieces) > 1 else pieces[0]                   # [T, 3, local]
         del pieces
         # channels [group][axis][atom] (groups are (type, axis)), one row per series
@@ -482,12 +413,8 @@ class Diffusion:
             chans[3 * s0:3 * (s0 + nloc[g])].view(3, nloc[g], T).copy_(v[:, :, s0:s0 + nloc[g]].permute(1, 2, 0))
             s0 += nloc[g]
         del v
-        if chans.shape[0]:
-            sums = ops.group_acf_fft(chans, goff, max_lag)                               # [3 G, max_lag]
-        else:                                       # a rank without atoms still joins the all-reduce
-            sums = torch.zeros((3 * G, max_lag), dtype=torch.float64, device=dev)
+        sums = all_reduce_groups(lambda c: ops.group_acf_fft(c, goff, max_lag), chans, 3 * G, max_lag)   # [3 G, max_lag]
         del chans
-        dist.all_reduce_sum_(sums)
         sums = sums.cpu().numpy().reshape(G, 3, max_lag)
         out = {"Time (s)": times[:max_lag] - times[0]}
         for g, lab in enumerate(labels):

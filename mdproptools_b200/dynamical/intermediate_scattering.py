@@ -35,7 +35,7 @@ from ..common.frames import _ClassMap, _value_counts, calc_atom_type_ids
 from ..io.dump import dump_files
 from ..io.pipeline import FrameBatches
 from ..structural.structure_factor import _cell, kset
-from .conductivity import even_times
+from .series import even_times
 
 
 def shard_bins(bin_off, r, w):

@@ -27,7 +27,7 @@ import pandas as pd
 import torch
 
 from .. import dist, ops
-from ..common.frames import calc_atom_type_ids
+from ..common.frames import _merge_frames, calc_atom_type_ids
 from ..io import dump as _dump
 from ..io.pipeline import FrameBatches
 
@@ -101,13 +101,10 @@ class ResidenceTime:
         if T == 0:
             raise ValueError(f"no dump frames found for {self.filename!r}")
         # every rank needs every frame's time and the sizes of the two sets (a rank may have had no frame at all)
-        tt = torch.zeros((T,), dtype=torch.int64, device=dev)
-        for idx, ts in own.items():
-            tt[idx] = ts
+        tt = _merge_frames(own, T, (), dev)
         nkl = torch.tensor([[len(rows_k[kl]), len(rows_l[kl])] if rows_k[kl] is not None else [0, 0] for kl in range(R)],
                            dtype=torch.int64, device=dev).reshape(R, 2)
         if w > 1:
-            dist.all_reduce_sum_(tt)
             dist.all_reduce_max_(nkl)
         times = [float(v) * self.dt for v in tt.cpu().numpy()]
         nkl = nkl.cpu().numpy()

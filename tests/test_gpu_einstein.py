@@ -373,6 +373,15 @@ def test_einstein_rejects_varying_charges_missing_positions_and_uneven_frames(op
                 getattr(cond(key), method)()
 
 
+def test_max_lag_below_one_is_rejected(ops, mini_dir, mini_mols, tmp_path):
+    """nernst, einstein and correlate_translational_dipole share the lag rule: max_lag = 0 names itself in the error."""
+    c = _mini_cond(mini_dir, mini_mols)
+    for call in (lambda: c.nernst(max_lag=0), lambda: c.einstein(max_lag=0),
+                 lambda: c.correlate_translational_dipole(c.get_translational_dipole(), max_lag=0)):
+        with pytest.raises(ValueError, match=r"max_lag must be at least 1 \(26 frames\)"):
+            call()
+
+
 # ------------------------------------------------------------------------------------------------
 # N ranks against one
 # ------------------------------------------------------------------------------------------------

@@ -320,6 +320,17 @@ def test_vacf_errors(ops, tmp_path):
         _diff(cases["ok"]).get_vdos(pd.DataFrame({"Time (s)": [0.0, 1.0], "vacf": [0.0, 1.0]}))
 
 
+def test_com_msd_all_origins_checks_molecule_atom_count(ops, mini_dir, mini_mols):
+    """Molecules that claim more or fewer atoms than the dump holds: the ValueError of get_msd_from_dump, raised on the host
+    before the centre-of-mass reduction would read past the arrays or drop atoms."""
+    df = _diff(mini_dir)
+    for extra in (1, -1):
+        mols = mini_mols[:-1] + [mini_mols[-1] + extra]
+        for call in (df.get_msd_all_origins, df.get_msd_from_dump):
+            with pytest.raises(ValueError, match="does not match length of index"):
+                call("dump.mini.*.dump", msd_type="com", num_mols=mols, num_atoms_per_mol=NUM_ATOMS, mass=MASS)
+
+
 # ------------------------------------------------------------------------------------------------
 # N ranks against one
 # ------------------------------------------------------------------------------------------------
