@@ -11,7 +11,9 @@
 // conj(P) gives N * conj(corr).  Stockham autosort: every stage reads one array and writes the other, no bit reversal, all
 // N/2 butterflies of a stage independent (one thread each).  Twiddles come from a table W[k] = exp(-2 pi i k / N),
 // k < N/2, computed once per call with sincospi (full fp64 accuracy: the result agrees with the direct sum to ~1e-15 of
-// max|corr| times log2 N).
+// max|corr| times log2 N where T - tau is large; the unbiased division by T - tau amplifies the absolute round-off of
+// the lag sum at the last lags, to 9.3e-12 of max|corr| at lag T - 1 of T = 10^7 -- inside the 1e-10 contract at every
+// lag, tests/test_gpu_long_series.py).
 #pragma once
 #include <math.h>
 #include <stdint.h>

@@ -737,6 +737,14 @@ def test_cumtrapz_kernel(ops):
         got = ops.cumtrapz(_dev(y), 0.37, 2.5, leading_zero=lead).cpu().numpy()
         ref = np.stack([2.5 * O.cumtrapz(r, 0.37, lead) for r in y])
         assert np.allclose(got, ref, rtol=0, atol=1e-12 * np.abs(ref).max())
+    # integer y, dx = 2^-3 and scale 2: every partial sum is exact, so the result is the int64 running sum bit for bit,
+    # at the lengths around the 1024-thread split (1025 trapezoids: one thread takes two) and at the long end
+    from tests import exact_series as ES
+    for T in (2, 3, 1024, 1025, 1026, 2049, 10 ** 6 + 1, 10 ** 7):
+        y = ES.ou_series(rng, 3, T, tau=100.0, sigma=1000.0)
+        for lead in (True, False):
+            got = ops.cumtrapz(_dev(y.astype(np.float64)), 0.125, 2.0, leading_zero=lead).cpu().numpy()
+            assert np.array_equal(got, ES.cumtrapz_exact(y, 0.125, 2.0, lead)), (T, lead)
 
 
 def test_pair_list_and_bitmask_autocorr(ops):
