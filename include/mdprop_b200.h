@@ -49,7 +49,8 @@ int64_t mdp_ctx_launch_count(mdp_ctx *ctx);
  * 6 = bitmask autocorrelation kernel, 7 = FFT all-origins MSD (the whole of mdp_cross_msd_fft), 8 = structure factor (the
  * whole of mdp_structure_factor: kernels k_sk_sort, k_sk_rho, k_sk_bins; and of mdp_sk_rho: k_sk_sort, k_sk_rho), 9 = binned
  * FFT correlation of complex series (the whole of mdp_isf_fft: kernels k_isf_*), 10 = grouped FFT autocorrelation (the
- * whole of mdp_group_acf_fft: kernels k_fft_*, k_msd_spec_acc).  mdp_ctx_timing_read synchronises
+ * whole of mdp_group_acf_fft: kernels k_fft_*, k_msd_spec_acc), 11 = reorientation channels (the whole of mdp_orient_series:
+ * kernel k_orient).  mdp_ctx_timing_read synchronises
  * on the recorded events, returns the summed milliseconds and the number of launches, and clears them. */
 int mdp_ctx_timing(mdp_ctx *ctx, int enable);
 int mdp_ctx_timing_read(mdp_ctx *ctx, int tag, double *ms_total, int64_t *count);
@@ -321,6 +322,26 @@ int mdp_sk_rho(mdp_ctx *ctx, int nframes, int64_t n, const double *xyz, const in
  * npairs * nbins * (N/2 + 1) * 8 bytes) above the context's scratch limit. */
 int mdp_isf_fft(mdp_ctx *ctx, int nchan, int64_t nk, int64_t T, const double *rho, int npairs, const int32_t *pairs, int nbins,
                 const int64_t *bin_off, int64_t nlags, double *out, void *stream);
+
+/* ---- reorientation (extension, no reference implementation; tests/reorient_oracle.py is the definition) --------------
+ * Channels of molecule-fixed unit vectors (csrc/orient.h), one time series per (channel, vector):
+ *   d_j = mic(r_j - r_i), d_k = mic(r_k - r_i) in the frame's restricted triclinic cell (rows a = (lx,0,0), b = (xy,ly,0),
+ *   c = (xz,yz,lz); sequential LAMMPS reduction: d -= rint(d_z/lz) c, then rint(d_y/ly) b, then rint(d_x/lx) a);
+ *   w = d_j (kind 0, bond), (d_j + d_k)/2 (kind 1, bisector), d_j x d_k (kind 2, normal);  u = w / |w|;
+ *   rows 0-2: ux, uy, uz;  rows 3-7: (ux^2 - uy^2)/sqrt2, (2uz^2 - ux^2 - uy^2)/sqrt6, sqrt2 ux uy, sqrt2 ux uz, sqrt2 uy uz,
+ * so that the sum of rows 0-2 of u(t).u(t') is P1(u.u') and 1.5 times the sum of rows 3-7 is P2(u.u'), exactly: the
+ * all-origins autocorrelation of each row group (mdp_group_acf_fft) gives C1 and C2 with no per-lag Legendre evaluation.
+ * xyz = DEVICE [nframes][3][n] positions (wrapped or unwrapped: the same vectors for molecules short next to half the cell);
+ * cell = HOST [nframes][6] = (lx, ly, lz, xy, xz, yz) per frame; atoms = HOST int32 [nvec][3] rows of xyz (i, j, k; k is
+ * ignored for a bond); out = DEVICE double [8][nvec][out_stride]: frame f of the call goes to column frame0 + f (0 <= frame0,
+ * frame0 + nframes <= out_stride), so that successive calls fill one series in place; other columns are left alone.
+ * fp64 throughout; with the library's unfused arithmetic the values are bit-identical to a host build of csrc/orient.h.
+ * A zero-length or non-finite w gives NaN channels for that vector and frame.
+ * MDP_ERR_ARG (checked on the host before anything is launched) for negative sizes, n >= 2^31, a kind outside [0, 3), an
+ * atom index outside [0, n), a vector that repeats an atom, a non-positive or non-finite length, a non-finite tilt, or
+ * frames outside the series. */
+int mdp_orient_series(mdp_ctx *ctx, int nframes, int64_t n, const double *xyz, const double *cell, int kind, int64_t nvec,
+                      const int32_t *atoms, double *out, int64_t out_stride, int64_t frame0, void *stream);
 
 /* ---- residence time (residence_time.py:70-148) ---------------------------------------------------
  * Survival correlation from per-pair time bitmasks.  masks = DEVICE uint64 [npairs][nwords], bit t of

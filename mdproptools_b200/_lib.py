@@ -76,6 +76,8 @@ _PROTOS = {
                            c_void_p, c_int64, c_int64, c_void_p]),
     "mdp_isf_fft": (c_int, [c_void_p, c_int, c_int64, c_int64, c_void_p, c_int, POINTER(c_int32), c_int, POINTER(c_int64), c_int64,
                             c_void_p, c_void_p]),
+    "mdp_orient_series": (c_int, [c_void_p, c_int, c_int64, c_void_p, POINTER(c_double), c_int, c_int64, POINTER(c_int32), c_void_p,
+                                  c_int64, c_int64, c_void_p]),
     "mdp_cumtrapz": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_double, c_double, c_int, c_void_p, c_void_p]),
     "mdp_bitmask_fill": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "mdp_bitmask_autocorr": (c_int, [c_void_p, c_int64, c_int, c_int64, c_void_p, c_void_p, c_void_p]),
@@ -97,6 +99,7 @@ EXPORTED_SYMBOLS = tuple(_PROTOS)
 
 PAIR_NO_CULL, PAIR_NO_SORT, PAIR_TRICLINIC, PAIR_F64 = 1, 2, 4, 16   # flags of mdp_pair_hist / mdp_pair_list
 SK_NLIM, SK_MAX_CLASSES, SK_EPS = 1024, 64, 1e-5       # mdp_structure_factor: Miller bound, classes, accuracy (csrc/sk_phase.h)
+ORIENT_KINDS = {"bond": 0, "bisector": 1, "normal": 2}  # mdp_orient_series: vector kinds (csrc/orient.h)
 
 
 def lib() -> ctypes.CDLL:

@@ -15,9 +15,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmdprop_b200.so")
 
-CU_SOURCES = ["ctx.cu", "pair.cu", "reduce.cu", "corr.cu", "dump_device.cu", "survival.cu", "shell.cu", "fftcorr.cu", "msdfft.cu", "sk.cu", "isffft.cu", "epilogue.cu"]
+CU_SOURCES = ["ctx.cu", "pair.cu", "reduce.cu", "corr.cu", "dump_device.cu", "survival.cu", "shell.cu", "fftcorr.cu", "msdfft.cu", "sk.cu", "isffft.cu", "orient.cu", "epilogue.cu"]
 CPP_SOURCES = ["dump_parse.cpp"]
-HEADERS = ["common.cuh", "pair_fast.cuh", "dump_line.h", "dump_rows.h", "survival_runs.h", "shell_grid.h", "fft_corr.h", "fft_pass.cuh", "msd_fft.h", "isf_fft.h", "sk_phase.h", "scratch_plan.h",
+HEADERS = ["common.cuh", "pair_fast.cuh", "dump_line.h", "dump_rows.h", "survival_runs.h", "shell_grid.h", "fft_corr.h", "fft_pass.cuh", "msd_fft.h", "isf_fft.h", "orient.h", "sk_phase.h", "scratch_plan.h",
            os.path.join("..", "..", "include", "mdprop_b200.h")]
 
 NVCC_FLAGS = [

@@ -377,6 +377,26 @@ def isf_fft(rho, pairs, bin_off, nlags):
     return out
 
 
+def orient_series(xyz, cells, kind, atoms, out, frame0=0):
+    """mdp_orient_series: xyz float64 [F,3,N]; cells host [F,6] = (lx, ly, lz, xy, xz, yz) per frame; kind 0 (bond), 1
+    (bisector) or 2 (normal); atoms host ints [nvec,3] (rows of xyz; the third is ignored for a bond); out float64
+    [8, nvec, T] -> out, with the channels of frame f at column frame0 + f (other columns untouched)."""
+    xyz = _f64(xyz, "xyz")
+    F, _, n = xyz.shape
+    cells = np.ascontiguousarray(cells, dtype=np.float64).reshape(-1)
+    if cells.size != 6 * F:
+        raise ValueError(f"cells must hold 6 values (lx, ly, lz, xy, xz, yz) per frame ({F} frames), got {cells.size}")
+    atoms = np.ascontiguousarray(atoms, dtype=np.int32).reshape(-1, 3)
+    out = _f64(out, "out")
+    if out.dim() != 3 or out.shape[0] != 8 or out.shape[1] != atoms.shape[0]:
+        raise ValueError(f"out must be [8, {atoms.shape[0]}, T], got {tuple(out.shape)}")
+    ctx = Context.get(xyz.device.index)
+    check(lib().mdp_orient_series(ctx.handle, F, n, ptr(xyz), _lib.dptr(cells), int(kind), atoms.shape[0],
+                                  atoms.ctypes.data_as(ctypes.POINTER(c_int32)), ptr(out), out.shape[2], int(frame0),
+                                  stream_ptr()), "mdp_orient_series")
+    return out
+
+
 def cumtrapz(y, dx, scale=1.0, leading_zero=True):
     y = _f64(y, "y")
     R, T = y.shape
